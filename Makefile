@@ -9,7 +9,7 @@ LIB       := shardmerge_b200/libshardmerge_b200.so
 HDRS      := $(CSRC)/fft_core.cuh $(CSRC)/fft_bodies.cuh $(CSRC)/plan.h $(CSRC)/sm_internal.h include/shardmerge_b200.h
 OBJS      := build/kernels_fft.o build/kernels_stats.o build/kernels_fstats.o build/kernels_elem.o build/pipeline.o
 
-all: $(LIB) hostemu oracle_ref
+all: $(LIB) hostemu
 
 $(LIB): $(OBJS)
 	$(NVCC) $(ARCH) -shared -o $@ $(OBJS) -cudart static
@@ -25,12 +25,12 @@ tests/hostemu/libsm_hostemu.so: tests/hostemu/hostemu.cpp $(HDRS)
 clean:
 	rm -rf build $(LIB) tests/hostemu/libsm_hostemu.so
 
-# the reference itself as checker / timed CPU arm on the GPU box: a git-ignored copy of its Python package (the repo
-# history holds no reference source; oracle/ref_runner.py imports it).  No-op where /root/reference does not exist.
-REFERENCE ?= /root/reference
+# the reference itself as checker / timed CPU arm: `make oracle_ref REFERENCE=<checkout of 54rt1n/shardmerge>` keeps a
+# git-ignored copy of its Python package in oracle/_ref (the repository holds no reference source; oracle/ref_runner.py
+# imports it from there).  Not part of `all`: the build reads nothing outside the repository.
 oracle_ref:
-	@if [ -d $(REFERENCE)/shard ]; then mkdir -p oracle/_ref && rm -rf oracle/_ref/shard && cp -r $(REFERENCE)/shard oracle/_ref/shard \
+	@if [ -n "$(REFERENCE)" ] && [ -d $(REFERENCE)/shard ]; then mkdir -p oracle/_ref && rm -rf oracle/_ref/shard && cp -r $(REFERENCE)/shard oracle/_ref/shard \
 	  && find oracle/_ref -name __pycache__ -prune -exec rm -rf {} + && echo "oracle/_ref <- $(REFERENCE)/shard"; \
-	 else echo "oracle_ref: $(REFERENCE) not present, keeping oracle/_ref as is"; fi
+	 else echo "oracle_ref: REFERENCE=$(REFERENCE) holds no shard/ package, keeping oracle/_ref as is"; fi
 
 .PHONY: all hostemu clean oracle_ref

@@ -3,7 +3,7 @@
 merged params/sec, weight GB/s; % of HBM roofline for the dominant kernel).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload llama8b|llama70b|tinyllama] [--layers L] [--finetunes M]
+                    [--workload llama8b|llama70b|tinyllama] [--layers L] [--finetunes M] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the workload's merged tensors: for every
 `model.layers.*` tensor of the named architecture, base + M finetunes (synthetic random-init
@@ -223,6 +223,31 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20                   # sampled values of all tensors together; the .npy headers stay well inside 64 MB
+
+
+def dump_outputs(torch, out_dir, outputs, catalog):
+    """Write this rank's merged tensors as out_dir/<name>.npy (float32, flattened).  A tensor larger than its share of
+    DUMP_BYTES is sampled at sorted flat indices drawn from a generator seeded with its catalog index, so the same
+    arguments give the same positions in every run and two builds can be compared value for value."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    per_tensor = DUMP_BYTES // 4 // len(catalog)
+    seeds = {name: idx for name, _, idx in catalog}
+    total = 0
+    for name, t in outputs.items():
+        flat = t.reshape(-1)
+        n = flat.numel()
+        if n > per_tensor:
+            pos = np.sort(np.random.default_rng(seeds[name]).choice(n, size=per_tensor, replace=False))
+            flat = flat[torch.from_numpy(pos).to(flat.device)]
+        arr = flat.float().cpu().numpy()
+        np.save(out_dir / f"{name}.npy", arr)
+        total += arr.nbytes
+    print(f"[bench] wrote {len(outputs)} merged tensors ({total / 2**20:.1f} MiB of float32) to {out_dir}", file=sys.stderr)
+
+
+# ------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -238,7 +263,12 @@ def main():
     ap.add_argument("--e2e-files", type=int, default=1, help="0: skip the second e2e measurement that writes the shard files")
     ap.add_argument("--prefetch-depth", type=int, default=-1, help="tensors whose uploads run ahead in the e2e loop (-1: the strategy's default)")
     ap.add_argument("--profile-json", default="", help="write the per-kernel-class summary here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the merged tensors of the last timed step to DIR/<tensor name>.npy (float32; a fixed, "
+                         "seeded sample of each tensor, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -335,6 +365,8 @@ def main():
     gpu_launches = E.PROFILER.launches
     E.PROFILER = None
     clocks = sampler.stop()
+    if args.dump_outputs:                                         # before the serial pass below overwrites `outputs`
+        dump_outputs(torch, Path(args.dump_outputs), outputs, catalog)
     elapsed_ms = max_over_ranks(sum(s0.elapsed_time(s1) for s0, s1 in ev))
     value = merged_params * args.steps / (elapsed_ms / 1000.0)
     if world > 1:

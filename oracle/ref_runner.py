@@ -1,11 +1,10 @@
 """ref_runner.py -- run the REFERENCE ITSELF (unmodified 54rt1n/shardmerge `shard` package) as checker / CPU arm.
 
 TEST INFRASTRUCTURE.  Only tests/, __graft_entry__.smoke() and bench.py's CPU legs import this; nothing under
-shardmerge_b200/ does.  The reference is found, in this order, at
-  * oracle/_ref/shard   -- a git-ignored copy made by `make oracle_ref` from /root/reference (it travels to the GPU
-                           box with the repo snapshot; the repo history holds no reference source), or
-  * /root/reference     -- the read-only checkout in the build container.
-`device="cuda"` on the B200 box is the parity oracle for large tensors (same reference code, cuFFT + CUDA
+shardmerge_b200/ does.  The reference is found at oracle/_ref/shard: a git-ignored copy that
+`make oracle_ref REFERENCE=<checkout of the reference>` makes (the repository holds no reference source).  Where it is
+absent, the tests that run it skip.
+`device="cuda"` on a B200 is the parity oracle for large tensors (same reference code, cuFFT + CUDA
 reductions; the CPU reference's fp32 `.norm()` is biased at Llama sizes, SURVEY.md 0 / 7.3-0); `device="cpu"` is the
 timed CPU baseline (`FourierMerge._merge_layer`, shard/merge/fast_fourier.py:103-276).
 """
@@ -17,7 +16,7 @@ import tempfile
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-_CANDIDATES = [HERE / "_ref", Path("/root/reference")]
+_CANDIDATES = [HERE / "_ref"]
 
 
 def ref_root():
@@ -35,7 +34,7 @@ def load():
     """-> (shard.tensor.functions, FourierMerge, MergeConfig, MergeModel, ShardLayer) of the reference."""
     root = ref_root()
     if root is None:
-        raise RuntimeError("reference not available: run `make oracle_ref` where /root/reference exists")
+        raise RuntimeError("reference not available: run `make oracle_ref REFERENCE=<checkout of the reference>`")
     if str(root) not in sys.path:
         sys.path.insert(0, str(root))
     import shard.tensor.functions as F
