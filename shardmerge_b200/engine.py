@@ -200,6 +200,12 @@ class Workspace:
         return (int(h[o:o + 4].view(torch.int32)[0]),
                 int(h[o + _lib.FS_STATE_BYTES:o + _lib.FS_STATE_BYTES + 4].view(torch.int32)[0]))
 
+    def select_sticky(self) -> int:
+        """Sticky status of every order statistic since `ctl` was zeroed, as of the last read_ctl(): non-zero when a sampled
+        window missed, was too wide or overflowed, i.e. a threshold came out NaN and the tensor has to be redone with
+        safe_select."""
+        return select_sticky_of(self.ctl_host)
+
     def read_ctl(self):
         """Synchronous read-back of the scalar block -> (float64[8], float32[16], int32[4], sel bytes)."""
         self.ctl_host.copy_(self.ctl, non_blocking=True)
@@ -207,6 +213,16 @@ class Workspace:
         h = self.ctl_host
         return (h[_OFF_DBL:_OFF_DBL + 64].view(torch.float64), h[_OFF_FLT:_OFF_FLT + 64].view(torch.float32),
                 h[_OFF_FLAGS:_OFF_FLAGS + 16].view(torch.int32), h[_OFF_SEL:_OFF_SEL + 128])
+
+
+def select_sticky_of(h: torch.Tensor) -> int:
+    """OR of the sticky words of the two select states (int32 slots 11 and 27 of `sel`) and of the two fused statistics
+    states in a host copy `h` (uint8) of a scalar block."""
+    sel32 = h[_OFF_SEL:_OFF_SEL + 128].view(torch.int32)
+    fs = _lib.CTL_FS_OFF + _lib.FS_STICKY_OFF
+    fs0 = int(h[fs:fs + 4].view(torch.int32)[0])
+    fs1 = int(h[fs + _lib.FS_STATE_BYTES:fs + _lib.FS_STATE_BYTES + 4].view(torch.int32)[0])
+    return int(sel32[11]) | int(sel32[16 + 11]) | fs0 | fs1
 
 
 _plans: dict = {}
@@ -572,13 +588,9 @@ class PendingPair:
         h = self.host_ctl
         dbl = h[0:64].view(torch.float64); flt = h[64:128].view(torch.float32)
         flags = h[128:144].view(torch.int32); ints = h[144:160].view(torch.int32)
-        fs = _lib.CTL_FS_OFF + _lib.FS_STICKY_OFF
-        sel32 = h[192:320].view(torch.int32)
-        st0 = int(h[fs:fs + 4].view(torch.int32)[0]) | int(sel32[11])
-        st1 = int(h[fs + _lib.FS_STATE_BYTES:fs + _lib.FS_STATE_BYTES + 4].view(torch.int32)[0]) | int(sel32[16 + 11])
         self.info = dict(norms=[float(flt[9]), float(flt[10])], target_norm=float(h[160:168].view(torch.float64)[0]),
                          swap=int(ints[0]), branch=_lib.BRANCH_NAMES.get(int(ints[1]), "?"),
-                         select_sticky=st0 | st1, flags=[int(v) for v in flags],
+                         select_sticky=select_sticky_of(h), flags=[int(v) for v in flags],
                          thr_cut=float(flt[0]), thr_cull=float(flt[1]), dot=float(flt[2]))
         _ring.give(h)
         self.host_ctl = None

@@ -505,13 +505,9 @@ class FourierMerge(MergeTensorsBase):
             stack, weights = nxt, nxt_w
             cull_pct = cull_pct / 2.0                          # :254
 
-        _, _, flags, sel = ws.read_ctl()
+        _, _, flags, _ = ws.read_ctl()
         info["flags"] = [int(v) for v in flags]
-        sel32 = sel.view(torch.int32)
-        fs_off = E._lib.CTL_FS_OFF + E._lib.FS_STICKY_OFF
-        fs_sticky = ws.ctl_host[fs_off:fs_off + 4].view(torch.int32)[0].item() | \
-            ws.ctl_host[fs_off + E._lib.FS_STATE_BYTES:fs_off + E._lib.FS_STATE_BYTES + 4].view(torch.int32)[0].item()
-        if (int(sel32[11]) | int(sel32[16 + 11]) | int(fs_sticky)) != 0:
+        if ws.select_sticky() != 0:
             # the sampled window of a fast order-statistic select missed (or its candidate buffer
             # overflowed): the thresholds are NaN.  Redo this tensor with the exhaustive select.
             if safe_select:
