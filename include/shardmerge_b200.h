@@ -48,7 +48,7 @@ void sm_plan_destroy(sm_plan* plan);
 int sm_plan_pitch(const sm_plan* plan);                 /* P, in floats                       */
 int sm_plan_row_freq(const sm_plan* plan, int stored);  /* stored row -> frequency index      */
 int sm_plan_col_passes(const sm_plan* plan);            /* column sweeps per transform: 0, 1, 2 */
-int sm_plan_col_launches(const sm_plan* plan);          /* kernel launches per column transform (column bands x sweeps) */
+int sm_plan_col_launches(const sm_plan* plan);          /* kernel launches per column transform (one per sweep) */
 int sm_plan_describe(const sm_plan* plan, char* buf, int buflen);   /* human-readable factorisation */
 size_t sm_plan_table_bytes(const sm_plan* plan);        /* device bytes for the twiddle tables */
 /* Fill the caller's table buffer (twiddles computed on the device in fp64, stored fp32). */

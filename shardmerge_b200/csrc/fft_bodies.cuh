@@ -266,7 +266,6 @@ struct ColArgs {
   const float* scale_ptr; float scale_host; int use_scale;   // outputs *= scale (last forward sweep)
   int write_im;                // 0: do not store the imaginary plane
   const int* wsel; int wskip;  // nullable: forward, do not store the imaginary plane if (*wsel != 0) == (wskip != 0)
-  int tile0;                   // first column tile of this launch (column bands, kernels_fft.cu: col_band_tiles)
 };
 
 struct ColGlobalSrc {
@@ -300,7 +299,7 @@ template <class Exec>
 SM_HD void col_body(Exec& ex, const SmPlan& pl, int tile, int inst, const ColArgs& a, const cf* twR, cf* smem) {
   const int T = ex.nthreads(), nwarps = T / 32;
   const int L = a.L;
-  const int col0 = (tile + a.tile0) * SM_COL_TILE;
+  const int col0 = tile * SM_COL_TILE;
   int s = 1, cur = 0;
   for (int st = 0; st < a.n_rad; ++st) {
     const int r = a.rad[st], nb = L / r;
@@ -375,91 +374,17 @@ struct ColCtArgs {
   int write_p1_fwd;            // forward: 0 -> do not store the imaginary plane
   const int* wsel; int wskip;  // nullable: forward, do not store the imaginary plane if (*wsel != 0) == (wskip != 0)
                                // (the fused chain: the model that ends up in role v1 only contributes Re, functions.py:108-136)
-  int tile0;                   // first column tile of this launch (column bands)
 };
 #define SM_COL_WRITE_P1(a) ((a).write_p1_fwd != 0 && !((a).wsel != nullptr && (*(a).wsel != 0) == ((a).wskip != 0)))
 
-template <bool kInverse>
-struct ColCtSrc {
-  const float* p0; const float* p1; size_t row0; size_t estride; bool valid; float thr;
-  SM_HD void load(int i, float& a, float& b) const {
-    a = 0.f; b = 0.f;
-    if (valid) {
-      const size_t off = row0 + (size_t)i * estride;
-      a = ldcg_f32(p0 + off); b = ldcg_f32(p1 + off);
-      if (kInverse) { if (b < thr && -b < thr) b = 0.f; }   // p1 is the real plane in the inverse
-    }
-  }
-};
-template <bool kBigTw>
-struct ColCtDst {
-  float* p0; float* p1; size_t row0; size_t estride; bool valid; const cf* twR; int inst; float scale; bool write_p1;
-  SM_HD void store(int k, float a, float b) const {
-    if (kBigTw) { if (inst != 0) { const cf w = twR[(size_t)inst * k]; cmul(a, b, w.x, w.y); } }
-    if (!valid) return;
-    const size_t off = row0 + (size_t)k * estride;
-    p0[off] = a * scale;
-    if (write_p1) p1[off] = b * scale;
-  }
-};
-
-// one CTA (NW warps) = one instance x 32 columns, L = R1*R2 (R2 == 1: single register stage)
-template <int R1, int R2, int NW, bool kInverse, bool kBigTw, class Exec>
-SM_HD void col_ct_body(Exec& ex, int tile, int inst, const ColCtArgs a, const cf* twR, cf* smem) {
-  constexpr int L = R1 * R2;
-  const int col0 = (tile + a.tile0) * SM_COL_TILE;
-  SM_FOR_THREADS(ex, tid) {
-    const int lane = tid & 31, wid = tid >> 5;
-    const int c = col0 + lane;
-    const bool valid = (c <= a.Ch);
-    const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
-    const size_t estride = (size_t)a.elem_mul * a.P;
-    const float thr = (kInverse && a.thr_ptr) ? *a.thr_ptr : 0.f;
-    const float scale = a.scale_ptr ? *a.scale_ptr : a.scale;
-    float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
-    ColCtSrc<kInverse> gsrc{p0, a.p1, row0, estride, valid, thr};
-    ColCtDst<kBigTw> gdst{p0, a.p1, row0, estride, valid, twR, inst, scale, kInverse ? true : SM_COL_WRITE_P1(a)};
-    if constexpr (R2 == 1) {
-      for (int b = wid; b < 1; b += NW) stockham_bfly<R1, true>(b, L, 1, a.tw_mul, twR, gsrc, gdst);
-    } else {
-      ColSmem sout{smem, lane};
-#pragma unroll
-      for (int b = wid; b < R2; b += NW) stockham_bfly<R1, false>(b, L, 1, a.tw_mul, twR, gsrc, sout);
-    }
-  }
-  if constexpr (R2 > 1) {
-    ex.sync();
-    SM_FOR_THREADS(ex, tid) {
-      const int lane = tid & 31, wid = tid >> 5;
-      const int c = col0 + lane;
-      const bool valid = (c <= a.Ch);
-      const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
-      const size_t estride = (size_t)a.elem_mul * a.P;
-      const float scale = a.scale_ptr ? *a.scale_ptr : a.scale;
-      float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
-      ColCtDst<kBigTw> gdst{p0, a.p1, row0, estride, valid, twR, inst, scale, kInverse ? true : SM_COL_WRITE_P1(a)};
-      ColSmem sin{smem, lane};
-#pragma unroll
-      for (int b = wid; b < R1; b += NW) stockham_bfly<R2, true>(b, L, R1, a.tw_mul, twR, sin, gdst);
-    }
-  }
-}
-
 // ------------------------------------------------------------------ paired-column sweeps (pf: two adjacent columns per thread)
-// Same transform as col_ct_body, but every thread carries columns (c, c+1) through the butterflies as one
-// packed value: half the FP / load-store / index instructions per element, 8-byte global accesses, 16-byte
+// Every thread carries two adjacent columns (c, c+1) through the butterflies as one packed value: half the FP /
+// load-store / index instructions per element of one column per thread, 8-byte global accesses, 16-byte
 // shared-memory accesses.  Lane mapping: 16 lanes x 2 columns = one 32-column tile row (128 B), two butterfly
 // slots per warp.  The pair (Ch, Ch+1) touches one zero-filled padding column, whose transform is zero again.
-#ifndef SM_COL_LD_EF
-#define SM_COL_LD_EF 0     // 1: the column sweeps' loads are streaming loads (ld.global.cs, evict-first; experiment: keep a sweep's OUTPUT in L2 for the next)
-#endif
 SM_HD pf ldcg_pf(const float* p) {
 #if defined(__CUDA_ARCH__)
-#if SM_COL_LD_EF
-  const float2 v = __ldcs(reinterpret_cast<const float2*>(p));     // ld.global.cs: evict-first in L1 and L2
-#else
   const float2 v = __ldcg(reinterpret_cast<const float2*>(p));
-#endif
   return pf_make(v.x, v.y);
 #else
   return pf_make(p[0], p[1]);
@@ -497,29 +422,6 @@ struct ColCtSrcP {
     }
   }
 };
-// first-stage source of the bulk-copy fed sweeps (kernels_fft.cu: k_col_pb): one instance x 32 columns of both planes staged
-// in shared memory as [element][32 floats]; the padding columns behind Ch are zero in the planes themselves
-SM_HD pf lds_pf(const float* p) {
-#if defined(__CUDA_ARCH__)
-  const float2 v = *reinterpret_cast<const float2*>(p);
-  return pf_make(v.x, v.y);
-#else
-  return pf_make(p[0], p[1]);
-#endif
-}
-template <bool kInverse>
-struct ColStagedSrcP {
-  const float* s0; const float* s1; int lane; float thr;
-  SM_HD void load(int i, pf& a, pf& b) const {
-    a = lds_pf(s0 + i * SM_COL_TILE + 2 * lane); b = lds_pf(s1 + i * SM_COL_TILE + 2 * lane);
-    if (kInverse) {                                        // p1 is the real plane in the inverse: cull on load
-      float b0 = pf_lo(b), b1 = pf_hi(b);
-      if (b0 < thr && -b0 < thr) b0 = 0.f;
-      if (b1 < thr && -b1 < thr) b1 = 0.f;
-      b = pf_make(b0, b1);
-    }
-  }
-};
 template <bool kBigTw>
 struct ColCtDstP {
   float* p0; float* p1; size_t row0; size_t estride; bool valid; const cf* twR; int inst; float scale; bool write_p1;
@@ -533,42 +435,37 @@ struct ColCtDstP {
 };
 
 // one CTA (NW warps = 2*NW butterfly slots) = one instance x 32 columns, L = R1*R2
-template <int R1, int R2, int NW, bool kInverse, bool kBigTw, class Exec, bool kStaged = false>
-SM_HD void col_ct_body_p(Exec& ex, int tile, int inst, const ColCtArgs a, const cf* twR, pf4* smem,
-                         const float* st0 = nullptr, const float* st1 = nullptr) {
+template <int R1, int R2, int NW, bool kInverse, bool kBigTw, class Exec>
+SM_HD void col_ct_body_p(Exec& ex, int tile, int inst, const ColCtArgs a, const cf* twR, pf4* smem) {
   constexpr int L = R1 * R2;
   constexpr int NS = 2 * NW;
-  const int col0 = (tile + a.tile0) * SM_COL_TILE;
+  const size_t col0 = (size_t)tile * SM_COL_TILE;
   SM_FOR_THREADS(ex, tid) {
     const int lane = tid & 15, slot = tid >> 4;
-    const int c = col0 + 2 * lane;
-    const bool valid = (c <= a.Ch);
-    const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
+    const size_t c = col0 + 2 * lane;
+    const bool valid = (c <= (size_t)a.Ch);
+    const size_t row0 = (size_t)(inst * a.inst_mul) * a.P + c;
     const size_t estride = (size_t)a.elem_mul * a.P;
     const float thr = (kInverse && a.thr_ptr) ? *a.thr_ptr : 0.f;
     const float scale = a.scale_ptr ? *a.scale_ptr : a.scale;
     float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
     ColCtSrcP<kInverse> gsrc{p0, a.p1, row0, estride, valid, thr};
-    ColStagedSrcP<kInverse> ssrc{st0, st1, lane, thr};
     ColCtDstP<kBigTw> gdst{p0, a.p1, row0, estride, valid, twR, inst, scale, kInverse ? true : SM_COL_WRITE_P1(a)};
     if constexpr (R2 == 1) {
       for (int b = slot; b < 1; b += NS) stockham_bfly<R1, true, pf>(b, L, 1, a.tw_mul, twR, gsrc, gdst);
     } else {
       ColSmemP sout{smem, lane};
 #pragma unroll
-      for (int b = slot; b < R2; b += NS) {
-        if constexpr (kStaged) stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, ssrc, sout);
-        else stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, gsrc, sout);
-      }
+      for (int b = slot; b < R2; b += NS) stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, gsrc, sout);
     }
   }
   if constexpr (R2 > 1) {
     ex.sync();
     SM_FOR_THREADS(ex, tid) {
       const int lane = tid & 15, slot = tid >> 4;
-      const int c = col0 + 2 * lane;
-      const bool valid = (c <= a.Ch);
-      const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
+      const size_t c = col0 + 2 * lane;
+      const bool valid = (c <= (size_t)a.Ch);
+      const size_t row0 = (size_t)(inst * a.inst_mul) * a.P + c;
       const size_t estride = (size_t)a.elem_mul * a.P;
       const float scale = a.scale_ptr ? *a.scale_ptr : a.scale;
       float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
@@ -583,30 +480,25 @@ SM_HD void col_ct_body_p(Exec& ex, int tile, int inst, const ColCtArgs a, const 
 // three register stages (radices <= 8) with the middle one in place: the two-stage sweeps of the long instances (L = 112 /
 // 128) need a radix-16 butterfly of packed values, 80 registers, 6 CTAs per SM; radices <= 8 need ~56 (the L = 64 sweeps
 // run at 6.0 TB/s with 9-10 CTAs per SM against 4.8 TB/s, profiles/r01).  L = R1*R2*R3, L / R1 <= 2 NW and L / R2 <= 2 NW.
-template <int R1, int R2, int R3, int NW, bool kInverse, bool kBigTw, class Exec, bool kStaged = false>
-SM_HD void col_ct_body_p3(Exec& ex, int tile, int inst, const ColCtArgs a, const cf* twR, pf4* smem,
-                          const float* st0 = nullptr, const float* st1 = nullptr) {
+template <int R1, int R2, int R3, int NW, bool kInverse, bool kBigTw, class Exec>
+SM_HD void col_ct_body_p3(Exec& ex, int tile, int inst, const ColCtArgs a, const cf* twR, pf4* smem) {
   constexpr int L = R1 * R2 * R3;
   constexpr int NS = 2 * NW;
   static_assert(L / R2 <= NS, "col_ct_body_p3: at most one middle-stage butterfly per slot (it runs in place)");
-  const int col0 = (tile + a.tile0) * SM_COL_TILE;
+  const size_t col0 = (size_t)tile * SM_COL_TILE;
   pf re2[R2], im2[R2];
   SM_FOR_THREADS(ex, tid) {
     const int lane = tid & 15, slot = tid >> 4;
-    const int c = col0 + 2 * lane;
-    const bool valid = (c <= a.Ch);
-    const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
+    const size_t c = col0 + 2 * lane;
+    const bool valid = (c <= (size_t)a.Ch);
+    const size_t row0 = (size_t)(inst * a.inst_mul) * a.P + c;
     const size_t estride = (size_t)a.elem_mul * a.P;
     const float thr = (kInverse && a.thr_ptr) ? *a.thr_ptr : 0.f;
     float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
     ColCtSrcP<kInverse> gsrc{p0, a.p1, row0, estride, valid, thr};
-    ColStagedSrcP<kInverse> ssrc{st0, st1, lane, thr};
     ColSmemP sm{smem, lane};
 #pragma unroll
-    for (int b = slot; b < L / R1; b += NS) {
-      if constexpr (kStaged) stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, ssrc, sm);
-      else stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, gsrc, sm);
-    }
+    for (int b = slot; b < L / R1; b += NS) stockham_bfly<R1, false, pf>(b, L, 1, a.tw_mul, twR, gsrc, sm);
   }
   ex.sync();
   SM_FOR_THREADS(ex, tid) {
@@ -638,9 +530,9 @@ SM_HD void col_ct_body_p3(Exec& ex, int tile, int inst, const ColCtArgs a, const
   ex.sync();
   SM_FOR_THREADS(ex, tid) {
     const int lane = tid & 15, slot = tid >> 4;
-    const int c = col0 + 2 * lane;
-    const bool valid = (c <= a.Ch);
-    const size_t row0 = (size_t)inst * a.inst_mul * a.P + c;
+    const size_t c = col0 + 2 * lane;
+    const bool valid = (c <= (size_t)a.Ch);
+    const size_t row0 = (size_t)(inst * a.inst_mul) * a.P + c;
     const size_t estride = (size_t)a.elem_mul * a.P;
     const float scale = a.scale_ptr ? *a.scale_ptr : a.scale;
     float* const p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;

@@ -4,9 +4,7 @@
 // The arithmetic lives in fft_bodies.cuh (host/device); this file supplies the device
 // execution policy, the launch geometry and the reductions that need CUDA intrinsics.
 #include <cstdarg>
-#include <cstdlib>
 #include <mutex>
-#include <cuda.h>            // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 #include "fft_bodies.cuh"
 #include "sm_internal.h"
 
@@ -70,14 +68,7 @@ __global__ void __launch_bounds__(512) k_col(const __grid_constant__ SmPlan pl, 
 }
 
 // ---- compile-time specialised kernels for the hot shapes (Llama / TinyLlama factorizations)
-template <int R1, int R2, int NW, bool kInverse, bool kBigTw>
-__global__ void __launch_bounds__(NW * 32, (R1 >= 11 || R2 >= 11) ? 3 : 4) k_col_ct(const ColCtArgs a, const cf* __restrict__ twR) {
-  sm_pdl_enter();
-  DeviceExec ex;
-  col_ct_body<R1, R2, NW, kInverse, kBigTw>(ex, (int)blockIdx.x, (int)blockIdx.y, a, twR, reinterpret_cast<cf*>(g_dyn_smem));
-}
-
-// paired-column variant (two adjacent columns per thread, packed f32x2 arithmetic); capping registers for a 7th
+// paired columns (two adjacent columns per thread, packed f32x2 arithmetic); capping registers for a 7th
 // resident CTA was measured slower (spills), so the compiler's own allocation (<= 80 registers) stands
 template <int R1, int R2, int NW, bool kInverse, bool kBigTw>
 __global__ void __launch_bounds__(NW * 32) k_col_p(const __grid_constant__ ColCtArgs a, const cf* __restrict__ twR) {
@@ -93,7 +84,7 @@ __global__ void __launch_bounds__(NW * 32) k_col_p3(const __grid_constant__ ColC
   col_ct_body_p3<R1, R2, R3, NW, kInverse, kBigTw>(ex, (int)blockIdx.x, (int)blockIdx.y, a, twR, reinterpret_cast<pf4*>(g_dyn_smem));
 }
 
-// ---- mbarrier / bulk-copy primitives (cp.async.bulk, the 1-D TMA path) used by the bulk-copy fed kernels below ----
+// ---- mbarrier / bulk-copy primitives (cp.async.bulk, the 1-D TMA path) used by the bulk-copy fed row kernels below ----
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
@@ -115,124 +106,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                  : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
   } while (!ok);
-}
-
-
-// ---- column sweeps fed by the bulk-copy engine (persistent) ---------------------------------------------------------
-// k_col_p / k_col_p3 above spend most of their stall cycles waiting for the global loads of their first stage
-// (long_scoreboard 5 - 8 of ~13 stall cycles per issue, profiles/r01 and r02): a CTA lives for one instance x 32 columns
-// and the loads of the next CTA start only when a slot frees up.  Here a CTA is persistent over the (tile, instance)
-// items, and the 2 L row segments (128 bytes each) of its NEXT item are copied global -> shared by cp.async.bulk into
-// one of two staging buffers while it transforms the current one; the first stage reads the staged planes, everything
-// after it is the body of k_col_p / k_col_p3.  No thread waits on a global load.  R3 == 1 selects the two-stage body.
-// use == 1: the staging copies are TWO tensor-map TMA loads per item (cp.async.bulk.tensor.3d, one box of L rows x 32 columns
-// per plane) instead of 2 L bulk copies of 128 bytes.  The maps describe a plane as (column, b, a) with row = a * Rb + b.
-struct ColMaps { CUtensorMap p0, p0_alt, p1; int use; };
-
-__device__ __forceinline__ void tma_load_3d(void* dst_smem, const CUtensorMap* map, int c0, int c1, int c2, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-               ::"r"(smem_u32(dst_smem)), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)) : "memory");
-}
-
-template <int R1, int R2, int R3, int NW, bool kInverse, bool kBigTw>
-__global__ void __launch_bounds__(NW * 32) k_col_pb(const __grid_constant__ ColCtArgs a, const cf* __restrict__ twR, int ntiles,
-                                                    int n_items, const __grid_constant__ ColMaps maps) {
-  constexpr int L = R1 * R2 * R3;
-  constexpr int T = NW * 32;
-  constexpr int kPlane = L * SM_COL_TILE;                 // floats per staged plane
-  DeviceExec ex;
-  __shared__ uint64_t bar[2];
-  pf4* work = reinterpret_cast<pf4*>(g_dyn_smem);                              // L x 16 pf4 = L x 256 bytes
-  float* stage = reinterpret_cast<float*>(g_dyn_smem) + (size_t)L * 64;        // 2 buffers x 2 planes x L x 32 floats
-  const int tid = threadIdx.x;
-  if (tid == 0) { mbar_init(&bar[0], 1); mbar_init(&bar[1], 1); mbar_fence_init(); }
-  __syncthreads();
-  const float* p0 = (a.sel != nullptr && *a.sel != 0) ? a.p0_alt : a.p0;
-  const float* p1 = a.p1;
-  auto issue = [&](int item, int buf) {
-    const int inst = item / ntiles, tile = item - inst * ntiles;
-    if (tid == 0) mbar_expect_tx(&bar[buf], 2u * (uint32_t)L * 128u);
-    float* dst = stage + (size_t)buf * 2 * kPlane;
-    const size_t col = (size_t)(tile + a.tile0) * SM_COL_TILE;
-    if (maps.use) {
-      if (tid == 0) {
-        const bool alt = (a.sel != nullptr && *a.sel != 0);
-        const int cb = a.elem_mul == 1 ? 0 : inst, ca = a.elem_mul == 1 ? inst : 0;     // sweep B / single sweep : sweep A
-        tma_load_3d(dst, alt ? &maps.p0_alt : &maps.p0, (int)col, cb, ca, &bar[buf]);
-        tma_load_3d(dst + kPlane, &maps.p1, (int)col, cb, ca, &bar[buf]);
-      }
-      return;
-    }
-    for (int i = tid; i < 2 * L; i += T) {
-      const int pl = i >= L ? 1 : 0, e = i - pl * L;
-      const float* src = (pl ? p1 : p0) + ((size_t)inst * a.inst_mul + (size_t)e * a.elem_mul) * a.P + col;
-      bulk_g2s(dst + (size_t)pl * kPlane + (size_t)e * SM_COL_TILE, src, 128u, &bar[buf]);
-    }
-  };
-  int item = (int)blockIdx.x, n = 0;
-  if (item < n_items) issue(item, 0);
-  for (; item < n_items; item += (int)gridDim.x, ++n) {
-    const int buf = n & 1;
-    const int next = item + (int)gridDim.x;
-    if (next < n_items) issue(next, buf ^ 1);            // that buffer was last read before the barrier that ended item n - 1
-    mbar_wait(&bar[buf], (uint32_t)(n >> 1) & 1u);
-    const int inst = item / ntiles, tile = item - inst * ntiles;
-    const float* s0 = stage + (size_t)buf * 2 * kPlane;
-    if constexpr (R3 == 1) col_ct_body_p<R1, R2, NW, kInverse, kBigTw, DeviceExec, true>(ex, tile, inst, a, twR, work, s0, s0 + kPlane);
-    else col_ct_body_p3<R1, R2, R3, NW, kInverse, kBigTw, DeviceExec, true>(ex, tile, inst, a, twR, work, s0, s0 + kPlane);
-    __syncthreads();                                     // the work buffer and this staging buffer are free again
-  }
-}
-
-// ---- both column sweeps of a four-step transform in ONE launch, the second one fed from L2 ----------------
-// A separate launch per sweep streams the whole spectrum through DRAM twice (16N bytes per transform).  Here the
-// CTAs of both sweeps share one 1-D grid, ordered so that the second-sweep CTAs of column tile t are dispatched
-// `lag` tiles after its first-sweep CTAs: by then those have finished (a per-tile counter makes that a guarantee,
-// not an assumption), and the tile's R x 32 complex values -- a few MB times `lag` -- are still in the 126 MB L2.
-// Block order is the dependency order, so a waiting CTA only ever waits for CTAs that were dispatched before it.
-struct Col2Sched { int ntiles, n1, n2, lag; unsigned int* cnt; unsigned int* done; };
-
-__device__ __forceinline__ void col2_decode(const Col2Sched& s, unsigned int b, int* phase, int* tile, int* inst) {
-  const unsigned int head = (unsigned int)s.lag * s.n1;
-  if (b < head) { *phase = 0; *tile = b / s.n1; *inst = b % s.n1; return; }
-  b -= head;
-  const unsigned int per = s.n1 + s.n2, mid = (unsigned int)(s.ntiles - s.lag) * per;
-  if (b < mid) {
-    const unsigned int g = b / per, r = b % per;
-    if (r < (unsigned int)s.n1) { *phase = 0; *tile = s.lag + g; *inst = r; }
-    else { *phase = 1; *tile = g; *inst = r - s.n1; }
-    return;
-  }
-  b -= mid;
-  *phase = 1; *tile = (s.ntiles - s.lag) + b / s.n2; *inst = b % s.n2;
-}
-
-// P = first sweep (R1 x R2), Q = second sweep (S1 x S2); forward: P has the inter-sweep twiddle, inverse: P has it too
-// (the inverse undoes sweep B first, which carries the big twiddle there -- fft_bodies.cuh: sm_col_args)
-template <int R1, int R2, int S1, int S2, int NW, bool kInverse>
-__global__ void __launch_bounds__(NW * 32, (R1 >= 11 || R2 >= 11 || S1 >= 11 || S2 >= 11) ? 3 : 4)
-k_col2_ct(const __grid_constant__ ColCtArgs a1, const __grid_constant__ ColCtArgs a2, const __grid_constant__ Col2Sched s,
-          const cf* __restrict__ twR) {
-  sm_pdl_enter();
-  DeviceExec ex;
-  int phase, tile, inst;
-  col2_decode(s, blockIdx.x, &phase, &tile, &inst);
-  cf* smem = reinterpret_cast<cf*>(g_dyn_smem);
-  if (phase == 0) {
-    col_ct_body<R1, R2, NW, kInverse, true>(ex, tile, inst, a1, twR, smem);
-    __syncthreads();
-    if (threadIdx.x == 0) { __threadfence(); atomicAdd(s.cnt + tile, 1u); }
-  } else {
-    if (threadIdx.x == 0) {
-      while (*((volatile unsigned int*)(s.cnt + tile)) < (unsigned int)s.n1) __nanosleep(64);
-      __threadfence();
-    }
-    __syncthreads();
-    col_ct_body<S1, S2, NW, kInverse, false>(ex, tile, inst, a2, twR, smem);
-    if (threadIdx.x == 0) {                      // the last second-sweep CTA of the tile re-arms its counters
-      if (atomicAdd(s.done + tile, 1u) == (unsigned int)s.n2 - 1u) { s.cnt[tile] = 0u; s.done[tile] = 0u; }
-    }
-  }
 }
 
 template <int R1, int R2, int R3, int R4, int T, bool kPad>
@@ -607,13 +480,11 @@ __global__ void __launch_bounds__(T, 3) k_row2_fwd(int R, int C, int P, const __
   }
 }
 
-// ---- paired-row forward pass, four stages (C = 14336: Ch = 7 x 16 x 8 x 8, T = 448) --------------------------------
-// Same idea as k_row2_fwd for rows whose packed pair no longer leaves room for a staging buffer: the work buffer alone
-// is Ch x 16 B = 112 KB (one CTA per SM).  Stage 1 therefore reads the bf16 rows straight from global memory -- 28
-// independent 4-byte loads per butterfly, ~50 KB in flight per SM -- and one thread asks the copy engine to pull the
-// NEXT pair's rows into L2 (cp.async.bulk.prefetch.L2) so those loads are L2 hits issued behind this pair's compute.
-// Stages 2 and 3 run in place, stage 4 forms the half spectrum in registers (butterflies t and S - t).  The one-row
-// kernel k_row_fwd_tma<7,16,8,8,448> executes 2.3x the instructions per element (profiles/r01_ncu_full_rows7_*).
+// ---- paired-row forward pass, four stages (C = 2048: Ch = 8 x 8 x 4 x 4, T = 128) ----------------------------------
+// Same idea as k_row2_fwd without a staging buffer: stage 1 reads the bf16 rows straight from global memory, and one
+// thread asks the copy engine to pull the NEXT pair's rows into L2 (cp.async.bulk.prefetch.L2) so those loads are L2
+// hits issued behind this pair's compute.  Stages 2 and 3 run in place, stage 4 forms the half spectrum in registers
+// (butterflies t and S - t).  The work buffer is padded (RowSmem2X<true>).
 __device__ __forceinline__ void bulk_prefetch_l2(const void* src_gmem, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src_gmem), "r"(bytes) : "memory");
 }
@@ -645,7 +516,7 @@ struct RowDeltaGlobal2 {         // stage-1 source: bf16 words of both rows stra
   }
 };
 
-template <int R1, int R2, int R3, int R4, int T, bool kPad, int kCtas>
+template <int R1, int R2, int R3, int R4, int T, int kCtas>
 __global__ void __launch_bounds__(T, kCtas) k_row2_fwd4(int R, int C, int P, const __grid_constant__ RowFwdArgs a,
                                                     const cf* __restrict__ twC, const cf* __restrict__ twQ,
                                                     double* __restrict__ sumsq) {
@@ -656,7 +527,7 @@ __global__ void __launch_bounds__(T, kCtas) k_row2_fwd4(int R, int C, int P, con
   constexpr int H2 = NB2 / T;
   static_assert(NB2 == H2 * T && H2 >= 1 && H2 <= 2 && NB3 == 2 * T && S4 == 2 * T, "k_row2_fwd4: 1-2 / 2 / 2 butterflies per thread in stages 2 / 3 / 4");
   __shared__ double wsum[16];
-  RowSmem2X<kPad> sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
+  RowSmem2X<true> sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
   const int tid = threadIdx.x;
   const int npairs = R >> 1;
   double accd = 0.0;
@@ -1204,8 +1075,8 @@ __global__ void __launch_bounds__(T, 3) k_row2_inv(int R, int C, int P, const __
   }
 }
 
-// ---- paired-row inverse pass, four stages (C = 14336): the mirror image of k_row2_fwd4 ------------------------------
-// No staging (the work buffer fills the SM): the tangle reads the two spectrum rows straight from global memory, the
+// ---- paired-row inverse pass, four stages (C = 2048): the mirror image of k_row2_fwd4 -------------------------------
+// No staging: the tangle reads the two spectrum rows straight from global memory, the
 // next pair's rows are pulled into L2 by the copy engine in the meantime; stages 2-3 in place; the last stage feeds the
 // epilogue with the bf16 base words loaded ahead of its shared-memory reads.
 struct RowTangleGlobal2 {
@@ -1224,7 +1095,7 @@ struct RowTangleGlobal2 {
   }
 };
 
-template <int R1, int R2, int R3, int R4, int T, bool kPad, int kCtas>
+template <int R1, int R2, int R3, int R4, int T, int kCtas>
 __global__ void __launch_bounds__(T, kCtas) k_row2_inv4(int R, int C, int P, const __grid_constant__ RowInvArgs a,
                                                     const cf* __restrict__ twC, const cf* __restrict__ twQ) {
   sm_pdl_enter();
@@ -1233,7 +1104,7 @@ __global__ void __launch_bounds__(T, kCtas) k_row2_inv4(int R, int C, int P, con
   constexpr int s2 = R1, s3 = R1 * R2;
   constexpr int H2 = NB2 / T;
   static_assert(NB2 == H2 * T && H2 >= 1 && H2 <= 2 && NB3 == 2 * T && S4 == 2 * T, "k_row2_inv4: 1-2 / 2 / 2 butterflies per thread in stages 2 / 3 / 4");
-  RowSmem2X<kPad> sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
+  RowSmem2X<true> sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
   const int tid = threadIdx.x;
   const int npairs = R >> 1;
   const float* im_plane = (a.sel != nullptr && *a.sel != 0) ? a.im_alt : a.im;
@@ -1517,7 +1388,6 @@ __global__ void k_inv_norm(const double* sumsq, float* out) {
 }
 
 // ------------------------------------------------------------------ host side
-static int col_band_tiles(const SmPlan& p);
 static std::once_flag g_attr_once;
 static int g_attr_rc = 0;
 static int ensure_attrs() {
@@ -1555,12 +1425,8 @@ extern "C" sm_plan* sm_plan_create(int R, int C) {
 extern "C" void sm_plan_destroy(sm_plan* plan) { delete plan; }
 extern "C" int sm_plan_pitch(const sm_plan* plan) { return plan->p.P; }
 extern "C" int sm_plan_col_passes(const sm_plan* plan) { return plan->p.col_passes; }
-extern "C" int sm_plan_col_launches(const sm_plan* plan) {     // kernel launches of ONE column transform (bands x sweeps)
-  const SmPlan& p = plan->p;
-  if (p.col_passes == 0) return 1;
-  if (p.col_passes == 1) return 1;
-  const int ntiles = sm_col_tiles(p), band = col_band_tiles(p);
-  return 2 * ((ntiles + band - 1) / band);
+extern "C" int sm_plan_col_launches(const sm_plan* plan) {     // kernel launches of ONE column transform (one per sweep)
+  return plan->p.col_passes == 2 ? 2 : 1;
 }
 extern "C" int sm_plan_row_freq(const sm_plan* plan, int stored) { return sm_row_freq(&plan->p, stored); }
 extern "C" size_t sm_plan_table_bytes(const sm_plan* plan) {
@@ -1595,7 +1461,6 @@ extern "C" int sm_plan_init_tables(const sm_plan* plan, void* tables, void* stre
     k_init_quads<<<(4 * nq + 255) / 256, 256, 0, st>>>(twQ, nq, p.Ch);
     SM_LAUNCH_CHECK();
   }
-  SM_CUDA_CHECK(cudaMemsetAsync(reinterpret_cast<char*>(tables) + sm_tab_off_K(p), 0, 8 * (size_t)sm_col_tiles(p), st));
   return 0;
 }
 
@@ -1628,29 +1493,7 @@ static cudaError_t opt_in(K kernel, bool* done) {
 }
 
 template <int R1, int R2, int NW>
-static int launch_col_ct_pair(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a, const cf* twR, cudaStream_t st) {
-  static bool done[4] = {false, false, false, false};
-  const int smem = (R2 > 1) ? R1 * R2 * SM_COL_TILE * 8 : 0;
-  cudaError_t e;
-#define SM_COL_CASE(INV, BIG, IDX)                                                        \
-  e = opt_in(k_col_ct<R1, R2, NW, INV, BIG>, &done[IDX]);                                 \
-  if (e != cudaSuccess) { sm_set_error("opt_in: %s", cudaGetErrorString(e)); return -100; } \
-  sm_launch(k_col_ct<R1, R2, NW, INV, BIG>, dim3(grid), dim3(NW * 32), (size_t)(smem), st, a, twR);
-  if (!inverse && big_tw) { SM_COL_CASE(false, true, 0) }
-  else if (!inverse) { SM_COL_CASE(false, false, 1) }
-  else if (big_tw) { SM_COL_CASE(true, true, 2) }
-  else { SM_COL_CASE(true, false, 3) }
-#undef SM_COL_CASE
-  SM_LAUNCH_CHECK();
-  return 0;
-}
-
-template <int R1, int R2, int R3, int NW>
-static int launch_col_pb(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a, const cf* twR, cudaStream_t st);
-
-template <int R1, int R2, int NW>
 static int launch_col_p(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a, const cf* twR, cudaStream_t st) {
-  if constexpr (R2 > 1) { const int rc = launch_col_pb<R1, R2, 1, NW>(inverse, big_tw, grid, a, twR, st); if (rc <= 0) return rc; }
   static bool done[4] = {false, false, false, false};
   const int smem = (R2 > 1) ? R1 * R2 * SM_COL_TILE * 8 : 0;
   cudaError_t e;
@@ -1669,7 +1512,6 @@ static int launch_col_p(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a
 
 template <int R1, int R2, int R3, int NW>
 static int launch_col_p3(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a, const cf* twR, cudaStream_t st) {
-  { const int rc = launch_col_pb<R1, R2, R3, NW>(inverse, big_tw, grid, a, twR, st); if (rc <= 0) return rc; }
   static bool done[4] = {false, false, false, false};
   const int smem = R1 * R2 * R3 * SM_COL_TILE * 8;
   cudaError_t e;
@@ -1686,135 +1528,20 @@ static int launch_col_p3(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& 
   return 0;
 }
 
-static int num_sms();
-// SM_COL_BULK=1 selects the persistent, bulk-copy fed sweeps (k_col_pb), SM_COL_BULK=2 the same fed by two tensor-map TMA
-// loads per item.  OFF by default: measured on the Llama-8B-shaped bench (profiles/r02_ab_col_bulk.log) they move 3.5 TB/s
-// (2 L bulk copies of 128 bytes per item) and 4.4 TB/s (tensor maps) against 5.1 TB/s for k_col_p / k_col_p3: the plain-load
-// kernels already keep 5 CTAs x 8 warps x 14 loads in flight per SM, the staging buffers cut the CTAs per SM to 2, and with
-// them the warps that cover the shared-memory latency of the butterflies.  Kept as A-B switches.
-static bool use_col_bulk() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_COL_BULK"); v = (e && (e[0] == '1' || e[0] == '2')) ? 1 : 0; }
-  return v != 0;
-}
-
-// SM_COL_BULK=2: the same with tensor-map TMA loads (two per item)
-static int col_bulk_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_COL_BULK"); v = e ? atoi(e) : 0; if (v < 0 || v > 2) v = 0; }
-  return v;
-}
-
-typedef CUresult (*SmEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static SmEncodeTiled tensor_map_encoder() {
-  static SmEncodeTiled fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    cudaDriverEntryPointQueryResult q;
-    void* p = nullptr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<SmEncodeTiled>(p);
-  }
-  return fn;
-}
-// plane [R][P] seen as (column, b, a) with row = a * Rb + b; box = 32 columns x (bb x ba) rows
-static bool make_col_map(CUtensorMap* m, const float* plane, int P, int Ra, int Rb, int bb, int ba) {
-  SmEncodeTiled enc = tensor_map_encoder();
-  if (!enc || plane == nullptr) return false;
-  cuuint64_t dims[3] = {(cuuint64_t)P, (cuuint64_t)Rb, (cuuint64_t)Ra};
-  cuuint64_t strides[2] = {(cuuint64_t)P * 4, (cuuint64_t)P * 4 * (cuuint64_t)Rb};
-  cuuint32_t box[3] = {SM_COL_TILE, (cuuint32_t)bb, (cuuint32_t)ba};
-  cuuint32_t es[3] = {1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(plane), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// persistent, bulk-copy fed variant of launch_col_p (R3 == 1) / launch_col_p3; returns 1 if it does not apply
-template <int R1, int R2, int R3, int NW>
-static int launch_col_pb(bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a, const cf* twR, cudaStream_t st) {
-  constexpr int L = R1 * R2 * R3;
-  constexpr int smem = L * 768;                         // work (L x 256) + two staging buffers of two planes (L x 128 each)
-  if (!use_col_bulk() || smem > 110 * 1024) return 1;
-  ColMaps maps;
-  maps.use = 0;
-  if (col_bulk_mode() == 2 && L <= 256) {
-    // sweep A (element stride Rb rows): box (32, 1, L) over dims (P, Rb, Ra = L); sweep B / single sweep (contiguous rows):
-    // box (32, L, 1) over dims (P, Rb = L, Ra = instances)
-    const bool contiguous = a.elem_mul == 1;
-    const int Rb = contiguous ? L : a.elem_mul, Ra = contiguous ? (int)grid.y : L;
-    const int bb = contiguous ? L : 1, ba = contiguous ? 1 : L;
-    bool ok = make_col_map(&maps.p0, a.p0, a.P, Ra, Rb, bb, ba) && make_col_map(&maps.p1, a.p1, a.P, Ra, Rb, bb, ba);
-    if (ok && a.p0_alt != nullptr) ok = make_col_map(&maps.p0_alt, a.p0_alt, a.P, Ra, Rb, bb, ba);
-    else if (ok) maps.p0_alt = maps.p0;
-    maps.use = ok ? 1 : 0;
-  }
-  static bool done[4] = {false, false, false, false};
-  static int occ[4] = {0, 0, 0, 0};
-  const int ntiles = (int)grid.x, n_items = (int)(grid.x * grid.y);
-  cudaError_t e;
-#define SM_COLPB_CASE(INV, BIG, IDX)                                                                        \
-  e = opt_in(k_col_pb<R1, R2, R3, NW, INV, BIG>, &done[IDX]);                                               \
-  if (e != cudaSuccess) { sm_set_error("opt_in: %s", cudaGetErrorString(e)); return -100; }               \
-  if (occ[IDX] == 0) {                                                                                    \
-    int o = 0;                                                                                            \
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_col_pb<R1, R2, R3, NW, INV, BIG>, NW * 32, smem) != cudaSuccess || o < 1) o = 1; \
-    occ[IDX] = o;                                                                                         \
-  }                                                                                                       \
-  {                                                                                                       \
-    int ctas = num_sms() * occ[IDX];                                                                      \
-    if (ctas > n_items) ctas = n_items;                                                                   \
-    k_col_pb<R1, R2, R3, NW, INV, BIG><<<ctas, NW * 32, smem, st>>>(a, twR, ntiles, n_items, maps);       \
-  }
-  if (!inverse && big_tw) { SM_COLPB_CASE(false, true, 0) }
-  else if (!inverse) { SM_COLPB_CASE(false, false, 1) }
-  else if (big_tw) { SM_COLPB_CASE(true, true, 2) }
-  else { SM_COLPB_CASE(true, false, 3) }
-#undef SM_COLPB_CASE
-  SM_LAUNCH_CHECK();
-  return 0;
-}
-
-static bool use_col_pairs() {       // SM_COL_PAIRS=0: one column per thread (k_col_ct), for A-B timing
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_COL_PAIRS"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-
 static int try_col_p(int n_rad, const int* rad, bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a,
                      const cf* twR, cudaStream_t st) {
-  if (n_rad != 2 || !use_col_pairs()) return 1;
+  if (n_rad != 2) return 1;
   const int r1 = rad[0], r2 = rad[1];
   if (r1 == 8 && r2 == 8) return launch_col_p<8, 8, 4>(inverse, big_tw, grid, a, twR, st);
   // the long instances as three stages of radices <= 8 (~52 registers instead of 80: 32 resident warps per SM instead
   // of 24; measured col_fwd -6 %, col_inv -4 %); a Stockham transform is natural order in / out whatever its radices,
   // so the plan's (16, 8) / (7, 16) split may be re-factored (L = 256 as 8 x 8 x 4 with 512-thread CTAs measured 1 % slower
-  // than its two-stage kernel and is not used).  SM_COL3=0: the two-stage kernels (A-B timing).
-  static int col3 = -1;
-  if (col3 < 0) { const char* e = getenv("SM_COL3"); col3 = (e && e[0] == '0') ? 0 : 1; }
-  if (col3 && r1 == 16 && r2 == 8) return launch_col_p3<8, 8, 2, 8>(inverse, big_tw, grid, a, twR, st);
-  if (col3 && r1 == 7 && r2 == 16) return launch_col_p3<7, 8, 2, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 16 && r2 == 8) return launch_col_p<16, 8, 4>(inverse, big_tw, grid, a, twR, st);
+  // than its two-stage kernel and is not used).
+  if (r1 == 16 && r2 == 8) return launch_col_p3<8, 8, 2, 8>(inverse, big_tw, grid, a, twR, st);
+  if (r1 == 7 && r2 == 16) return launch_col_p3<7, 8, 2, 8>(inverse, big_tw, grid, a, twR, st);
   if (r1 == 16 && r2 == 16) return launch_col_p<16, 16, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 7 && r2 == 16) return launch_col_p<7, 16, 4>(inverse, big_tw, grid, a, twR, st);
   if (r1 == 11 && r2 == 8) return launch_col_p<11, 8, 4>(inverse, big_tw, grid, a, twR, st);
   if (r1 == 8 && r2 == 4) return launch_col_p<8, 4, 2>(inverse, big_tw, grid, a, twR, st);
-  return 1;
-}
-
-// returns 1 if no specialised kernel exists for this factorization
-static int try_col_ct(int n_rad, const int* rad, bool inverse, bool big_tw, dim3 grid, const ColCtArgs& a,
-                      const cf* twR, cudaStream_t st) {
-  if (n_rad != 2) return 1;
-  const int r1 = rad[0], r2 = rad[1];
-  if (r1 == 8 && r2 == 8) return launch_col_ct_pair<8, 8, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 16 && r2 == 8) return launch_col_ct_pair<16, 8, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 16 && r2 == 16) return launch_col_ct_pair<16, 16, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 7 && r2 == 16) return launch_col_ct_pair<7, 16, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 11 && r2 == 8) return launch_col_ct_pair<11, 8, 8>(inverse, big_tw, grid, a, twR, st);
-  if (r1 == 8 && r2 == 4) return launch_col_ct_pair<8, 4, 4>(inverse, big_tw, grid, a, twR, st);
   return 1;
 }
 
@@ -1827,92 +1554,12 @@ static int num_sms() {
   }
   return g_num_sms;
 }
-static bool g_use_tma = true;     // SM_ROW_TMA=0 falls back to the one-CTA-per-row kernels (debug / A-B timing)
-static bool use_tma() {
-  static int init = 0;
-  if (!init) { const char* e = getenv("SM_ROW_TMA"); if (e && e[0] == '0') g_use_tma = false; init = 1; }
-  return g_use_tma;
-}
-
-// Measured (profiles/r01, 4096x4096): the fused launch takes 63 us against 28 + 22 us for two launches -- the
-// sweeps are latency / issue bound, not DRAM bound, and the second launch already reads mostly from L2 -- so it is
-// OFF by default (SM_COL_FUSED=1 enables it for A-B timing).
-static bool g_use_col2 = false;
-static bool use_col2() {
-  static int init = 0;
-  if (!init) { const char* e = getenv("SM_COL_FUSED"); if (e && e[0] == '1') g_use_col2 = true; init = 1; }
-  return g_use_col2;
-}
-
-template <int R1, int R2, int S1, int S2, int NW>
-static int launch_col2(bool inverse, const ColCtArgs& a1, const ColCtArgs& a2, Col2Sched s, const cf* twR, cudaStream_t st) {
-  static bool done[2] = {false, false};
-  static int occ[2] = {0, 0};
-  const int smem1 = (R2 > 1) ? R1 * R2 * SM_COL_TILE * 8 : 0, smem2 = (S2 > 1) ? S1 * S2 * SM_COL_TILE * 8 : 0;
-  const int smem = smem1 > smem2 ? smem1 : smem2;
-  cudaError_t e;
-  const int w = inverse ? 1 : 0;
-  if (!inverse) {
-    e = opt_in(k_col2_ct<R1, R2, S1, S2, NW, false>, &done[0]);
-    if (e == cudaSuccess && occ[0] == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[0], k_col2_ct<R1, R2, S1, S2, NW, false>, NW * 32, smem);
-  } else {
-    e = opt_in(k_col2_ct<R1, R2, S1, S2, NW, true>, &done[1]);
-    if (e == cudaSuccess && occ[1] == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[1], k_col2_ct<R1, R2, S1, S2, NW, true>, NW * 32, smem);
-  }
-  if (e != cudaSuccess) { sm_set_error("col2 setup: %s", cudaGetErrorString(e)); return -100; }
-  const int slots = num_sms() * (occ[w] > 0 ? occ[w] : 1);
-  int lag = (2 * slots + s.n1 - 1) / s.n1 + 1;
-  if (lag < 2) lag = 2;
-  if (lag > s.ntiles) lag = s.ntiles;
-  s.lag = lag;
-  const unsigned int grid = (unsigned int)s.ntiles * (unsigned int)(s.n1 + s.n2);
-  if (!inverse) sm_launch(k_col2_ct<R1, R2, S1, S2, NW, false>, dim3(grid), dim3(NW * 32), (size_t)(smem), st, a1, a2, s, twR);
-  else sm_launch(k_col2_ct<R1, R2, S1, S2, NW, true>, dim3(grid), dim3(NW * 32), (size_t)(smem), st, a1, a2, s, twR);
-  SM_LAUNCH_CHECK();
-  return 0;
-}
-
-// returns 1 if the pair of factorizations has no fused kernel
-static int try_col2_ct(const int* p_rad, int p_n, const int* q_rad, int q_n, bool inverse, const ColCtArgs& a1, const ColCtArgs& a2,
-                       const Col2Sched& s, const cf* twR, cudaStream_t st) {
-  if (p_n != 2 || q_n != 2) return 1;
-  const int r1 = p_rad[0], r2 = p_rad[1], s1 = q_rad[0], s2 = q_rad[1];
-#define SM_COL2_CASE(A, B, C_, D)                                                                                   \
-  if (r1 == A && r2 == B && s1 == C_ && s2 == D) return launch_col2<A, B, C_, D, 8>(inverse, a1, a2, s, twR, st);
-  SM_COL2_CASE(8, 8, 8, 8)        // R = 4096
-  SM_COL2_CASE(7, 16, 16, 8)      // R = 14336 forward (112 x 128)
-  SM_COL2_CASE(16, 8, 7, 16)      // R = 14336 inverse
-  SM_COL2_CASE(8, 8, 16, 8)       // R = 8192 (64 x 128)
-  SM_COL2_CASE(16, 8, 8, 8)
-  SM_COL2_CASE(7, 16, 16, 16)     // R = 28672 (112 x 256)
-  SM_COL2_CASE(16, 16, 7, 16)
-  SM_COL2_CASE(11, 8, 8, 8)       // R = 5632 (88 x 64)
-  SM_COL2_CASE(8, 8, 11, 8)
-#undef SM_COL2_CASE
-  return 1;
-}
-
-static bool use_row_pairs() {       // SM_ROW_PAIRS=0: one row per CTA iteration (k_row_fwd_tma), for A-B timing
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_ROW_PAIRS"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-
 // paired-row forward pass (k_row2_fwd); returns 1 if this shape / mode has none
-// SM_ROW2_OCC=n caps the resident CTAs per SM of the persistent paired-row kernels (default: what fits, 3): fewer leave
-// shared memory for another lane's kernels on the same SM (A-B switch)
-static int row2_occ(int occ) {
-  static int cap = -1;
-  if (cap < 0) { const char* e = getenv("SM_ROW2_OCC"); cap = e ? atoi(e) : 0; }
-  if (occ < 1) occ = 1;
-  return (cap > 0 && cap < occ) ? cap : occ;
-}
-
 template <int R1, int R2, int R3, int R4, int T, bool kPad>
 static int try_row2_fwd(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
   if constexpr (R4 == 1 && kPad && (R1 * R2 * R3) / R3 == 2 * T && (R1 * R2 * R3) / R1 == T && (R1 * R2 * R3) / R2 == T) {
     constexpr int CH = R1 * R2 * R3;
-    if (!use_row_pairs() || fa.mode != 0 || (p.R & 1) || p.R < 2 || p.C % 8 != 0) return 1;
+    if (fa.mode != 0 || (p.R & 1) || p.R < 2 || p.C % 8 != 0) return 1;
     static bool done = false;
     static int occ = 0;
     const int work_bytes = ((CH + (CH >> 4) + 1) * 16 + 127) / 128 * 128;
@@ -1921,7 +1568,7 @@ static int try_row2_fwd(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, co
     cudaError_t e = opt_in(k_row2_fwd<R1, R2, R3, T, false>, &done);
     if (e == cudaSuccess && occ == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_row2_fwd<R1, R2, R3, T, false>, T, smem);
     if (e != cudaSuccess) { sm_set_error("row2 setup: %s", cudaGetErrorString(e)); return -100; }
-    int grid = num_sms() * row2_occ(occ);
+    int grid = num_sms() * (occ > 0 ? occ : 1);
     if (grid > p.R / 2) grid = p.R / 2;
     sm_launch(k_row2_fwd<R1, R2, R3, T, false>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes);
     SM_LAUNCH_CHECK();
@@ -1934,51 +1581,43 @@ static int try_row2_fwd(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, co
 // paired-row four-stage passes (k_row2_fwd4 / k_row2_inv4) with their own factorization Ch = R1*R2*R3*R4 (it need not be
 // the plan's: the twiddle tables do not depend on it and the quad table covers first radices down to 8);
 // return 1 if this mode has none
-template <int R1, int R2, int R3, int R4, int T, bool kPad, int kCtas>
+template <int R1, int R2, int R3, int R4, int T, int kCtas>
 static int launch_row2_fwd4(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3 * R4;
-  if (!use_row_pairs() || fa.mode != 0 || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.Ch != CH) return 1;
+  if (fa.mode != 0 || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.Ch != CH) return 1;
   static bool done = false;
-  const int smem = (kPad ? CH + (CH >> 3) + 1 : CH) * 16;
+  const int smem = (CH + (CH >> 3) + 1) * 16;
   if (smem > 227 * 1024 - 256) return 1;
-  cudaError_t e = opt_in(k_row2_fwd4<R1, R2, R3, R4, T, kPad, kCtas>, &done);
+  cudaError_t e = opt_in(k_row2_fwd4<R1, R2, R3, R4, T, kCtas>, &done);
   if (e != cudaSuccess) { sm_set_error("row2 fwd4 setup: %s", cudaGetErrorString(e)); return -100; }
   int grid = num_sms() * kCtas;
   if (grid > p.R / 2) grid = p.R / 2;
-  sm_launch(k_row2_fwd4<R1, R2, R3, R4, T, kPad, kCtas>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq);
+  sm_launch(k_row2_fwd4<R1, R2, R3, R4, T, kCtas>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq);
   SM_LAUNCH_CHECK();
   return 0;
 }
 
-template <int R1, int R2, int R3, int R4, int T, bool kPad, int kCtas>
+template <int R1, int R2, int R3, int R4, int T, int kCtas>
 static int launch_row2_inv4(const SmPlan& p, const RowInvArgs& ia, const cf* twC, const cf* twQ, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3 * R4;
-  if (!use_row_pairs() || ia.cull_thr != nullptr || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0 || p.Ch != CH) return 1;
+  if (ia.cull_thr != nullptr || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0 || p.Ch != CH) return 1;
   static bool done = false;
-  const int smem = (kPad ? CH + (CH >> 3) + 1 : CH) * 16;
+  const int smem = (CH + (CH >> 3) + 1) * 16;
   if (smem > 227 * 1024 - 256) return 1;
-  cudaError_t e = opt_in(k_row2_inv4<R1, R2, R3, R4, T, kPad, kCtas>, &done);
+  cudaError_t e = opt_in(k_row2_inv4<R1, R2, R3, R4, T, kCtas>, &done);
   if (e != cudaSuccess) { sm_set_error("row2 inv4 setup: %s", cudaGetErrorString(e)); return -100; }
   int grid = num_sms() * kCtas;
   if (grid > p.R / 2) grid = p.R / 2;
-  sm_launch(k_row2_inv4<R1, R2, R3, R4, T, kPad, kCtas>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, ia, twC, twQ);
+  sm_launch(k_row2_inv4<R1, R2, R3, R4, T, kCtas>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, ia, twC, twQ);
   SM_LAUNCH_CHECK();
   return 0;
-}
-
-// which four-stage paired kernel serves the plan's row length: C = 14336 as 7 x 16 x 8 x 8 (one CTA of 448 threads per
-// SM), C = 8192 as 8 x 8 x 8 x 8 (two CTAs of 256 threads, padded buffer) whatever the plan's own radices are
-static bool use_row_eo() {          // SM_ROW_EO=0: C = 14336 rows as row pairs (k_row2_*4) instead of even / odd halves, for A-B timing
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_ROW_EO"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
 }
 
 // one row per CTA, lanes = even / odd halves (k_row1_fwd_eo): Ch = 2 * R1*R2*R3*R4
 template <int R1, int R2, int R3, int R4, int T, int kCtas>
 static int launch_row1_fwd_eo(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3 * R4;
-  if (!use_row_pairs() || fa.mode != 0 || p.R < 1 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
+  if (fa.mode != 0 || p.R < 1 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
   static bool done = false;
   const int smem = CH * 16;
   cudaError_t e = opt_in(k_row1_fwd_eo<R1, R2, R3, R4, T, kCtas>, &done);
@@ -1994,7 +1633,7 @@ static int launch_row1_fwd_eo(const SmPlan& p, const RowFwdArgs& fa, const cf* t
 template <int R1, int R2, int R3, int T>
 static int launch_row1_fwd_eo3(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3;
-  if (!use_row_pairs() || fa.mode != 0 || p.R < 2 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
+  if (fa.mode != 0 || p.R < 2 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
   static bool done = false;
   static int occ = 0;
   const int work_bytes = ((CH + (CH >> 4) + 1) * 16 + 127) / 128 * 128;
@@ -2002,7 +1641,7 @@ static int launch_row1_fwd_eo3(const SmPlan& p, const RowFwdArgs& fa, const cf* 
   cudaError_t e = opt_in(k_row2_fwd<R1, R2, R3, T, true>, &done);
   if (e == cudaSuccess && occ == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_row2_fwd<R1, R2, R3, T, true>, T, smem);
   if (e != cudaSuccess) { sm_set_error("row1 fwd eo3 setup: %s", cudaGetErrorString(e)); return -100; }
-  int grid = num_sms() * row2_occ(occ);
+  int grid = num_sms() * (occ > 0 ? occ : 1);
   if (grid > p.R) grid = p.R;
   sm_launch(k_row2_fwd<R1, R2, R3, T, true>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes);
   SM_LAUNCH_CHECK();
@@ -2010,20 +1649,18 @@ static int launch_row1_fwd_eo3(const SmPlan& p, const RowFwdArgs& fa, const cf* 
 }
 
 static int try_row2_fwd4(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
-  if (p.Ch == 4096 && use_row_eo()) return launch_row1_fwd_eo3<16, 16, 8, 128>(p, fa, twC, twQ, sumsq, st);
+  if (p.Ch == 4096) return launch_row1_fwd_eo3<16, 16, 8, 128>(p, fa, twC, twQ, sumsq, st);
   if (p.Ch == 14336) return launch_row1_fwd_eo<7, 16, 8, 8, 448, 1>(p, fa, twC, twQ, sumsq, st);
-  if (p.Ch == 7168 && use_row_eo()) return launch_row1_fwd_eo<7, 8, 8, 8, 224, 2>(p, fa, twC, twQ, sumsq, st);
-  if (p.Ch == 7168) return launch_row2_fwd4<7, 16, 8, 8, 448, false, 1>(p, fa, twC, twQ, sumsq, st);
-  if (p.Ch == 4096) return launch_row2_fwd4<8, 8, 8, 8, 256, true, 2>(p, fa, twC, twQ, sumsq, st);
+  if (p.Ch == 7168) return launch_row1_fwd_eo<7, 8, 8, 8, 224, 2>(p, fa, twC, twQ, sumsq, st);
   // TinyLlama shapes: C = 2048 as row pairs 8 x 8 x 4 x 4, C = 5632 as even / odd halves of 11 x 8 x 4 x 4
-  if (p.Ch == 1024) return launch_row2_fwd4<8, 8, 4, 4, 128, true, 4>(p, fa, twC, twQ, sumsq, st);
+  if (p.Ch == 1024) return launch_row2_fwd4<8, 8, 4, 4, 128, 4>(p, fa, twC, twQ, sumsq, st);
   if (p.Ch == 2816) return launch_row1_fwd_eo<11, 8, 4, 4, 176, 2>(p, fa, twC, twQ, sumsq, st);
   return 1;
 }
 template <int R1, int R2, int R3, int R4, int T, int kCtas>
 static int launch_row1_inv_eo(const SmPlan& p, const RowInvArgs& ia, const cf* twC, const cf* twQ, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3 * R4;
-  if (!use_row_pairs() || ia.cull_thr != nullptr || p.R < 1 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
+  if (ia.cull_thr != nullptr || p.R < 1 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
   static bool done = false;
   const int smem = CH * 16;
   cudaError_t e = opt_in(k_row1_inv_eo<R1, R2, R3, R4, T, kCtas>, &done);
@@ -2038,7 +1675,7 @@ static int launch_row1_inv_eo(const SmPlan& p, const RowInvArgs& ia, const cf* t
 template <int R1, int R2, int R3, int T>
 static int launch_row1_inv_eo3(const SmPlan& p, const RowInvArgs& ia, const cf* twC, const cf* twQ, cudaStream_t st) {
   constexpr int CH = R1 * R2 * R3;
-  if (!use_row_pairs() || ia.cull_thr != nullptr || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0 || p.Ch != 2 * CH) return 1;
+  if (ia.cull_thr != nullptr || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0 || p.Ch != 2 * CH) return 1;
   static bool done = false;
   static int occ = 0;
   const int work_bytes = ((CH + (CH >> 4) + 1) * 16 + 127) / 128 * 128;
@@ -2046,7 +1683,7 @@ static int launch_row1_inv_eo3(const SmPlan& p, const RowInvArgs& ia, const cf* 
   cudaError_t e = opt_in(k_row2_inv<R1, R2, R3, T, true>, &done);
   if (e == cudaSuccess && occ == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_row2_inv<R1, R2, R3, T, true>, T, smem);
   if (e != cudaSuccess) { sm_set_error("row1 inv eo3 setup: %s", cudaGetErrorString(e)); return -100; }
-  int grid = num_sms() * row2_occ(occ);
+  int grid = num_sms() * (occ > 0 ? occ : 1);
   if (grid > p.R) grid = p.R;
   sm_launch(k_row2_inv<R1, R2, R3, T, true>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, ia, twC, twQ, work_bytes);
   SM_LAUNCH_CHECK();
@@ -2054,12 +1691,10 @@ static int launch_row1_inv_eo3(const SmPlan& p, const RowInvArgs& ia, const cf* 
 }
 
 static int try_row2_inv4(const SmPlan& p, const RowInvArgs& ia, const cf* twC, const cf* twQ, cudaStream_t st) {
-  if (p.Ch == 4096 && use_row_eo()) return launch_row1_inv_eo3<16, 16, 8, 128>(p, ia, twC, twQ, st);
+  if (p.Ch == 4096) return launch_row1_inv_eo3<16, 16, 8, 128>(p, ia, twC, twQ, st);
   if (p.Ch == 14336) return launch_row1_inv_eo<7, 16, 8, 8, 448, 1>(p, ia, twC, twQ, st);
-  if (p.Ch == 7168 && use_row_eo()) return launch_row1_inv_eo<7, 8, 8, 8, 224, 2>(p, ia, twC, twQ, st);
-  if (p.Ch == 7168) return launch_row2_inv4<7, 16, 8, 8, 448, false, 1>(p, ia, twC, twQ, st);
-  if (p.Ch == 4096) return launch_row2_inv4<8, 8, 8, 8, 256, true, 2>(p, ia, twC, twQ, st);
-  if (p.Ch == 1024) return launch_row2_inv4<8, 8, 4, 4, 128, true, 4>(p, ia, twC, twQ, st);
+  if (p.Ch == 7168) return launch_row1_inv_eo<7, 8, 8, 8, 224, 2>(p, ia, twC, twQ, st);
+  if (p.Ch == 1024) return launch_row2_inv4<8, 8, 4, 4, 128, 4>(p, ia, twC, twQ, st);
   if (p.Ch == 2816) return launch_row1_inv_eo<11, 8, 4, 4, 176, 2>(p, ia, twC, twQ, st);
   return 1;
 }
@@ -2069,7 +1704,7 @@ template <int R1, int R2, int R3, int R4, int T, bool kPad>
 static int try_row2_inv(const SmPlan& p, const RowInvArgs& ia, const cf* twC, const cf* twQ, cudaStream_t st) {
   if constexpr (R4 == 1 && kPad && (R1 * R2 * R3) / R3 == 2 * T && (R1 * R2 * R3) / R1 == T && (R1 * R2 * R3) / R2 == T) {
     constexpr int CH = R1 * R2 * R3;
-    if (!use_row_pairs() || ia.cull_thr != nullptr || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0) return 1;
+    if (ia.cull_thr != nullptr || (p.R & 1) || p.R < 2 || p.C % 8 != 0 || p.P % 4 != 0) return 1;
     static bool done = false;
     static int occ = 0;
     const int work_bytes = ((CH + (CH >> 4) + 1) * 16 + 127) / 128 * 128;
@@ -2078,7 +1713,7 @@ static int try_row2_inv(const SmPlan& p, const RowInvArgs& ia, const cf* twC, co
     cudaError_t e = opt_in(k_row2_inv<R1, R2, R3, T, false>, &done);
     if (e == cudaSuccess && occ == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_row2_inv<R1, R2, R3, T, false>, T, smem);
     if (e != cudaSuccess) { sm_set_error("row2 inv setup: %s", cudaGetErrorString(e)); return -100; }
-    int grid = num_sms() * row2_occ(occ);
+    int grid = num_sms() * (occ > 0 ? occ : 1);
     if (grid > p.R / 2) grid = p.R / 2;
     sm_launch(k_row2_inv<R1, R2, R3, T, false>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, ia, twC, twQ, work_bytes);
     SM_LAUNCH_CHECK();
@@ -2094,13 +1729,13 @@ static int launch_row_ct(bool inverse, const SmPlan& p, const RowFwdArgs* fa, co
   static bool done[4] = {false, false, false, false};
   static int occ[2] = {0, 0};
   constexpr int CH = R1 * R2 * R3 * R4;
-  if (!inverse && use_tma()) {
+  if (!inverse) {
     int rc = try_row2_fwd<R1, R2, R3, R4, T, kPad>(p, *fa, twC, twQ, sumsq, st);
     if (rc <= 0) return rc;
     rc = try_row2_fwd4(p, *fa, twC, twQ, sumsq, st);
     if (rc <= 0) return rc;
   }
-  if (inverse && use_tma()) {
+  if (inverse) {
     int rc = try_row2_inv<R1, R2, R3, R4, T, kPad>(p, *ia, twC, twQ, st);
     if (rc <= 0) return rc;
     rc = try_row2_inv4(p, *ia, twC, twQ, st);
@@ -2113,7 +1748,7 @@ static int launch_row_ct(bool inverse, const SmPlan& p, const RowFwdArgs* fa, co
   const int work_bytes = (((!inverse ? (nst >= 2 ? 2 : 1) : (nst >= 3 ? 2 : 1)) * bufstride * 8) + 127) / 128 * 128;
   const int stage_bytes = !inverse ? 4 * p.C : 8 * p.P + ((ia->out_mode == 0) ? 2 * p.C : 0);
   const bool aligned = (p.C % 8 == 0);
-  if (use_tma() && aligned && work_bytes + stage_bytes <= 227 * 1024 - 256 && p.R >= 2) {
+  if (aligned && work_bytes + stage_bytes <= 227 * 1024 - 256 && p.R >= 2) {
     const int smem = work_bytes + stage_bytes;
     const int which = inverse ? 1 : 0;
     if (!inverse) {
@@ -2126,13 +1761,7 @@ static int launch_row_ct(bool inverse, const SmPlan& p, const RowFwdArgs* fa, co
         e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[1], k_row_inv_tma<R1, R2, R3, R4, T, kPad>, T, smem);
     }
     if (e != cudaSuccess) { sm_set_error("row tma setup: %s", cudaGetErrorString(e)); return -100; }
-    int per_sm = occ[which] > 0 ? occ[which] : 1;
-    {                               // SM_ROW_OCC=n caps the resident row CTAs per SM (leaves room for another lane's kernels)
-      static int cap = -1;
-      if (cap < 0) { const char* e = getenv("SM_ROW_OCC"); cap = e ? atoi(e) : 0; }
-      if (cap > 0 && per_sm > cap) per_sm = cap;
-    }
-    int grid = num_sms() * per_sm;
+    int grid = num_sms() * (occ[which] > 0 ? occ[which] : 1);
     if (grid > p.R) grid = p.R;
     if (!inverse) sm_launch(k_row_fwd_tma<R1, R2, R3, R4, T, kPad>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, *fa, twC, twQ, sumsq, work_bytes);
     else sm_launch(k_row_inv_tma<R1, R2, R3, R4, T, kPad>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, *ia, twC, twQ, work_bytes);
@@ -2198,25 +1827,23 @@ extern "C" int sm_fwd_rows_f32(const sm_plan* plan, const void* tables, const fl
 static int launch_col(const SmPlan& p, const void* tables, int sweep, int inverse, float* re, float* im,
                       const float* cull_thr, const float* scale_dev, float scale_host, int use_scale,
                       int write_im, cudaStream_t st, float* im_alt = nullptr, const int* sel = nullptr,
-                      const int* wsel = nullptr, int wskip = 0, int tile0 = 0, int band_tiles = 0) {
+                      const int* wsel = nullptr, int wskip = 0) {
   if (ensure_attrs()) return -100;
   ColArgs ca{};
   int n_inst = 0;
   sm_col_args(p, sweep, inverse, &ca, &n_inst);
   ca.re = re; ca.im = im; ca.cull_thr = cull_thr; ca.im_alt = im_alt; ca.sel = sel;
   ca.scale_ptr = scale_dev; ca.scale_host = scale_host; ca.use_scale = use_scale;
-  ca.write_im = write_im; ca.wsel = wsel; ca.wskip = wskip; ca.tile0 = tile0;
-  const int ntiles = band_tiles > 0 ? band_tiles : (p.Ch + 1 + SM_COL_TILE - 1) / SM_COL_TILE;
+  ca.write_im = write_im; ca.wsel = wsel; ca.wskip = wskip;
+  const int ntiles = sm_col_tiles(p);
   {
     ColCtArgs c{};
     c.p0 = inverse ? im : re; c.p1 = inverse ? re : im;
     c.p0_alt = inverse ? im_alt : nullptr; c.sel = inverse ? sel : nullptr;
     c.P = p.P; c.Ch = p.Ch; c.inst_mul = ca.inst_mul; c.elem_mul = ca.elem_mul; c.tw_mul = ca.tw_mul;
     c.thr_ptr = cull_thr; c.scale_ptr = use_scale ? scale_dev : nullptr;
-    c.scale = use_scale ? scale_host : 1.0f; c.write_p1_fwd = write_im; c.wsel = wsel; c.wskip = wskip; c.tile0 = tile0;
-    int rc = try_col_p(ca.n_rad, ca.rad, inverse != 0, ca.big_tw != 0, dim3(ntiles, n_inst), c, tabR(p, tables), st);
-    if (rc <= 0) return rc;
-    rc = try_col_ct(ca.n_rad, ca.rad, inverse != 0, ca.big_tw != 0, dim3(ntiles, n_inst), c, tabR(p, tables), st);
+    c.scale = use_scale ? scale_host : 1.0f; c.write_p1_fwd = write_im; c.wsel = wsel; c.wskip = wskip;
+    const int rc = try_col_p(ca.n_rad, ca.rad, inverse != 0, ca.big_tw != 0, dim3(ntiles, n_inst), c, tabR(p, tables), st);
     if (rc <= 0) return rc;
   }
   const int threads = (sweep == 0) ? p.thrA : p.thrB;
@@ -2224,54 +1851,6 @@ static int launch_col(const SmPlan& p, const void* tables, int sweep, int invers
   sm_launch(k_col, dim3(dim3(ntiles, n_inst)), dim3(threads), (size_t)(smem), st, p, ca, tabR(p, tables));
   SM_LAUNCH_CHECK();
   return 0;
-}
-
-// Column bands: the two sweeps of a four-step column transform run band by band over the column tiles, sweep A of a
-// band immediately followed by sweep B of the same band, so that the second sweep finds the band (R x 32 x tiles x 8 B)
-// in the 126 MB L2 instead of streaming the whole spectrum through DRAM a second time (a spectrum is 0.07 - 1.9 GB).
-// SM_COL_BAND_MB sets the band size; 0 = one launch per sweep, which is the DEFAULT: measured on the Llama-8B-shaped bench
-// (profiles/r02_band_sweep.log) bands of 16 / 32 / 64 MB take 9.1 / 7.1 / 5.9 ms per 4 layers for the forward sweeps against
-// 5.1 ms unbanded -- the sweeps are latency bound, and the per-launch ramp-up / tail of 5 - 15 small launches costs more than
-// the L2 hits save.  Kept as an A-B switch.
-static int col_band_tiles(const SmPlan& p) {
-  static int mb = -1;
-  if (mb < 0) { const char* e = getenv("SM_COL_BAND_MB"); mb = e ? atoi(e) : 0; if (mb < 0) mb = 0; }
-  const int ntiles = sm_col_tiles(p);
-  if (mb == 0) return ntiles;
-  const double tile_bytes = (double)p.R * SM_COL_TILE * 8.0;
-  int t = (int)((double)mb * 1048576.0 / tile_bytes);
-  if (t < 1) t = 1;
-  return t < ntiles ? t : ntiles;
-}
-
-// both sweeps of a two-sweep plan in one launch (k_col2_ct); returns 1 if this plan has no fused kernel
-static int launch_col2_pair(const SmPlan& p, const void* tables, int inverse, float* re, float* im, const float* cull_thr,
-                            const float* scale_dev, float scale_host, int write_im, cudaStream_t st,
-                            float* im_alt = nullptr, const int* sel = nullptr) {
-  if (p.col_passes != 2 || !use_col2()) return 1;
-  ColArgs ca[2];
-  int n_inst[2];
-  ColCtArgs c[2];
-  for (int k = 0; k < 2; ++k) {                  // k-th sweep in execution order
-    const int sweep = inverse ? 1 - k : k;
-    ca[k] = ColArgs{};
-    sm_col_args(p, sweep, inverse, &ca[k], &n_inst[k]);
-    const bool lastk = (k == 1);
-    c[k] = ColCtArgs{};
-    c[k].p0 = inverse ? im : re; c[k].p1 = inverse ? re : im;
-    c[k].p0_alt = inverse ? im_alt : nullptr; c[k].sel = inverse ? sel : nullptr;
-    c[k].P = p.P; c[k].Ch = p.Ch; c[k].inst_mul = ca[k].inst_mul; c[k].elem_mul = ca[k].elem_mul; c[k].tw_mul = ca[k].tw_mul;
-    c[k].thr_ptr = (inverse && k == 0) ? cull_thr : nullptr;                    // cull on the first inverse load
-    const bool use_scale = (!inverse && lastk);                                  // 1/||delta|| on the last forward store
-    c[k].scale_ptr = use_scale ? scale_dev : nullptr;
-    c[k].scale = use_scale ? scale_host : 1.0f;
-    c[k].write_p1_fwd = (!inverse && lastk) ? write_im : 1;
-  }
-  Col2Sched s{};
-  s.ntiles = sm_col_tiles(p); s.n1 = n_inst[0]; s.n2 = n_inst[1];
-  s.cnt = reinterpret_cast<unsigned int*>(const_cast<char*>(reinterpret_cast<const char*>(tables)) + sm_tab_off_K(p));
-  s.done = s.cnt + s.ntiles;
-  return try_col2_ct(ca[0].rad, ca[0].n_rad, ca[1].rad, ca[1].n_rad, inverse != 0, c[0], c[1], s, tabR(p, tables), st);
 }
 
 extern "C" int sm_fwd_cols(const sm_plan* plan, const void* tables, float* re, float* im,
@@ -2283,25 +1862,16 @@ int sm_fwd_cols_sel(const sm_plan* plan, const void* tables, float* re, float* i
                     int write_im, const int* wsel, int wskip, void* stream) {
   const SmPlan& p = plan->p;
   cudaStream_t st = (cudaStream_t)stream;
-  {
-    const int rc = launch_col2_pair(p, tables, 0, re, im, nullptr, scale_dev, scale_host, write_im, st);
-    if (rc <= 0) return rc;
-  }
   if (p.col_passes == 0) {
     sm_launch(k_scale_row, dim3((p.Ch + 1 + 255) / 256), dim3(256), (size_t)(0), st, re, im, p.Ch + 1, scale_dev, scale_host, write_im);
     SM_LAUNCH_CHECK();
     return 0;
   }
-  const int ntiles = sm_col_tiles(p);
-  const int band = p.col_passes == 2 ? col_band_tiles(p) : ntiles;
-  for (int t0 = 0; t0 < ntiles; t0 += band) {
-    const int nt = ntiles - t0 < band ? ntiles - t0 : band;
-    for (int sweep = 0; sweep < p.col_passes; ++sweep) {
-      const bool lastsweep = (sweep == p.col_passes - 1);
-      int rc = launch_col(p, tables, sweep, 0, re, im, nullptr, scale_dev, scale_host, lastsweep ? 1 : 0,
-                          lastsweep ? write_im : 1, st, nullptr, nullptr, lastsweep ? wsel : nullptr, wskip, t0, nt);
-      if (rc) return rc;
-    }
+  for (int sweep = 0; sweep < p.col_passes; ++sweep) {
+    const bool lastsweep = (sweep == p.col_passes - 1);
+    int rc = launch_col(p, tables, sweep, 0, re, im, nullptr, scale_dev, scale_host, lastsweep ? 1 : 0,
+                        lastsweep ? write_im : 1, st, nullptr, nullptr, lastsweep ? wsel : nullptr, wskip);
+    if (rc) return rc;
   }
   return 0;
 }
@@ -2315,20 +1885,11 @@ extern "C" int sm_inv_norm(const double* sumsq, float* out, void* stream) {
 int sm_inv_cols_sel(const sm_plan* plan, const void* tables, float* re, float* im, float* im_alt, const int* sel,
                     const float* cull_thr, void* stream) {
   const SmPlan& p = plan->p;
-  {
-    const int rc = launch_col2_pair(p, tables, 1, re, im, cull_thr, nullptr, 1.f, 1, (cudaStream_t)stream, im_alt, sel);
-    if (rc <= 0) return rc;
-  }
-  const int ntiles = sm_col_tiles(p);
-  const int band = p.col_passes == 2 ? col_band_tiles(p) : ntiles;
-  for (int t0 = 0; t0 < ntiles; t0 += band) {
-    const int nt = ntiles - t0 < band ? ntiles - t0 : band;
-    for (int i = 0; i < p.col_passes; ++i) {
-      const int sweep = p.col_passes - 1 - i;   // undo sweep B first, then sweep A
-      int rc = launch_col(p, tables, sweep, 1, re, im, i == 0 ? cull_thr : nullptr, nullptr, 1.f, 0, 1,
-                          (cudaStream_t)stream, im_alt, sel, nullptr, 0, t0, nt);
-      if (rc) return rc;
-    }
+  for (int i = 0; i < p.col_passes; ++i) {
+    const int sweep = p.col_passes - 1 - i;   // undo sweep B first, then sweep A
+    int rc = launch_col(p, tables, sweep, 1, re, im, i == 0 ? cull_thr : nullptr, nullptr, 1.f, 0, 1,
+                        (cudaStream_t)stream, im_alt, sel);
+    if (rc) return rc;
   }
   return 0;
 }

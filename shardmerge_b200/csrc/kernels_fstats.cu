@@ -41,7 +41,6 @@
 // Only tensors with more than 2^20 elements come here (sm_fstats_supported); smaller ones are launch
 // bound and use the step-by-step kernels.
 #include <cstddef>
-#include <cstdlib>
 #include "sm_internal.h"
 
 namespace {
@@ -87,11 +86,7 @@ struct FsWs {                        // carved out of the caller's workspace
   // not zeroed (guarded by scnt):
   float2* sbkt;                      // [n_lists][scap]  (|re0| with "multiplicity 1" in the sign bit, |re1|)
   unsigned int scap, n_lists;
-  unsigned long long* dbg;           // development: per-CTA phase timestamps (NULL in production)
 };
-
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define FS_STAMP(slot) do { if (ws.dbg && threadIdx.x == 0) ws.dbg[(blockIdx.x) * 8 + (slot)] = gtimer(); } while (0)
 
 __device__ __forceinline__ unsigned int absbits(float v) { return __float_as_uint(v) & 0x7fffffffu; }
 __device__ __forceinline__ int sgn(float v) { return (v > 0.f) - (v < 0.f); }
@@ -242,7 +237,6 @@ __global__ void __launch_bounds__(kSampleThreads) k_fs_sample(const __grid_const
   const float* re1 = sw ? c.reX : c.reY;
   BlendScal bs{};
   if (MODE == 1) { bs.thr = *c.thr_cut; bs.dot = c.scal4[0]; bs.ct = c.scal4[1]; bs.sn = c.scal4[2]; bs.rn = c.scal4[3]; bs.t_sum = c.t_sum; }
-  FS_STAMP(0);
 #pragma unroll
   for (int j = 0; j < kSampleBins / kSampleThreads; ++j) s_h[threadIdx.x + kSampleThreads * j] = 0u;
   {  // this kernel also clears the histograms of the pass that follows (fire-and-forget stores, done long before it starts):
@@ -279,15 +273,12 @@ __global__ void __launch_bounds__(kSampleThreads) k_fs_sample(const __grid_const
     }
   }
   __syncthreads();
-  FS_STAMP(1);
 #pragma unroll
   for (int j = 0; j < kSampleBins / kSampleThreads; ++j) {
     const unsigned int v = s_h[threadIdx.x + kSampleThreads * j];
     if (v) atomicAdd(ws.shist + threadIdx.x + kSampleThreads * j, v);
   }
-  FS_STAMP(2);
   const bool last = fs_last_block(st);
-  FS_STAMP(3);
   if (!last) return;
   const bool want_a = (k_lo >= 0 && k_lo < (long long)ns), want_b = (k_hi >= 0 && k_hi < (long long)ns);
   {
@@ -324,7 +315,6 @@ __global__ void __launch_bounds__(kSampleThreads) k_fs_sample(const __grid_const
     st->ticket = 0u;
     ws.meta[0] = status == 0u ? (unsigned int)width : 0u;   // the counters the pass that follows may touch (a dead pass: none)
   }
-  FS_STAMP(4);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -369,7 +359,7 @@ constexpr size_t kPassDynSmem = (size_t)kPassWarps * kQCap * (2 * sizeof(float4)
 // work distribution: every CTA (= SM) owns an equal contiguous share of the items; inside it a warp takes chunks
 // of kChunkIters x 64 consecutive float4 items, the first by its own number, further ones from a shared-memory
 // counter (fetched one chunk ahead), so all warps of an SM finish together.  With a static split over 4 CTAs per
-// SM the slowest CTA finished 40 % after the fastest (phase timestamps, tools/fs_stamps.py).
+// SM the slowest CTA finished 40 % after the fastest (measured with per-CTA phase timestamps).
 constexpr unsigned int kChunkIters = 2, kChunkItems = kChunkIters * 64;
 __shared__ unsigned int g_fs_chunk;
 
@@ -523,7 +513,6 @@ __global__ void __launch_bounds__(kPassThreads, kPassCtasPerSm) k_fs_pass(const 
   __shared__ int s_ok;
   unsigned int* const s_hist = g_fs_coarse;
   constexpr int NT = kPassThreads;
-  FS_STAMP(0);
   const bool sw = (c.sel != nullptr && *c.sel != 0);
   const float* __restrict__ re0 = sw ? c.reY : c.reX;
   const float* __restrict__ re1 = sw ? c.reX : c.reY;
@@ -620,7 +609,6 @@ __global__ void __launch_bounds__(kPassThreads, kPassCtasPerSm) k_fs_pass(const 
       chunk = __shfl_sync(0xffffffffu, next, 0);
     }
     if (qn > 0) fs_drain<MODE>(wid, 0, qn, da);
-    FS_STAMP(1);
   }
   {
     unsigned long long below = 2ull * below_in + da.below;
@@ -648,9 +636,7 @@ __global__ void __launch_bounds__(kPassThreads, kPassCtasPerSm) k_fs_pass(const 
       atomicAdd(&st->s_in[0], r0); atomicAdd(&st->s_in[1], r1); atomicAdd(&st->s_in[2], r2);
     }
   }
-  FS_STAMP(3);
   const bool last_cta = fs_last_block(st);
-  FS_STAMP(4);
   if (!last_cta) return;
 
   // ---- last CTA: coarse bin of the statistic -> exact key from that bin's fine counters
@@ -711,7 +697,6 @@ __global__ void __launch_bounds__(kPassThreads, kPassCtasPerSm) k_fs_pass(const 
     }
     if (thr_out) *thr_out = st->value;
   }
-  FS_STAMP(5);
 }
 
 // cutoff pass, second half: the side-list entries with |re1| >= key join the SLERP sums; the last CTA turns the sums
@@ -797,7 +782,7 @@ extern "C" size_t sm_fstats_ws_bytes(const sm_plan* plan) {
   const unsigned int n_lists = fs_grid(p).x;
   size_t b = fs_zero_bytes();
   b += (size_t)n_lists * fs_scap(p, n_lists) * 8;
-  return b + 512 + 65536;        // + alignment, development timestamps (SM_FS_STAMPS)
+  return b + 512;                // + alignment
 }
 
 static int fs_carve(const sm_plan* plan, void* wsp, size_t ws_bytes, FsWs* w) {
@@ -817,9 +802,7 @@ static int fs_carve(const sm_plan* plan, void* wsp, size_t ws_bytes, FsWs* w) {
   w->zero_bytes = (size_t)(b - z0);
   w->n_lists = fs_grid(p).x;
   w->scap = fs_scap(p, w->n_lists);
-  w->sbkt = reinterpret_cast<float2*>(b); b += (size_t)w->n_lists * w->scap * 8;
-  b = reinterpret_cast<char*>(((uintptr_t)b + 63) / 64 * 64);
-  w->dbg = getenv("SM_FS_STAMPS") ? reinterpret_cast<unsigned long long*>(b) : nullptr;   // development only
+  w->sbkt = reinterpret_cast<float2*>(b);
   return 0;
 }
 
@@ -852,7 +835,6 @@ extern "C" int sm_fstats_cutoff(const sm_plan* plan, const float* reX, const flo
   fs_sample_ranks(rank, total, &k_lo, &k_hi);
   sm_launch(k_fs_sample<0>, dim3(fs_sample_grid()), dim3(kSampleThreads), (size_t)(0), s, p, c, st, w, rank, k_lo, k_hi);
   SM_LAUNCH_CHECK();
-  if (getenv("SM_FS_ONLY_SAMPLE")) return 0;
   if ((rc = fs_pass_attr())) return rc;
   sm_launch(k_fs_pass<0>, dim3(w.n_lists), dim3(kPassThreads), (size_t)(kPassDynSmem), s, p, c, st, w, nullptr, thr_cut_out);
   SM_LAUNCH_CHECK();

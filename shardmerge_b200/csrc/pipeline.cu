@@ -10,15 +10,8 @@
 // from there.  The chain always continues down the SLERP branch (what the BASELINE configs
 // take); if k_prepare found another branch, or an order-statistic window missed, the caller sees
 // it in the scalar block afterwards and re-runs that tensor on the step-by-step path.
-#include <cstdlib>
 #include <vector>
 #include "sm_internal.h"
-
-bool sm_pdl_enabled() {              // SM_PDL=0: plain stream-ordered launches (A-B switch, sm_internal.h)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SM_PDL"); v = (e != nullptr && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
 
 namespace {
 

@@ -37,12 +37,11 @@ void sm_set_error(const char* fmt, ...);
 // B200 (tools/ubench_pdl.cu), 17 boundaries per pair merge.  No kernel issues griddepcontrol.launch_dependents: with an early
 // trigger the next kernel's CTAs become resident and sit in the wait while the current one runs, which saves nothing more in
 // a single stream (same ubench) and, with several lanes, takes the SM slots the OTHER lanes' kernels would have filled
-// (value 53.0 -> 49.7 Gparam/s, profiles/r02_ab_pdl.log).  SM_PDL=0 launches plainly (A-B switch).
+// (value 53.0 -> 49.7 Gparam/s, profiles/r02_ab_pdl.log).
 #ifdef __CUDACC__
 __device__ __forceinline__ void sm_pdl_enter() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
 }
-bool sm_pdl_enabled();
 template <class... KA, class... A>
 static inline void sm_launch(void (*kernel)(KA...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -50,7 +49,7 @@ static inline void sm_launch(void (*kernel)(KA...), dim3 grid, dim3 block, size_
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = sm_pdl_enabled() ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<A&&>(args)...);      // errors surface in SM_LAUNCH_CHECK()
 }
 #endif
@@ -64,10 +63,9 @@ static inline int sm_quad_count(const SmPlan& p) {     // entries b < Ch / r for
   const int n = p.Ch / p.row_rad[0], n8 = (p.Ch % 8 == 0) ? p.Ch / 8 : 0;
   return n > n8 ? n : n8;
 }
-// after the quads: 2 x ntiles u32 tile counters of the fused two-sweep column kernel (zero between launches)
+static inline size_t sm_tab_bytes(const SmPlan& p) { return sm_tab_off_Q(p) + 32 * (size_t)sm_quad_count(p); }
+// column tiles (SM_COL_TILE columns each) over the Ch + 1 columns of the half spectrum
 static inline int sm_col_tiles(const SmPlan& p) { return (p.Ch + 1 + SM_COL_TILE - 1) / SM_COL_TILE; }
-static inline size_t sm_tab_off_K(const SmPlan& p) { return (sm_tab_off_Q(p) + 32 * (size_t)sm_quad_count(p) + 63) / 64 * 64; }
-static inline size_t sm_tab_bytes(const SmPlan& p) { return sm_tab_off_K(p) + 8 * (size_t)sm_col_tiles(p) + 64; }
 
 // iteration space of the element-wise / statistics kernels over the valid half spectrum
 #define SM_EW_THREADS 256

@@ -92,7 +92,7 @@ class FourierMerge(MergeTensorsBase):
         self.defer_checks = False        # True inside merge(): _merge_layer returns before the check
         self._lane_streams: dict = {}    # device index -> [streams]
         self._lane_next = 0
-        self.fused_tree = os.environ.get("SHARDMERGE_FUSED_TREE", "1") != "0"   # 0: pair tree on the step-by-step path (A-B)
+        self.fused_tree = True           # False: pair trees (3+ finetunes) run on the step-by-step path
         self._tree_waiting: list = []    # pair trees whose row passes are enqueued but whose norms have not been read yet
         self.keep_intermediates = False  # tests: keep the tree's fp32 round results in self.last_tree
         self.last_tree: list = []

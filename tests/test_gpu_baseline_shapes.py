@@ -2,8 +2,8 @@
 
   (a) forward spectrum and inverse transform of every 2-D Llama-3.1-8B / 70B / TinyLlama shape against an independent
       fp64 FFT (torch.fft on the device -- TEST-ONLY checker, cuFFT never runs on the product path), through
-      Plan.row_freq(): one case per packed kernel instantiation the bench times, plus the SM_*=0 fallbacks in
-      subprocesses (the switches are read once per process);
+      Plan.row_freq(): one case per packed kernel instantiation the bench times, plus the one-row kernels
+      (k_row_fwd_tma / k_row_inv_tma, k_row_fwd_ct / k_row_inv_ct) at the shapes and input types that select them;
   (b) FourierMerge.merge_sources against oracle/oracle_np.merge_layer at 1024x4096, 4096x4096, 14336x4096, 4096x14336
       and 8192x8192 with north_star's bounds: fp32 merged delta rel-L2 <= 1e-5 once the flipped bins are set aside
       (and outright when nothing flips), bf16 within 1 ulp on >= 99.99 % when nothing flips; flips are listed;
@@ -16,8 +16,6 @@
 import glob
 import json
 import os
-import subprocess
-import sys
 import time
 from pathlib import Path
 
@@ -78,15 +76,17 @@ def _rel(a, b):
     return float(((a - b).abs() ** 2).sum().sqrt() / (b.abs() ** 2).sum().sqrt())
 
 
-def forward_inverse_check(E, shape, seed=0):
-    """-> (forward rel-L2 vs fp64 rfft2, inverse rel-L2 vs the input given the fp64 spectrum)."""
+def forward_inverse_check(E, shape, seed=0, f32=False):
+    """-> (forward rel-L2 vs fp64 rfft2, inverse rel-L2 vs the input given the fp64 spectrum).
+    f32: the forward pass reads the delta as an fp32 source instead of forming it from the bf16 pair."""
     R, C = shape
     base, fts = synth(shape, seed)
     delta = fts[0].float() - base.float()
     ws = E.get_workspace(R, C, DEV)
     pl = ws.plan
     ws.ctl.zero_()
-    E.fwd_rows(ws, 0, E.Source(base=base, ft=fts[0]), E.D_SUMSQ0)
+    src = E.Source(x32=delta) if f32 else E.Source(base=base, ft=fts[0])
+    E.fwd_rows(ws, 0, src, E.D_SUMSQ0)
     E.fwd_cols(ws, 0, scale=1.0)
     freq = pl.row_freq().to(DEV)
     ref = torch.fft.rfft2(delta.double())                     # [R][Ch+1] complex128, natural row order
@@ -116,30 +116,20 @@ def test_forward_and_inverse_vs_fp64_fft(E, shape):
     torch.cuda.empty_cache()
 
 
-FALLBACKS = [{"SM_COL_PAIRS": "0"}, {"SM_ROW_PAIRS": "0"}, {"SM_ROW_TMA": "0"}, {"SM_ROW_EO": "0"}, {"SM_COL_FUSED": "1"},
-             {"SM_COL_BULK": "1"}, {"SM_COL_BULK": "2"}]
+# The paired-row kernels take bf16 pairs of rows only.  An fp32 source, an odd row count or a single row selects the one-row
+# kernels instead: k_row_fwd_tma / k_row_inv_tma where the row and its staging fit in shared memory (fp32 at the Llama-8B
+# shapes; 4095x4096, 2047x2048), else k_row_fwd_ct / k_row_inv_ct (a single row; fp32 at 8192x28672).
+ONE_ROW = [(s, True) for s in LLAMA8B] + [((4095, 4096), False), ((2047, 2048), False), ((1, 4096), False),
+                                         ((1, 8192), False), ((8192, 28672), True)]
 
 
-@pytest.mark.parametrize("env", FALLBACKS, ids=lambda e: ",".join(f"{k}={v}" for k, v in e.items()))
-def test_fallback_kernels_vs_fp64_fft(env):
-    """The A-B switches select other kernel instantiations for the same shapes; each set is checked the same way."""
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    code = ("import sys, json; sys.path.insert(0, %r); import torch\n"
-            "from shardmerge_b200 import engine as E\n"
-            "from tests.test_gpu_baseline_shapes import forward_inverse_check, LLAMA8B\n"
-            "out = {}\n"
-            "for s in LLAMA8B + [(8192, 8192), (2048, 5632)]:\n"
-            "    f, i, p, d = forward_inverse_check(E, s, seed=1)\n"
-            "    out['%%dx%%d' %% s] = [f, i, p]\n"
-            "print('RESULT ' + json.dumps(out))\n") % str(ROOT)
-    r = subprocess.run([sys.executable, "-c", code], env={**os.environ, **env}, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    res = json.loads(r.stdout.split("RESULT ")[1])
-    tag = ",".join(f"{k}={v}" for k, v in env.items())
-    record("fft_vs_fp64_fallbacks", tag, **{k: dict(forward_rel_l2=v[0], inverse_rel_l2=v[1]) for k, v in res.items()})
-    for k, (f, i, p) in res.items():
-        assert f <= 1e-6 and i <= 1e-6 and p, (tag, k, f, i, p)
+@pytest.mark.parametrize("shape,f32", ONE_ROW, ids=lambda v: f"{v[0]}x{v[1]}" if isinstance(v, tuple) else ("f32" if v else "bf16"))
+def test_one_row_kernels_vs_fp64_fft(E, shape, f32):
+    fwd, inv, pad_ok, desc = forward_inverse_check(E, shape, f32=f32)
+    record("fft_vs_fp64_one_row", f"{shape[0]}x{shape[1]}" + (" f32" if f32 else ""), forward_rel_l2=fwd, inverse_rel_l2=inv, plan=desc)
+    assert fwd <= 1e-6 and inv <= 1e-6 and pad_ok, (fwd, inv, pad_ok)
+    E.clear_caches()
+    torch.cuda.empty_cache()
 
 
 def _merger():
