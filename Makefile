@@ -7,7 +7,7 @@ NVFLAGS   := $(ARCH) -std=c++17 -O3 -lineinfo -Xcompiler -fPIC -Xptxas -v
 CSRC      := shardmerge_b200/csrc
 LIB       := shardmerge_b200/libshardmerge_b200.so
 HDRS      := $(CSRC)/fft_core.cuh $(CSRC)/fft_bodies.cuh $(CSRC)/plan.h $(CSRC)/sm_internal.h include/shardmerge_b200.h
-OBJS      := build/kernels_fft.o build/kernels_stats.o build/kernels_fstats.o build/kernels_elem.o build/pipeline.o
+OBJS      := build/kernels_fft.o build/kernels_stats.o build/kernels_fstats.o build/kernels_elem.o build/kernels_lora.o build/pipeline.o
 
 all: $(LIB) hostemu
 

@@ -285,6 +285,16 @@ int sm_elem_merge_bf16(int mode, size_t n, const void* base, const void* const* 
  * dtype 0: fp32, 1: bf16.  Both tensors are read once (HBM-bound). */
 int sm_cosine_cols(int dtype, int R, int C, const void* a, const void* b, double* out_sum, void* stream);
 
+/* ---- PEFT LoRA adapters: the finetuned weight formed from the base and the adapter's low-rank factors ------------------
+ * ft_out[i][j] = round_to_dtype(base)( fp32(base[i][j]) + scaling * acc[i][j] ) with
+ * acc[i][j] = sum_{k=0..r-1} fp32(lora_B[i][k]) * fp32(lora_A[k][j]): one fp32 FMA per term, ascending k, starting from 0;
+ * the product with `scaling` and the add are rounded separately; the final rounding is round-to-nearest-even, and NaN and
+ * Inf propagate as IEEE arithmetic does.  base and ft_out are [R][C] row-major in base_dtype, lora_A is [r][C] and lora_B
+ * [R][r], both in ab_dtype (dtype codes of sm_elem_merge: 0 fp32, 1 bf16, 2 fp16).  Any R, C, r >= 1 (R <= 4,194,240);
+ * ft_out must not alias base.  No allocation; asynchronous on `stream`. */
+int sm_lora_materialize(int R, int C, int r, int base_dtype, const void* base, int ab_dtype, const void* lora_A,
+                        const void* lora_B, float scaling, void* ft_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

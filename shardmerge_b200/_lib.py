@@ -46,6 +46,7 @@ SIGNATURES = {
     "sm_elem_merge": (_i, [_i, _i, _sz, _vp, _vp, _i, _vp, _vp]),
     "sm_elem_merge_bf16": (_i, [_i, _sz, _vp, _vp, _i, _vp, _vp]),
     "sm_cosine_cols": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp]),
+    "sm_lora_materialize": (_i, [_i, _i, _i, _i, _vp, _i, _vp, _vp, _f, _vp, _vp]),
     "sm_copy_bytes": (_i, [_vp, _vp, _sz, _vp]),
     "sm_expand_full": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "sm_pack_half": (_i, [_vp, _vp, _vp, _vp, _vp]),

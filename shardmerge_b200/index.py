@@ -7,16 +7,19 @@ can be passed to FourierMerge instead of these classes.
   InMemoryIndex        tensors handed over as dicts (tests, benchmarks, synthetic models)
   LocalSafetensorsIndex {storage_dir}/{org}/{model}/model.safetensors.index.json + shards on disk,
                        read lazily, uploaded with pinned staging, nothing kept after use
-                       (the reference keeps every tensor it ever read in RAM, index.py:79,265).
+                       (the reference keeps every tensor it ever read in RAM, index.py:79,265);
+                       or a PEFT LoRA adapter directory (shardmerge_b200/lora.py), bound to a base.
 """
 from __future__ import annotations
 
 import json
 import re
 from pathlib import Path
-from typing import Dict, List, Set
+from typing import Dict, List, Optional, Set
 
 import torch
+
+from . import lora
 
 
 class TensorPromise:
@@ -181,17 +184,44 @@ class LocalSafetensorsIndex(_IndexBase):
         self._readers = None
         self._pin_free: Dict[int, list] = {}             # pinned buffers by size
         self._pin_busy: list = []                        # (event, buffer): handed back once the upload has finished
+        self._adapters: Dict[str, lora.Adapter] = {}     # adapter model uri -> its parsed config and header
         import threading
         self._pin_lock = threading.Lock()
 
     async def add_model(self, model_uri: str, revision: str = "main"):
-        if model_uri in self.model_indexes:
+        if model_uri in self.model_indexes or model_uri in self._adapters:
             return
-        path = self.storage_dir / model_uri / "model.safetensors.index.json"
+        directory = self.storage_dir / model_uri
+        path = directory / "model.safetensors.index.json"
+        if not path.exists() and lora.is_adapter_dir(directory):
+            _, entries = self._meta(directory / lora.WEIGHTS_FILE)
+            self._adapters[model_uri] = lora.Adapter(model_uri, lora.read_config(directory),
+                                                     {k: (d, s) for k, (d, s, _, _) in entries.items()})
+            return
         if not path.exists():
             raise FileNotFoundError(f"{path} not found (shardmerge_b200 does not download models)")
         with open(path) as fh:
             self._register(model_uri, json.load(fh))
+
+    # ---- LoRA adapters ---------------------------------------------------------------------------------------
+    # An adapter has no tensors under base names: once bound to a base it reports that base's keys, order and shapes.
+    # `prefetch(adapter, name)` uploads only the factors or the full replacement of `name` (the keys of
+    # adapter_part(adapter, name)), and `get_tensor(adapter, key)` hands each over by its key in the adapter's file.
+    def is_adapter(self, model_uri: str) -> bool:
+        return model_uri in self._adapters
+
+    def bind_adapter(self, model_uri: str, base_uri: str):
+        """Bind an added adapter to the added full model `base_uri`; raises lora.UnsupportedAdapter."""
+        if base_uri in self._adapters:
+            raise lora.UnsupportedAdapter(f"adapter {model_uri}: its base {base_uri} is an adapter, not a full model")
+        self._adapters[model_uri].bind(base_uri, self.tensor_shapes(base_uri))
+        self.model_indexes[model_uri] = self.model_indexes[base_uri]
+        self._order[model_uri] = self._order[base_uri]
+
+    def adapter_part(self, model_uri: str, tensor_name: str) -> Optional[lora.Part]:
+        """How `model_uri`'s `tensor_name` is formed when `model_uri` is a bound adapter, else None."""
+        adapter = self._adapters.get(model_uri)
+        return None if adapter is None else adapter.part(tensor_name)
 
     # ---- safetensors headers ---------------------------------------------------------------------------------
     def _meta(self, shard: Path) -> tuple:
@@ -208,13 +238,20 @@ class LocalSafetensorsIndex(_IndexBase):
         return meta
 
     def _shard_of(self, model_uri: str, tensor_name: str) -> Path:
+        adapter = self._adapters.get(model_uri)
+        if adapter is not None:
+            if tensor_name not in adapter.tensors:
+                raise KeyError(f"Tensor {tensor_name} not found in adapter {model_uri}")
+            return self.storage_dir / model_uri / lora.WEIGHTS_FILE
         index = self.model_indexes[model_uri]
         if tensor_name not in index["weight_map"]:
             raise KeyError(f"Tensor {tensor_name} not found in model {model_uri}")
         return self.storage_dir / model_uri / index["weight_map"][tensor_name]
 
     def tensor_shapes(self, model_uri: str) -> Dict[str, tuple]:
-        """shapes from the safetensors headers (no tensor data is read)."""
+        """shapes from the safetensors headers (no tensor data is read); a bound adapter has its base's."""
+        if model_uri in self._adapters:
+            return self.tensor_shapes(self._adapters[model_uri].base)
         out: Dict[str, tuple] = {}
         index = self.model_indexes[model_uri]
         for shard in sorted(set(index["weight_map"].values())):
@@ -274,6 +311,11 @@ class LocalSafetensorsIndex(_IndexBase):
         return torch.empty(max(nbytes, 1), dtype=torch.uint8).pin_memory()
 
     def prefetch(self, model_uri: str, tensor_name: str, device: str):
+        adapter = self._adapters.get(model_uri)
+        for key in adapter.part(tensor_name).keys if adapter is not None else (tensor_name,):
+            self._prefetch_key(model_uri, key, device)
+
+    def _prefetch_key(self, model_uri: str, tensor_name: str, device: str):
         dev = torch.device(device)
         if dev.type != "cuda":
             return
@@ -320,7 +362,7 @@ class LocalSafetensorsIndex(_IndexBase):
                 pre = self._take_prefetched(model_uri, tensor_name, device)
                 if pre is not None:
                     return pre
-                self.prefetch(model_uri, tensor_name, device)               # not announced: the same path, waited for at once
+                self._prefetch_key(model_uri, tensor_name, device)          # not announced: the same path, waited for at once
                 return self._take_prefetched(model_uri, tensor_name, device)
             return self._host_tensor(model_uri, tensor_name)
 

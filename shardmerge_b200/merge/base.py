@@ -16,12 +16,15 @@ from typing import List
 import torch
 
 from ..config import MergeConfig, MergeModel
+from ..lora import UnsupportedAdapter
 from ..writer import ModelWriter, ShardLayer
 
 logger = logging.getLogger(__name__)
 
 
 class MergeTensorsBase(ABC):
+    merges_adapters = False      # True: _merge_layer forms a LoRA adapter's finetuned tensors (index managers with is_adapter)
+
     def __init__(self, config: MergeConfig, index_manager=None):
         if index_manager is None:
             raise ValueError("shardmerge_b200 strategies need an index_manager (see shardmerge_b200.index)")
@@ -61,6 +64,17 @@ class MergeTensorsBase(ABC):
         for m in self.config.finetune_merge:
             await im.add_model(m.base)
             await im.add_model(m.model)
+        is_adapter = getattr(im, "is_adapter", None)
+        if is_adapter is not None:
+            if is_adapter(self.config.output_base_model):
+                raise UnsupportedAdapter(f"adapter {self.config.output_base_model}: output_base_model must be a full model")
+            for m in self.config.finetune_merge:
+                if not is_adapter(m.model):
+                    continue
+                if not self.merges_adapters:
+                    raise UnsupportedAdapter(f"adapter {m.model}: {type(self).__name__} does not merge LoRA adapters; "
+                                             f"FourierMerge (merge/fast_fourier.py) does, or merge the materialised checkpoint")
+                im.bind_adapter(m.model, m.base)      # the adapter is applied to this entry's base; refusals raise here
         want = im.get_model_keys(self.config.output_base_model)
         for m in self.config.finetune_merge:
             have = im.get_model_keys(m.model)

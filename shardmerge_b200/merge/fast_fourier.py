@@ -23,6 +23,7 @@ from typing import List, Optional
 import torch
 
 from .. import engine as E
+from .. import lora
 from ..config import MergeConfig
 from ..constants import INPUT_LAYER, OUTPUT_LAYER
 from ..tensor.functions import correlated_pairs
@@ -75,6 +76,7 @@ class _PendingTree:
 
 
 class FourierMerge(MergeTensorsBase):
+    merges_adapters = True       # a LoRA adapter's finetuned tensor is formed on the device from its factors (lora.py)
     pipeline_depth = 1           # merge(): one tensor stays in flight while the previous one is settled / written
     # Consecutive tensors alternate between `lanes` CUDA streams (each with its own workspace): every kernel of the
     # chain has a latency-bound prologue / epilogue (single-CTA statistics epilogues, launch gaps, tail waves) that
@@ -141,11 +143,31 @@ class FourierMerge(MergeTensorsBase):
                                      f"FFT path:\n{lines}")
 
     # -------------------------------------------------------------------------------------
+    def _adapter_part(self, model_uri: str, name: str) -> Optional[lora.Part]:
+        """lora.Part of `name` when `model_uri` is a LoRA adapter, else None (also for index managers without adapters)."""
+        part_of = getattr(self.index_manager, "adapter_part", None)
+        return None if part_of is None else part_of(model_uri, name)
+
+    async def _adapter_tensor(self, model_uri: str, part: lora.Part, base: Optional[torch.Tensor], device: str) -> torch.Tensor:
+        """The adapter's finetuned tensor: `base` itself, the adapter's full tensor, or base + scaling * B @ A formed on the
+        device from the factors (the base tensor is the caller's: it crosses the host link once per merged tensor)."""
+        if part.kind == "base":
+            return base
+        got = [await self.index_manager.get_tensor(model_uri, key, device=device).get() for key in part.keys]
+        if part.kind == "full":
+            return got[0]
+        return lora.materialize(base, got[0], got[1], part.scaling)
+
     async def _passthrough(self, shard_layer, device, attr: str) -> torch.Tensor:
         chosen = next((m for m in self.config.finetune_merge if getattr(m, attr)), None)
         source = chosen.model if chosen is not None else self.config.output_base_model
-        logger.info(f"Passthrough - {shard_layer.layer_name} from {source}")
-        return await self.index_manager.get_tensor(source, shard_layer.layer_name, device=device).get()
+        name = shard_layer.layer_name
+        logger.info(f"Passthrough - {name} from {source}")
+        part = self._adapter_part(source, name)
+        if part is not None:
+            base = None if part.kind == "full" else await self.index_manager.get_tensor(chosen.base, name, device=device).get()
+            return await self._adapter_tensor(source, part, base, device)
+        return await self.index_manager.get_tensor(source, name, device=device).get()
 
     def prefetch_layer(self, shard_layer, device: str):
         prefetch = getattr(self.index_manager, "prefetch", None)
@@ -155,7 +177,11 @@ class FourierMerge(MergeTensorsBase):
         if number in (INPUT_LAYER, OUTPUT_LAYER):
             attr = "is_input" if number == INPUT_LAYER else "is_output"
             chosen = next((m for m in self.config.finetune_merge if getattr(m, attr)), None)
-            prefetch(chosen.model if chosen is not None else self.config.output_base_model, name, device)
+            source = chosen.model if chosen is not None else self.config.output_base_model
+            part = self._adapter_part(source, name)
+            if part is not None and part.kind != "full":
+                prefetch(chosen.base, name, device)
+            prefetch(source, name, device)          # an adapter's factors or full tensor, if it has any for `name`
             return
         wanted = [self.config.output_base_model]
         for m in self.config.finetune_merge:
@@ -186,7 +212,9 @@ class FourierMerge(MergeTensorsBase):
         for m in models:
             if m.base not in base_cache:
                 base_cache[m.base] = await fetch(m.base)
-            sources.append(E.make_source(base_cache[m.base], await fetch(m.model), weight=m.alpha, name=m.model))
+            part = self._adapter_part(m.model, name)
+            ft = await fetch(m.model) if part is None else await self._adapter_tensor(m.model, part, base_cache[m.base], device)
+            sources.append(E.make_source(base_cache[m.base], ft, weight=m.alpha, name=m.model))
         base_out = base_cache.get(self.config.output_base_model)
         if base_out is None:
             base_out = await fetch(self.config.output_base_model)
