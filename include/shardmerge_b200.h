@@ -295,6 +295,21 @@ int sm_cosine_cols(int dtype, int R, int C, const void* a, const void* b, double
 int sm_lora_materialize(int R, int C, int r, int base_dtype, const void* base, int ab_dtype, const void* lora_A,
                         const void* lora_B, float scaling, void* ft_out, void* stream);
 
+/* ---- A checkpoint's difference from its base: the dense products of a randomized SVD of delta ---------------------------
+ * delta[i][j] = fp32(M[i][j]) - fp32(W[i][j]) (one rounded fp32 subtraction) of two [R][C] row-major tensors W in w_dtype
+ * and M in m_dtype (dtype codes 0 fp32, 1 bf16, 2 fp16); delta is formed on load and never stored.
+ *   sm_lowrank_right:  Y[R][k] = delta . X[C][k];  if sumsq is non-null, *sumsq = sum of fp32(delta^2) in fp64
+ *   sm_lowrank_left:   Z[k][C] = Q[R][k]^T . delta
+ * X, Q, Y, Z are fp32 row-major.  Every output element is fp32 FMA chains over pieces of the reduction (C or R) added in a
+ * fixed order: the result is bit-identical from run to run.  ws is a 16-byte aligned device workspace of at least
+ * sm_lowrank_ws_bytes(R, C, k) bytes (one size serves both calls).  Any R, C, k >= 1 with R, C <= 8,388,480.
+ * No allocation; asynchronous on `stream`. */
+size_t sm_lowrank_ws_bytes(int R, int C, int k);
+int sm_lowrank_right(int R, int C, int k, int w_dtype, const void* W, int m_dtype, const void* M, const float* X, float* Y,
+                     double* sumsq, void* ws, size_t ws_bytes, void* stream);
+int sm_lowrank_left(int R, int C, int k, int w_dtype, const void* W, int m_dtype, const void* M, const float* Q, float* Z,
+                    void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

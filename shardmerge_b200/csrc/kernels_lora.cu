@@ -11,8 +11,7 @@
 // shared memory through chunks of kKc values of k, so any r >= 1 keeps the exact ascending chain.  HBM traffic is the base
 // read and the result write (2N + 2N bytes for bf16) plus the factors, which the CTAs of a tile column share through L2;
 // the kernel does r FMAs per element.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
+#include "elem_codec.cuh"
 #include "fft_core.cuh"
 #include "sm_internal.h"
 
@@ -27,56 +26,7 @@ using smfft::pf_make;
 constexpr int kTm = 64, kTn = 128, kKc = 32, kThreads = 256;
 constexpr int kRowsPerThread = 4, kColsPerThread = 8;
 
-template <int DT> struct LoraCodec;
-template <> struct LoraCodec<0> {                    // fp32
-  __device__ static float load(const void* p, size_t i) { return __ldg(reinterpret_cast<const float*>(p) + i); }
-  __device__ static void load8(const void* p, size_t i, float (&f)[8]) {
-    const float4* q = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p) + i);
-    const float4 a = __ldg(q), b = __ldg(q + 1);
-    f[0] = a.x; f[1] = a.y; f[2] = a.z; f[3] = a.w; f[4] = b.x; f[5] = b.y; f[6] = b.z; f[7] = b.w;
-  }
-  __device__ static void store(void* p, size_t i, float v) { reinterpret_cast<float*>(p)[i] = v; }
-  __device__ static void store8(void* p, size_t i, const float (&o)[8]) {
-    float4* q = reinterpret_cast<float4*>(reinterpret_cast<float*>(p) + i);
-    q[0] = make_float4(o[0], o[1], o[2], o[3]); q[1] = make_float4(o[4], o[5], o[6], o[7]);
-  }
-};
-template <> struct LoraCodec<1> {                    // bf16
-  __device__ static float h2f(uint32_t u) { return __uint_as_float(u << 16); }
-  __device__ static uint32_t f2h(float x) { __nv_bfloat16 h = __float2bfloat16_rn(x); return *reinterpret_cast<uint16_t*>(&h); }
-  __device__ static float load(const void* p, size_t i) { return h2f(__ldg(reinterpret_cast<const uint16_t*>(p) + i)); }
-  __device__ static void load8(const void* p, size_t i, float (&f)[8]) {
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(p) + i));
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int e = 0; e < 4; ++e) { f[2 * e] = h2f(w[e] & 0xffffu); f[2 * e + 1] = h2f(w[e] >> 16); }
-  }
-  __device__ static void store(void* p, size_t i, float v) { reinterpret_cast<uint16_t*>(p)[i] = (uint16_t)f2h(v); }
-  __device__ static void store8(void* p, size_t i, const float (&o)[8]) {
-    uint32_t w[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) w[e] = f2h(o[2 * e]) | (f2h(o[2 * e + 1]) << 16);
-    *reinterpret_cast<uint4*>(reinterpret_cast<uint16_t*>(p) + i) = make_uint4(w[0], w[1], w[2], w[3]);
-  }
-};
-template <> struct LoraCodec<2> {                    // fp16
-  __device__ static float h2f(uint32_t u) { const uint16_t s = (uint16_t)u; return __half2float(*reinterpret_cast<const __half*>(&s)); }
-  __device__ static uint32_t f2h(float x) { __half h = __float2half_rn(x); return *reinterpret_cast<uint16_t*>(&h); }
-  __device__ static float load(const void* p, size_t i) { return h2f(__ldg(reinterpret_cast<const uint16_t*>(p) + i)); }
-  __device__ static void load8(const void* p, size_t i, float (&f)[8]) {
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(p) + i));
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int e = 0; e < 4; ++e) { f[2 * e] = h2f(w[e] & 0xffffu); f[2 * e + 1] = h2f(w[e] >> 16); }
-  }
-  __device__ static void store(void* p, size_t i, float v) { reinterpret_cast<uint16_t*>(p)[i] = (uint16_t)f2h(v); }
-  __device__ static void store8(void* p, size_t i, const float (&o)[8]) {
-    uint32_t w[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) w[e] = f2h(o[2 * e]) | (f2h(o[2 * e + 1]) << 16);
-    *reinterpret_cast<uint4*>(reinterpret_cast<uint16_t*>(p) + i) = make_uint4(w[0], w[1], w[2], w[3]);
-  }
-};
+template <int DT> using LoraCodec = ElemCodec<DT>;
 
 struct LoraArgs {
   const void* base; const void* A; const void* B; void* out;

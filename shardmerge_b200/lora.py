@@ -13,12 +13,16 @@ For every base tensor W of the base the adapter is bound to, the finetune's tens
   - with a full tensor:    that tensor;
   - otherwise:             W itself.
 `Adapter.bind` checks every key and shape against the base and raises `UnsupportedAdapter` for what it cannot represent.
+`save_adapter` writes the same format (what `extract.extract_lora` produces).
 """
 from __future__ import annotations
 
 import json
 import math
+import os
 import re
+import shutil
+import tempfile
 from dataclasses import dataclass
 from pathlib import Path
 from typing import Dict, Optional, Tuple
@@ -138,6 +142,53 @@ class Adapter:
 
     def part(self, tensor_name: str) -> Part:
         return self.parts.get(tensor_name, BASE_PART)
+
+
+def save_adapter(directory, tensors: Dict[str, object], config: dict) -> None:
+    """Write a PEFT LoRA adapter that `Adapter.bind` reads back, every LoRA pair with scaling 1.0.
+
+    `tensors` maps a base tensor name to a (lora_A [r'][C], lora_B [R][r']) pair of contiguous CPU tensors, for a
+    `<module>.weight`, or to a contiguous CPU tensor stored whole (`modules_to_save`).  `config` gives `r` and
+    `base_model_name_or_path`; this function sets the rest: peft_type LORA, lora_alpha = r, an `alpha_pattern` entry
+    alpha = r' for every module whose r' < r, `target_modules` (the modules' last names), `modules_to_save`, and use_dora,
+    fan_in_fan_out and use_rslora false.  The directory appears complete or not at all: the files are written into a
+    temporary sibling that is renamed into place; `directory` may exist only if it is empty."""
+    from .writer import write_safetensors
+
+    directory = Path(directory)
+    if directory.exists() and (not directory.is_dir() or any(directory.iterdir())):
+        raise FileExistsError(f"{directory} exists and is not an empty directory")
+    r = int(config["r"])
+    weights: Dict[str, torch.Tensor] = {}
+    alpha_pattern: Dict[str, int] = {}
+    targets, full = set(), set()
+    for name, value in tensors.items():
+        if isinstance(value, tuple):
+            A, B = value
+            if not name.endswith(".weight") or A.ndim != 2 or B.ndim != 2 or A.shape[0] != B.shape[1] or not 1 <= A.shape[0] <= r:
+                raise ValueError(f"save_adapter: {name} needs lora_A [r'][C], lora_B [R][r'] with 1 <= r' <= {r}")
+            module = name[: -len(".weight")]
+            weights[f"{KEY_PREFIX}{module}.lora_A.weight"] = A
+            weights[f"{KEY_PREFIX}{module}.lora_B.weight"] = B
+            targets.add(module.rsplit(".", 1)[-1])
+            if A.shape[0] < r:
+                alpha_pattern[module] = int(A.shape[0])
+        else:
+            weights[KEY_PREFIX + name] = value
+            full.add(name.rsplit(".", 1)[0] if "." in name else name)
+    cfg = dict(config)
+    cfg.update({"peft_type": "LORA", "r": r, "lora_alpha": r, "alpha_pattern": alpha_pattern,
+                "target_modules": sorted(targets), "modules_to_save": sorted(full) or None,
+                "use_dora": False, "fan_in_fan_out": False, "use_rslora": False})
+    tmp = Path(tempfile.mkdtemp(prefix=f".{directory.name}.", dir=directory.parent))
+    try:
+        (tmp / CONFIG_FILE).write_text(json.dumps(cfg, indent=2, sort_keys=True))
+        write_safetensors(tmp / WEIGHTS_FILE, weights, metadata={"format": "pt"})
+        os.chmod(tmp, 0o755)
+        os.replace(tmp, directory)
+    except BaseException:
+        shutil.rmtree(tmp, ignore_errors=True)
+        raise
 
 
 def materialize(base: torch.Tensor, lora_A: torch.Tensor, lora_B: torch.Tensor, scaling: float) -> torch.Tensor:
