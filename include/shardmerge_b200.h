@@ -91,6 +91,7 @@ int sm_inv_norm(const double* sumsq, float* out, void* stream);
  * u32 hi, u32 ncand, u32 cap, u32 status, f32 value, u32 sticky}; `sticky` ORs the status of
  * every select that used this state since the caller last zeroed it. */
 #define SM_SELECT_STATE_BYTES 64
+#define SM_SELECT_STICKY_OFF 44
 size_t sm_select_ws_bytes(const sm_plan* plan, int n_planes, int mode);
 int sm_select_kth_abs(const sm_plan* plan, const float* plane0, const float* plane1, uint64_t rank,
                       int mode, void* sel_state, void* ws, size_t ws_bytes, float* thr_out, void* stream);
@@ -183,13 +184,14 @@ int sm_pack_half(const sm_plan* plan, const float* in_c64, float* re, float* im,
 
 /* ---- fused pair merge (no host synchronisation) ---------------------------------------------
  * The regular-layer body of FourierMerge._merge_layer (shard/merge/fast_fourier.py:147-276) for two
- * bf16 finetunes, issued as ONE stream-ordered chain from a single call: row passes -> device-side
+ * finetunes, issued as ONE stream-ordered chain from a single call: row passes -> device-side
  * decisions (which model is `a`, :212-215; branch, :223-244; target_norm, :165) -> column sweeps ->
  * cutoff statistic -> SLERP sums -> blend -> cull statistic -> inverse sweeps -> epilogue.
  * The chain always runs the SLERP branch; afterwards the scalar block tells the caller whether that
- * was right: ints[SM_I_BRANCH] != SM_BRANCH_SLERP, a non-zero status in either fused-statistics state
- * (SM_CTL_FS + k * SM_FS_STATE_BYTES + SM_FS_STATUS_OFF) or a non-zero `sticky` in either select state
- * (small tensors), or flags[1] / flags[3] (Inf) mean "redo this tensor on the step-by-step path / raise".
+ * was right: ints[SM_I_BRANCH] != SM_BRANCH_SLERP, a non-zero sticky word in either fused-statistics state
+ * (SM_CTL_FS + k * SM_FS_STATE_BYTES + SM_FS_STICKY_OFF) or in either select state (small tensors,
+ * SM_CTL_SEL + k * SM_SELECT_STATE_BYTES + SM_SELECT_STICKY_OFF), or flags[1] / flags[3] (Inf) mean
+ * "redo this tensor on the step-by-step path / raise".
  *
  * Scalar block layout (SM_CTL_BYTES device bytes, zeroed by the call): */
 #define SM_CTL_BYTES   1024
@@ -229,28 +231,21 @@ typedef struct sm_pair_args {
   double cutoff_pct, cull_pct;
   double target_norm_offset;
   int select_mode;                         /* 0 fast (sampled window), 1 safe                     */
+  /* One pair merge INSIDE the pairwise tree that FourierMerge._merge_layer builds for more than two finetunes
+   * (shard/merge/fast_fourier.py:171-254: round 1 merges pairs of deltas, later rounds merge the fp32 results, cull_pct
+   * halves per round, target_norm is the mean over ALL models' norms, :165).  Zero / NULL in a field keeps the plain
+   * two-finetune merge above: */
+  const float* x32_0; const float* x32_1;  /* non-NULL: that input is an fp32 [R][C] tensor (an earlier round's result)
+                                              instead of (base, ft)                                                      */
+  int rows_done;                           /* 1: the row passes of both inputs already ran into (re[k], im[k]) and
+                                              `sumsq` holds their sums of squares (round 1: the caller transforms every
+                                              model once, reads the norms, pairs them on the host, :180-186)             */
+  double sumsq[2];
+  double target_norm;                      /* > 0: use it instead of the mean of the two norms                         */
+  float* out_f32;                          /* non-NULL: write merged * target_norm as fp32 (no base add, no bf16 cast)  */
 } sm_pair_args;
 
-int sm_pair_merge_slerp_async(const sm_plan* plan, const void* tables, const sm_pair_args* args, void* stream);
-
-/* The same chain as one pair merge INSIDE the pairwise tree that FourierMerge._merge_layer builds for more than two
- * finetunes (shard/merge/fast_fourier.py:171-254: round 1 merges pairs of deltas, later rounds merge the fp32 results,
- * cull_pct halves per round, target_norm is the mean over ALL models' norms, :165).  `ext` adds what the tree needs:
- *   x32_0 / x32_1  non-NULL: that input is an fp32 [R][C] tensor (an earlier round's result) instead of (base, ft);
- *   rows_done      1: the row passes of both inputs already ran into (re[k], im[k]) and `sumsq` holds their sums of
- *                  squares (round 1: the caller transforms every model once, reads the norms, pairs them on the host
- *                  like correlated_pairs does, :180-186);
- *   target_norm    > 0: use it instead of the mean of the two norms;
- *   out_f32        non-NULL: write merged * target_norm as fp32 (no base add, no bf16 cast): an intermediate of the tree.
- * Branch / role decisions stay on the device as in sm_pair_merge_slerp_async. */
-typedef struct sm_pair_ext {
-  const float* x32_0; const float* x32_1;
-  int rows_done;
-  double sumsq[2];
-  double target_norm;
-  float* out_f32;
-} sm_pair_ext;
-int sm_pair_merge_tree_async(const sm_plan* plan, const void* tables, const sm_pair_args* args, const sm_pair_ext* ext, void* stream);
+int sm_pair_merge_async(const sm_plan* plan, const void* tables, const sm_pair_args* args, void* stream);
 
 /* Per-kernel-class CUDA-event timing of the fused chain (bench.py roofline).  Classes: */
 #define SM_CLS_ROW_FWD 0

@@ -53,8 +53,7 @@ SIGNATURES = {
     "sm_copy_bytes": (_i, [_vp, _vp, _sz, _vp]),
     "sm_expand_full": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "sm_pack_half": (_i, [_vp, _vp, _vp, _vp, _vp]),
-    "sm_pair_merge_slerp_async": (_i, [_vp, _vp, _vp, _vp]),
-    "sm_pair_merge_tree_async": (_i, [_vp, _vp, _vp, _vp, _vp]),
+    "sm_pair_merge_async": (_i, [_vp, _vp, _vp, _vp]),
     "sm_profile_enable": (_i, [_i]),
     "sm_profile_collect": (_i, [_vp, _vp, _vp, _i]),
 }
@@ -65,18 +64,22 @@ class PairArgs(C.Structure):
     _fields_ = [("base0", _vp), ("ft0", _vp), ("base1", _vp), ("ft1", _vp), ("base_out", _vp), ("out_bf16", _vp),
                 ("re", _vp * 3), ("im", _vp * 2), ("ctl", _vp), ("sel_ws", _vp), ("sel_ws_bytes", _sz),
                 ("t", _d), ("t_sum", _f), ("cutoff_pct", _d), ("cull_pct", _d), ("target_norm_offset", _d),
-                ("select_mode", _i)]
+                ("select_mode", _i), ("x32_0", _vp), ("x32_1", _vp), ("rows_done", _i), ("sumsq", _d * 2),
+                ("target_norm", _d), ("out_f32", _vp)]
 
 
-class PairExt(C.Structure):
-    """sm_pair_ext of include/shardmerge_b200.h"""
-    _fields_ = [("x32_0", _vp), ("x32_1", _vp), ("rows_done", _i), ("sumsq", _d * 2), ("target_norm", _d), ("out_f32", _vp)]
-
-
+# the scalar block of the fused pair merge and the statistics states inside it: the header's #defines, one to one
+SM_SELECT_STATE_BYTES, SM_SELECT_STICKY_OFF = 64, 44
+SM_FS_STATE_BYTES, SM_FS_STATUS_OFF, SM_FS_STICKY_OFF = 128, 28, 72
+SM_CTL_BYTES, SM_CTL_SUMSQ, SM_CTL_SUMS, SM_CTL_FLT, SM_CTL_FLAGS, SM_CTL_INT, SM_CTL_TN, SM_CTL_SEL, SM_CTL_FS = (
+    1024, 0, 16, 64, 128, 144, 160, 192, 512)
+SM_F_THR_CUT, SM_F_THR_CULL, SM_F_DOT, SM_F_SCALE_X, SM_F_SCALE_Y, SM_F_OUT_SCALE, SM_F_NORM_X, SM_F_NORM_Y = (
+    0, 1, 2, 6, 7, 8, 9, 10)
+SM_I_SWAP, SM_I_BRANCH = 0, 1
+SM_BRANCH_SLERP, SM_BRANCH_ADD, SM_BRANCH_ARITH, SM_BRANCH_EARLY, SM_BRANCH_LINEAR = 0, 1, 2, 3, 4
+BRANCH_NAMES = {SM_BRANCH_SLERP: "slerp", SM_BRANCH_ADD: "add", SM_BRANCH_ARITH: "arith", SM_BRANCH_EARLY: "slerp-early",
+                SM_BRANCH_LINEAR: "slerp-linear"}
 CLS_NAMES = ["row_fwd", "col_fwd", "stats_cutoff", "reduce", "scalars", "blend_cull", "select1", "col_inv", "row_inv"]
-BRANCH_NAMES = {0: "slerp", 1: "add", 2: "arith", 3: "slerp-early", 4: "slerp-linear"}
-SELECT_STATE_BYTES = 64
-FS_STATE_BYTES, FS_STATUS_OFF, FS_STICKY_OFF, CTL_FS_OFF, CTL_BYTES = 128, 28, 72, 512, 1024
 
 
 class ShardMergeLibraryError(RuntimeError):

@@ -28,6 +28,7 @@ struct SelState {              // must match SM_SELECT_STATE_BYTES / the header 
   unsigned int pad[4];
 };
 static_assert(sizeof(SelState) == SM_SELECT_STATE_BYTES, "SelState layout");
+static_assert(offsetof(SelState, sticky) == SM_SELECT_STICKY_OFF, "SelState sticky offset");
 
 __device__ __forceinline__ unsigned int absbits(float v) { return __float_as_uint(v) & 0x7fffffffu; }
 __device__ __forceinline__ int sgn(float v) { return (v > 0.f) - (v < 0.f); }   // torch.sign: NaN -> 0

@@ -85,18 +85,7 @@ extern "C" int sm_profile_collect(double* ms, double* bytes, int* launches, int 
   return 0;
 }
 
-static int pair_chain(const sm_plan* plan, const void* tables, const sm_pair_args* a, const sm_pair_ext* x, void* stream);
-
-extern "C" int sm_pair_merge_slerp_async(const sm_plan* plan, const void* tables, const sm_pair_args* a, void* stream) {
-  return pair_chain(plan, tables, a, nullptr, stream);
-}
-
-extern "C" int sm_pair_merge_tree_async(const sm_plan* plan, const void* tables, const sm_pair_args* a, const sm_pair_ext* x,
-                                        void* stream) {
-  return pair_chain(plan, tables, a, x, stream);
-}
-
-static int pair_chain(const sm_plan* plan, const void* tables, const sm_pair_args* a, const sm_pair_ext* x, void* stream) {
+extern "C" int sm_pair_merge_async(const sm_plan* plan, const void* tables, const sm_pair_args* a, void* stream) {
   const SmPlan& p = plan->p;
   cudaStream_t st = (cudaStream_t)stream;
   const double N = (double)p.R * (double)p.C;
@@ -111,21 +100,21 @@ static int pair_chain(const sm_plan* plan, const void* tables, const sm_pair_arg
   const int col_launches = sm_plan_col_launches(plan);
   int rc;
   SM_CUDA_CHECK(cudaMemsetAsync(ctl, 0, SM_CTL_BYTES, st));
-  const bool rows_done = x != nullptr && x->rows_done != 0;
+  const bool rows_done = a->rows_done != 0;
   if (!rows_done) {
     // bf16 (base, finetune) pairs: 2N + 2N read, 4N written; fp32 tree intermediates: 4N read, 4N written
     Scope s(st, SM_CLS_ROW_FWD, 16.0 * N, 2);
-    if (x != nullptr && x->x32_0 != nullptr) {
-      if ((rc = sm_fwd_rows_f32(plan, tables, x->x32_0, 1.f, 1.f, a->re[0], a->im[0], dbl + 0, st))) return rc;
+    if (a->x32_0 != nullptr) {
+      if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_0, 1.f, 1.f, a->re[0], a->im[0], dbl + 0, st))) return rc;
     } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base0, a->ft0, a->re[0], a->im[0], dbl + 0, st))) return rc;
-    if (x != nullptr && x->x32_1 != nullptr) {
-      if ((rc = sm_fwd_rows_f32(plan, tables, x->x32_1, 1.f, 1.f, a->re[1], a->im[1], dbl + 1, st))) return rc;
+    if (a->x32_1 != nullptr) {
+      if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_1, 1.f, 1.f, a->re[1], a->im[1], dbl + 1, st))) return rc;
     } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base1, a->ft1, a->re[1], a->im[1], dbl + 1, st))) return rc;
   }
   {
     Scope s(st, SM_CLS_SCALARS, 0.0, 1);
-    sm_launch(k_prepare, dim3(1), dim3(1), (size_t)(0), st, ctl, a->target_norm_offset, x ? x->target_norm : 0.0, rows_done ? 1 : 0,
-                               rows_done ? x->sumsq[0] : 0.0, rows_done ? x->sumsq[1] : 0.0);
+    sm_launch(k_prepare, dim3(1), dim3(1), (size_t)(0), st, ctl, a->target_norm_offset, a->target_norm, rows_done ? 1 : 0,
+                               rows_done ? a->sumsq[0] : 0.0, rows_done ? a->sumsq[1] : 0.0);
     SM_LAUNCH_CHECK();
   }
   {
@@ -183,10 +172,10 @@ static int pair_chain(const sm_plan* plan, const void* tables, const sm_pair_arg
   }
   {
     Scope s(st, SM_CLS_ROW_INV, 8.0 * N, 1);
-    if (x != nullptr && x->out_f32 != nullptr) {
+    if (a->out_f32 != nullptr) {
       // an intermediate of the pair tree: merged * target_norm as fp32, the base is added after the last round only
       if ((rc = sm_inv_rows_f32_sel(plan, tables, a->re[2], a->im[0], a->im[1], swap, cull ? flt + SM_F_THR_CULL : nullptr,
-                                    x->out_f32, flt + SM_F_OUT_SCALE, 1.f, 1, flags, st))) return rc;
+                                    a->out_f32, flt + SM_F_OUT_SCALE, 1.f, 1, flags, st))) return rc;
     } else if ((rc = sm_inv_rows_bf16_sel(plan, tables, a->re[2], a->im[0], a->im[1], swap, cull ? flt + SM_F_THR_CULL : nullptr,
                                           a->base_out, a->out_bf16, flt + SM_F_OUT_SCALE, 1.f, 1, flags, st))) return rc;
   }

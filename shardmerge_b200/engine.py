@@ -25,13 +25,13 @@ import torch
 
 from . import _lib
 
-# offsets inside the per-workspace scalar block (bytes)
-_CTL_BYTES = _lib.CTL_BYTES
-_OFF_DBL, _OFF_FLT, _OFF_FLAGS, _OFF_SEL = 0, 64, 128, 192
-# float64 slots
-D_SUMSQ0, D_SUMSQ1, D_S00, D_S11, D_S01 = 0, 1, 2, 3, 4
-# float32 slots
-F_THR_CUT, F_THR_CULL, F_DOT, F_COS, F_SIN, F_RELNORM, F_INV0, F_INV1 = 0, 1, 2, 3, 4, 5, 6, 7
+# slots of the scalar block (_lib mirrors its layout from include/shardmerge_b200.h): float64 from SM_CTL_SUMSQ ...
+D_SUMSQ0, D_SUMSQ1 = 0, 1
+D_S00 = (_lib.SM_CTL_SUMS - _lib.SM_CTL_SUMSQ) // 8
+D_S11, D_S01 = D_S00 + 1, D_S00 + 2
+# ... and float32 from SM_CTL_FLT (cos, sin, relnorm follow dot: scal4 of sm_slerp_scalars)
+F_THR_CUT, F_THR_CULL, F_DOT = _lib.SM_F_THR_CUT, _lib.SM_F_THR_CULL, _lib.SM_F_DOT
+F_COS, F_SIN, F_RELNORM = F_DOT + 1, F_DOT + 2, F_DOT + 3
 
 
 class UnsupportedShape(ValueError):
@@ -172,11 +172,8 @@ class Workspace:
         self.re = [torch.zeros((plan.R, plan.P), dtype=torch.float32, device=dev) for _ in range(n_spectra)]
         self.im = [torch.zeros((plan.R, plan.P), dtype=torch.float32, device=dev) for _ in range(n_spectra)]
         self.re_out = torch.zeros((plan.R, plan.P), dtype=torch.float32, device=dev)   # blend output of the fused chain
-        self.ctl = torch.zeros(_CTL_BYTES, dtype=torch.uint8, device=dev)
-        self.dbl = self.ctl[_OFF_DBL:_OFF_DBL + 64].view(torch.float64)
-        self.flt = self.ctl[_OFF_FLT:_OFF_FLT + 64].view(torch.float32)
-        self.flags = self.ctl[_OFF_FLAGS:_OFF_FLAGS + 16].view(torch.int32)
-        self.sel = self.ctl[_OFF_SEL:_OFF_SEL + 128]
+        self.ctl = torch.zeros(_lib.SM_CTL_BYTES, dtype=torch.uint8, device=dev)
+        self.dbl, self.flt, self.flags, _, _, self.sel = ctl_views(self.ctl)
         self.safe_select = safe_select
         mode = 1 if safe_select else 0
         # select scratch in front, the fused statistics' persistent histograms behind it (sm_fstats_* uses the LAST
@@ -185,20 +182,18 @@ class Workspace:
         nbytes = (nbytes + 255) // 256 * 256 + plan.lib.sm_fstats_ws_bytes(plan.handle)
         self.sel_ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
         # pinned landing zone for the scalar block
-        self.ctl_host = torch.empty(_CTL_BYTES, dtype=torch.uint8).pin_memory()
+        self.ctl_host = torch.empty(_lib.SM_CTL_BYTES, dtype=torch.uint8).pin_memory()
 
     # typed pointers into the scalar block
     def dptr(self, slot): return self.dbl.data_ptr() + 8 * slot
     def fptr(self, slot): return self.flt.data_ptr() + 4 * slot
-    def selptr(self, which): return self.sel.data_ptr() + 64 * which
-    def fsptr(self, which): return self.ctl.data_ptr() + _lib.CTL_FS_OFF + _lib.FS_STATE_BYTES * which
+    def selptr(self, which): return self.sel.data_ptr() + _lib.SM_SELECT_STATE_BYTES * which
+    def fsptr(self, which): return self.ctl.data_ptr() + _lib.SM_CTL_FS + _lib.SM_FS_STATE_BYTES * which
 
     def fs_status(self):
-        """(status of the fused cutoff state, status of the fused blend/cull state) -- synchronous."""
+        """(sticky word of the fused cutoff state, sticky word of the fused blend/cull state) -- synchronous."""
         h = self.ctl.cpu()
-        o = _lib.CTL_FS_OFF + _lib.FS_STICKY_OFF
-        return (int(h[o:o + 4].view(torch.int32)[0]),
-                int(h[o + _lib.FS_STATE_BYTES:o + _lib.FS_STATE_BYTES + 4].view(torch.int32)[0]))
+        return tuple(_word(h, o) for o in _FS_STICKY)
 
     def select_sticky(self) -> int:
         """Sticky status of every order statistic since `ctl` was zeroed, as of the last read_ctl(): non-zero when a sampled
@@ -210,19 +205,36 @@ class Workspace:
         """Synchronous read-back of the scalar block -> (float64[8], float32[16], int32[4], sel bytes)."""
         self.ctl_host.copy_(self.ctl, non_blocking=True)
         torch.cuda.current_stream(self.plan.device).synchronize()
-        h = self.ctl_host
-        return (h[_OFF_DBL:_OFF_DBL + 64].view(torch.float64), h[_OFF_FLT:_OFF_FLT + 64].view(torch.float32),
-                h[_OFF_FLAGS:_OFF_FLAGS + 16].view(torch.int32), h[_OFF_SEL:_OFF_SEL + 128])
+        dbl, flt, flags, _, _, sel = ctl_views(self.ctl_host)
+        return dbl, flt, flags, sel
+
+
+def ctl_views(h: torch.Tensor):
+    """Views of a scalar block `h` (uint8, on the device or a host copy) as include/shardmerge_b200.h lays it out:
+    (float64 from SM_CTL_SUMSQ: the sums of squares of x and y, then the SLERP sums (D_*); float32 slots SM_F_*; the u32
+    nan / inf counters as int32; int32 slots SM_I_*; float64 target_norm; the bytes of the two select states)."""
+    L = _lib
+    return (h[L.SM_CTL_SUMSQ:L.SM_CTL_FLT].view(torch.float64), h[L.SM_CTL_FLT:L.SM_CTL_FLAGS].view(torch.float32),
+            h[L.SM_CTL_FLAGS:L.SM_CTL_INT].view(torch.int32), h[L.SM_CTL_INT:L.SM_CTL_TN].view(torch.int32),
+            h[L.SM_CTL_TN:L.SM_CTL_TN + 8].view(torch.float64), h[L.SM_CTL_SEL:L.SM_CTL_SEL + 2 * L.SM_SELECT_STATE_BYTES])
+
+
+# byte offsets of the sticky words of the two select states and of the two fused statistics states
+_SEL_STICKY = [_lib.SM_CTL_SEL + k * _lib.SM_SELECT_STATE_BYTES + _lib.SM_SELECT_STICKY_OFF for k in (0, 1)]
+_FS_STICKY = [_lib.SM_CTL_FS + k * _lib.SM_FS_STATE_BYTES + _lib.SM_FS_STICKY_OFF for k in (0, 1)]
+
+
+def _word(h: torch.Tensor, off: int) -> int:
+    return int(h[off:off + 4].view(torch.int32)[0])
 
 
 def select_sticky_of(h: torch.Tensor) -> int:
-    """OR of the sticky words of the two select states (int32 slots 11 and 27 of `sel`) and of the two fused statistics
-    states in a host copy `h` (uint8) of a scalar block."""
-    sel32 = h[_OFF_SEL:_OFF_SEL + 128].view(torch.int32)
-    fs = _lib.CTL_FS_OFF + _lib.FS_STICKY_OFF
-    fs0 = int(h[fs:fs + 4].view(torch.int32)[0])
-    fs1 = int(h[fs + _lib.FS_STATE_BYTES:fs + _lib.FS_STATE_BYTES + 4].view(torch.int32)[0])
-    return int(sel32[11]) | int(sel32[16 + 11]) | fs0 | fs1
+    """OR of the sticky words of the two select states and of the two fused statistics states in a host copy `h`
+    (uint8) of a scalar block."""
+    sticky = 0
+    for off in _SEL_STICKY + _FS_STICKY:
+        sticky |= _word(h, off)
+    return sticky
 
 
 _plans: dict = {}
@@ -321,7 +333,6 @@ def make_source(base: Optional[torch.Tensor], ft: Optional[torch.Tensor], x32: O
 # kernel wrappers
 # ------------------------------------------------------------------------------------------
 def fwd_rows(ws: Workspace, slot: int, src: Source, sumsq_slot: int, m1: float = 1.0, m2: float = 1.0):
-    pl, lib = ws.plan, ws.plan.lib
     fwd_rows_ptr(ws, slot, src, ws.dptr(sumsq_slot), m1, m2)
 
 
@@ -537,7 +548,7 @@ class _PinnedPool:
 
     def take(self) -> torch.Tensor:
         if not self.free:
-            buf = torch.empty((self.CHUNK, _CTL_BYTES), dtype=torch.uint8).pin_memory()
+            buf = torch.empty((self.CHUNK, _lib.SM_CTL_BYTES), dtype=torch.uint8).pin_memory()
             self.chunks.append(buf)
             self.free.extend(buf[i] for i in range(self.CHUNK))
         return self.free.pop()
@@ -586,12 +597,11 @@ class PendingPair:
             return self.info
         self.event.synchronize()
         h = self.host_ctl
-        dbl = h[0:64].view(torch.float64); flt = h[64:128].view(torch.float32)
-        flags = h[128:144].view(torch.int32); ints = h[144:160].view(torch.int32)
-        self.info = dict(norms=[float(flt[9]), float(flt[10])], target_norm=float(h[160:168].view(torch.float64)[0]),
-                         swap=int(ints[0]), branch=_lib.BRANCH_NAMES.get(int(ints[1]), "?"),
+        _, flt, flags, ints, tn, _ = ctl_views(h)
+        self.info = dict(norms=[float(flt[_lib.SM_F_NORM_X]), float(flt[_lib.SM_F_NORM_Y])], target_norm=float(tn[0]),
+                         swap=int(ints[_lib.SM_I_SWAP]), branch=_lib.BRANCH_NAMES.get(int(ints[_lib.SM_I_BRANCH]), "?"),
                          select_sticky=select_sticky_of(h), flags=[int(v) for v in flags],
-                         thr_cut=float(flt[0]), thr_cull=float(flt[1]), dot=float(flt[2]))
+                         thr_cut=float(flt[F_THR_CUT]), thr_cull=float(flt[F_THR_CULL]), dot=float(flt[F_DOT]))
         _ring.give(h)
         self.host_ctl = None
         return self.info
@@ -609,24 +619,22 @@ def pair_merge_async(ws: Workspace, s0: Source, s1: Source, base_out: Optional[t
     pl, lib = ws.plan, ws.plan.lib
     dev = pl.device
     a = _lib.PairArgs()
-    x = _lib.PairExt()
-    use_ext = rows_done or target_norm > 0 or out.dtype == torch.float32 or not s0.is_bf16 or not s1.is_bf16
     if s0.is_bf16:
         a.base0, a.ft0 = s0.base.data_ptr(), s0.ft.data_ptr()
     else:
-        x.x32_0 = s0.x32.data_ptr()
+        a.x32_0 = s0.x32.data_ptr()
     if s1.is_bf16:
         a.base1, a.ft1 = s1.base.data_ptr(), s1.ft.data_ptr()
     else:
-        x.x32_1 = s1.x32.data_ptr()
+        a.x32_1 = s1.x32.data_ptr()
     if out.dtype == torch.bfloat16:
         a.base_out, a.out_bf16 = base_out.data_ptr(), out.data_ptr()
     else:
-        x.out_f32 = out.data_ptr()
-    x.rows_done = 1 if rows_done else 0
+        a.out_f32 = out.data_ptr()
+    a.rows_done = 1 if rows_done else 0
     if rows_done:
-        x.sumsq[0], x.sumsq[1] = float(sumsq[0]), float(sumsq[1])
-    x.target_norm = float(target_norm)
+        a.sumsq[0], a.sumsq[1] = float(sumsq[0]), float(sumsq[1])
+    a.target_norm = float(target_norm)
     a.re[0], a.re[1], a.re[2] = ws.re[slots[0]].data_ptr(), ws.re[slots[1]].data_ptr(), ws.re_out.data_ptr()
     a.im[0], a.im[1] = ws.im[slots[0]].data_ptr(), ws.im[slots[1]].data_ptr()
     a.ctl = ws.ctl.data_ptr()
@@ -640,11 +648,7 @@ def pair_merge_async(ws: Workspace, s0: Source, s1: Source, base_out: Optional[t
         cl = lib.sm_plan_col_launches(pl.handle)          # launches of one column transform (column bands x sweeps)
         PROFILER.launches += (0 if rows_done else 2) + 1 + 2 * cl + ((2 + 2) if fs else (11 + 2 + 1 + 11)) + (cl if sweeps else 0) + 1
         PROFILER.fused_calls += 1
-    if use_ext:
-        rc = lib.sm_pair_merge_tree_async(pl.handle, pl.tables.data_ptr(), ctypes.byref(a), ctypes.byref(x), _stream(dev))
-    else:
-        rc = lib.sm_pair_merge_slerp_async(pl.handle, pl.tables.data_ptr(), ctypes.byref(a), _stream(dev))
-    _lib.check(rc, "sm_pair_merge_async")
+    _lib.check(lib.sm_pair_merge_async(pl.handle, pl.tables.data_ptr(), ctypes.byref(a), _stream(dev)), "sm_pair_merge_async")
     if _ring is None:
         _ring = _PinnedPool()
     host = _ring.take()

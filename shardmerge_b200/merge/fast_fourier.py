@@ -18,7 +18,7 @@ import asyncio
 import hashlib
 import logging
 import os
-from typing import List, Optional
+from typing import List, NamedTuple, Optional
 
 import torch
 
@@ -26,7 +26,7 @@ from .. import engine as E
 from .. import lora
 from ..config import MergeConfig
 from ..constants import INPUT_LAYER, OUTPUT_LAYER
-from ..tensor.functions import correlated_pairs
+from ..tensor.functions import correlated_pairs, retry_on_select_miss
 from .base import MergeTensorsBase
 
 logger = logging.getLogger(__name__)
@@ -46,6 +46,36 @@ def task_arithmetic(t0: torch.Tensor, t1: torch.Tensor) -> torch.Tensor:
 
 def clamp(value: float, min_value: float, max_value: float) -> float:
     return max(min_value, min(value, max_value))
+
+
+class TreeStep(NamedTuple):
+    """One entry of a round of the pair tree, in the order correlated_pairs yields it (the order of the next round's
+    stack).  y = -1: the model at x is carried to the next round unmerged (a_w is its weight, b_w is 0)."""
+    x: int
+    y: int
+    a_w: float
+    b_w: float
+    cull_pct: float
+    last: bool           # the pair of the last round: it gives the merged tensor
+
+
+def tree_plan(sumsq: List[float], weights: List[float], cull_start_pct: float, target_norm_offset: float):
+    """The schedule of the pairwise tree of fast_fourier.py:165-254 -> (fp32 norms, target_norm, rounds of TreeSteps).
+    The reference pairs every round by the products of the ORIGINAL norms list (stale after round 1, :180-184), so the
+    whole schedule follows from the models' sums of squares of delta and their weights."""
+    norms = [E.f32(v ** 0.5) for v in sumsq]
+    target_norm = torch.tensor(norms, dtype=torch.float32).mean().item() + target_norm_offset      # fp32 mean, :165
+    nt = torch.tensor(norms, dtype=torch.float32)
+    rounds, w, cull_pct = [], list(weights), cull_start_pct
+    while len(w) > 1:
+        n = len(w)
+        corr = torch.triu(nt[:n, None] * nt[None, :n], diagonal=1)                                 # fp32 products
+        steps = [TreeStep(x, y, w[x], w[y] if y >= 0 else 0.0, cull_pct, n == 2)
+                 for x, y, _ in correlated_pairs(corr, way="least")]
+        rounds.append(steps)
+        w = [s.a_w if s.y < 0 else (s.a_w + s.b_w) / 2.0 for s in steps]
+        cull_pct = cull_pct / 2.0                                                                  # :254
+    return norms, target_norm, rounds
 
 
 class _PendingTree:
@@ -94,7 +124,6 @@ class FourierMerge(MergeTensorsBase):
         self.defer_checks = False        # True inside merge(): _merge_layer returns before the check
         self._lane_streams: dict = {}    # device index -> [streams]
         self._lane_next = 0
-        self.fused_tree = True           # False: pair trees (3+ finetunes) run on the step-by-step path
         self._tree_waiting: list = []    # pair trees whose row passes are enqueued but whose norms have not been read yet
         self.keep_intermediates = False  # tests: keep the tree's fp32 round results in self.last_tree
         self.last_tree: list = []
@@ -261,7 +290,7 @@ class FourierMerge(MergeTensorsBase):
             return merged_t.t().contiguous()
         all_bf16 = (not safe_select and base_out.dtype == torch.bfloat16 and base_out.ndim in (1, 2)
                     and all(src.is_bf16 for src in sources))
-        is_tree = all_bf16 and 3 <= len(sources) <= 120 and self.fused_tree
+        is_tree = all_bf16 and 3 <= len(sources) <= 120
         if self._tree_waiting and not is_tree:
             # a pair tree whose norms have not been read yet keeps its row spectra in its lane's workspace: enqueue its
             # pair merges before anything else may be given that lane
@@ -277,21 +306,13 @@ class FourierMerge(MergeTensorsBase):
         out = torch.empty(base_out.shape, dtype=torch.bfloat16, device=dev)
         a_w, b_w = sources[0].weight, sources[1].weight
         base_c = base_out.contiguous()
-        kwargs = dict(t=a_w / (a_w + b_w), t_sum=1.0, cutoff_pct=0.08, cull_pct=self.cull_start_pct,
-                      target_norm_offset=self.target_norm_offset, layer_name=layer_name)
-        if self.lanes > 1 and defer:
-            # the chain runs on this tensor's lane; the caller's stream is not made to wait for it -- whoever
-            # consumes `out` does so after resolve (a host-side wait for the lane's last event)
-            lane_i, lane = self._next_lane(dev)
-            ws = E.get_workspace(R, C, dev, n_spectra=2, lane=lane_i)
-            lane.wait_event(torch.cuda.current_stream(dev).record_event())      # inputs are ready on the caller's stream
-            with torch.cuda.stream(lane):
-                pend = E.pair_merge_async(ws, sources[0], sources[1], base_c, out, **kwargs)
-            for t_ in (out, base_c, sources[0].base, sources[0].ft, sources[1].base, sources[1].ft):
-                t_.record_stream(lane)
-        else:
-            ws = E.get_workspace(R, C, dev, n_spectra=2)
-            pend = E.pair_merge_async(ws, sources[0], sources[1], base_c, out, **kwargs)
+        # on a lane the caller's stream is not made to wait for the chain -- whoever consumes `out` does so after
+        # resolve (a host-side wait for the lane's last event)
+        ws, lane = self._lane_workspace(dev, defer, R, C, 2, [out, base_c] + [t for src in sources for t in (src.base, src.ft)])
+        with torch.cuda.stream(lane):
+            pend = E.pair_merge_async(ws, sources[0], sources[1], base_c, out, t=a_w / (a_w + b_w), t_sum=1.0,
+                                      cutoff_pct=0.08, cull_pct=self.cull_start_pct,
+                                      target_norm_offset=self.target_norm_offset, layer_name=layer_name)
         pend.redo = lambda: self._merge_sources_steps(sources, base_out, dev, layer_name, False)
         if defer:
             self.pending.append(pend)
@@ -299,13 +320,26 @@ class FourierMerge(MergeTensorsBase):
         self._resolve(pend)
         return out
 
-    def _next_lane(self, dev):
-        streams = self._lane_streams.get(dev.index)
-        if streams is None:
-            streams = self._lane_streams[dev.index] = [torch.cuda.Stream(device=dev) for _ in range(self.lanes)]
-        lane_i = self._lane_next % self.lanes
-        self._lane_next += 1
-        return lane_i, streams[lane_i]
+    def _lane_workspace(self, dev, defer: bool, R: int, C: int, n_spectra: int, tensors):
+        """(workspace, stream) for one tensor's fused chains.  Deferred with several lanes, consecutive tensors take turns
+        on the lane streams: the lane waits for the caller's stream (the inputs and a new workspace are ready there) and
+        `tensors` are recorded on it, so their memory is not reused before the lane is done.  Otherwise: lane 0 on the
+        caller's stream."""
+        caller = torch.cuda.current_stream(dev)
+        lane_i, lane = 0, caller
+        if self.lanes > 1 and defer:
+            streams = self._lane_streams.get(dev.index)
+            if streams is None:
+                streams = self._lane_streams[dev.index] = [torch.cuda.Stream(device=dev) for _ in range(self.lanes)]
+            lane_i = self._lane_next % self.lanes
+            self._lane_next += 1
+            lane = streams[lane_i]
+        ws = E.get_workspace(R, C, dev, n_spectra=n_spectra, lane=lane_i)
+        if lane is not caller:
+            lane.wait_event(caller.record_event())
+            for t in tensors:
+                t.record_stream(lane)
+        return ws, lane
 
     # -------------------------------------------------------------------------------------
     def _merge_sources_tree(self, sources: List[E.Source], base_out: torch.Tensor, dev, layer_name: str = "",
@@ -320,15 +354,9 @@ class FourierMerge(MergeTensorsBase):
         M = len(sources)
         out = torch.empty(base_out.shape, dtype=torch.bfloat16, device=dev)
         base_c = base_out.contiguous()
-        caller = torch.cuda.current_stream(dev)
-        if self.lanes > 1 and defer:
-            lane_i, lane = self._next_lane(dev)
-            lane.wait_event(caller.record_event())               # inputs are ready on the caller's stream
-        else:
-            lane_i, lane = 0, caller
+        ws, lane = self._lane_workspace(dev, defer, R, C, M, [out, base_c] + [t for src in sources for t in (src.base, src.ft)])
         # ---- phase A (enqueue only): every model's row pass, the sums of squares on their way to pinned host memory
         with torch.cuda.stream(lane):
-            ws = E.get_workspace(R, C, dev, n_spectra=M, lane=lane_i)
             sums = torch.zeros(M, dtype=torch.float64, device=dev)
             for i, src in enumerate(sources):
                 E.fwd_rows_ptr(ws, i, src, sums.data_ptr() + 8 * i)
@@ -337,9 +365,6 @@ class FourierMerge(MergeTensorsBase):
             sums_host.copy_(sums, non_blocking=True)
             sums_ready = torch.cuda.Event()
             sums_ready.record(lane)
-        if lane is not caller:
-            for t_ in [out, base_c] + [t for src in sources for t in (src.base, src.ft)]:
-                t_.record_stream(lane)
         pend = _PendingTree(out, [], layer_name, None, None)
 
         # ---- phase B: the one host wait (norms), pairing on the host, every pair merge as a fused chain on the lane
@@ -347,45 +372,33 @@ class FourierMerge(MergeTensorsBase):
             sums_ready.synchronize()
             sumsq = sums_host.tolist()
             E.give_pinned_slot(slot)
-            norms = [E.f32(v ** 0.5) for v in sumsq]
-            target_norm = torch.tensor(norms, dtype=torch.float32).mean().item() + self.target_norm_offset   # :165
+            norms, target_norm, rounds = tree_plan(sumsq, [src.weight for src in sources], self.cull_start_pct,
+                                                   self.target_norm_offset)
             pend.norms, pend.target_norm = norms, target_norm
             with torch.cuda.stream(lane):
                 # stack entry: (source, slot holding its row spectrum or None, sum of squares or None)
                 stack = [(src, i, sumsq[i]) for i, src in enumerate(sources)]
-                weights = [src.weight for src in sources]
-                cull_pct = self.cull_start_pct
                 kept = []
-                while len(stack) > 1:
-                    n = len(stack)
-                    corr = torch.zeros((n, n), dtype=torch.float32)
-                    for i in range(n):
-                        for j in range(i + 1, n):
-                            corr[i, j] = torch.tensor(norms[i], dtype=torch.float32) * torch.tensor(norms[j], dtype=torch.float32)
-                    pairs = list(correlated_pairs(corr, way="least"))
-                    last_round = len(pairs) == 1 and pairs[0][1] >= 0
-                    nxt, nxt_w = [], []
-                    for x, y, _ in pairs:
-                        if y < 0:
-                            src, _, _ = stack[x]
-                            nxt.append((src, None, None)); nxt_w.append(weights[x])   # carried over; its rows are redone when it is paired
+                for steps in rounds:
+                    nxt = []
+                    for st in steps:
+                        if st.y < 0:
+                            nxt.append((stack[st.x][0], None, None))    # carried over; its rows are redone when it is paired
                             continue
-                        (sa, slot_a, ss_a), (sb, slot_b, ss_b) = stack[x], stack[y]
-                        a_w, b_w = weights[x], weights[y]
+                        (sa, slot_a, ss_a), (sb, slot_b, ss_b) = stack[st.x], stack[st.y]
                         rows_done = slot_a is not None and slot_b is not None
-                        res = out if last_round else torch.empty((R, C), dtype=torch.float32, device=dev)
+                        res = out if st.last else torch.empty((R, C), dtype=torch.float32, device=dev)
                         pend.parts.append(E.pair_merge_async(
-                            ws, sa, sb, base_c, res, t=a_w / (a_w + b_w), t_sum=1.0, cutoff_pct=0.08, cull_pct=cull_pct,
-                            target_norm_offset=self.target_norm_offset, layer_name=layer_name,
+                            ws, sa, sb, base_c, res, t=st.a_w / (st.a_w + st.b_w), t_sum=1.0, cutoff_pct=0.08,
+                            cull_pct=st.cull_pct, target_norm_offset=self.target_norm_offset, layer_name=layer_name,
                             slots=(slot_a, slot_b) if rows_done else (0, 1), rows_done=rows_done,
                             sumsq=(ss_a, ss_b) if rows_done else None, target_norm=target_norm))
-                        if not last_round:
-                            inter = E.Source(x32=res, weight=(a_w + b_w) / 2.0, name=name_hash(f"{sa.name}_{sb.name}"))
-                            nxt.append((inter, None, None)); nxt_w.append((a_w + b_w) / 2.0)
+                        if not st.last:
+                            inter = E.Source(x32=res, weight=(st.a_w + st.b_w) / 2.0, name=name_hash(f"{sa.name}_{sb.name}"))
+                            nxt.append((inter, None, None))
                             if self.keep_intermediates:
                                 kept.append((sa.name, sb.name, res))
-                    stack, weights = nxt, nxt_w
-                    cull_pct = cull_pct / 2.0                         # :254
+                    stack = nxt
             if self.keep_intermediates:
                 self.last_tree = kept
 
@@ -433,6 +446,11 @@ class FourierMerge(MergeTensorsBase):
         """Step-by-step path: any number of models, any branch, host decisions between the stages."""
         if len(sources) == 0:
             raise IndexError("list index out of range")      # what the reference does with no applicable model
+        return retry_on_select_miss(lambda safe: self._steps_pass(sources, base_out, dev, layer_name, safe),
+                                    f"on {layer_name}", safe_select)
+
+    def _steps_pass(self, sources: List[E.Source], base_out: torch.Tensor, dev, layer_name: str, safe_select: bool):
+        """One run of the step path -> (merged tensor or None, sticky status of its order statistics)."""
         R, C = E.shape_rc(base_out)              # a tensor with leading dimensions is a stack of slices: all its rows
         base_bf16 = base_out if base_out.dtype == torch.bfloat16 else None
         # its own workspace (lane "steps"): a redo or a 1 / 3+ model tensor runs on the caller's stream while fused
@@ -444,44 +462,30 @@ class FourierMerge(MergeTensorsBase):
 
         # row passes of every model: delta, row FFT, sum of squares -> norms in one read-back
         extra = torch.zeros(max(len(sources), 2), dtype=torch.float64, device=dev)
-        sumsq_ptrs = [extra.data_ptr() + 8 * i for i in range(len(sources))]
         for i, s in enumerate(sources):
-            _rows_into(ws, i, s, sumsq_ptrs[i])
-        norms = [E.f32(v ** 0.5) for v in extra.to("cpu").tolist()[: len(sources)]]
+            E.fwd_rows_ptr(ws, i, s, extra.data_ptr() + 8 * i)
+        norms, target_norm, rounds = tree_plan(extra.to("cpu").tolist()[: len(sources)], [s.weight for s in sources],
+                                               self.cull_start_pct, self.target_norm_offset)
         for s, n in zip(sources, norms):
             s.norm = n
         info["norms"] = list(norms)
-        # torch.tensor(layer_norms).mean() is an fp32 mean (fast_fourier.py:165)
-        target_norm = torch.tensor(norms, dtype=torch.float32).mean().item() + self.target_norm_offset
         info["target_norm"] = target_norm
-        cull_pct = self.cull_start_pct
 
         if len(sources) == 1:
             # loop skipped: result = raw delta, alpha ignored (fast_fourier.py:171,256-257)
-            return _finish_elementwise(sources[0], None, 1.0, 0.0, 1.0, base_out, ws)
+            return _finish_elementwise(sources[0], None, 1.0, 0.0, 1.0, base_out, ws), 0
 
         # stack entries: (source, slot of its row spectrum or None)
         stack = [(s, i) for i, s in enumerate(sources)]
-        weights = [s.weight for s in sources]
-        stale_norms = list(norms)
         out_final: Optional[torch.Tensor] = None
-        while len(stack) > 1:
-            n = len(stack)
-            corr = torch.zeros((n, n), dtype=torch.float32)
-            for i in range(n):
-                for j in range(i + 1, n):
-                    # the reference multiplies the ORIGINAL layer_norms list (stale after round 1, :180-184)
-                    corr[i, j] = torch.tensor(stale_norms[i], dtype=torch.float32) * torch.tensor(stale_norms[j], dtype=torch.float32)
-            nxt, nxt_w = [], []
-            pairs = list(correlated_pairs(corr, way="least"))
-            n_pairs = sum(1 for _, y, _ in pairs if y >= 0)
-            last_round = (n_pairs == 1 and len(pairs) == 1)
-            for x, y, _ in pairs:
-                if y < 0:
-                    nxt.append(stack[x]); nxt_w.append(weights[x])
+        for steps in rounds:
+            nxt = []
+            for st in steps:
+                if st.y < 0:
+                    nxt.append(stack[st.x])
                     continue
-                (sa, slot_a), (sb, slot_b) = stack[x], stack[y]
-                a_w, b_w = weights[x], weights[y]
+                (sa, slot_a), (sb, slot_b) = stack[st.x], stack[st.y]
+                a_w, b_w = st.a_w, st.b_w
                 # intermediates of an earlier round have no row spectrum yet: run their row pass into a
                 # slot nobody in the current stack still needs (norm_a/norm_b of :209-210 come with it)
                 busy = {sl for _, sl in stack if sl is not None} | {sl for _, sl in nxt if sl is not None}
@@ -498,7 +502,7 @@ class FourierMerge(MergeTensorsBase):
                     sa, sb, slot_a, slot_b, na, nb = sb, sa, slot_b, slot_a, nb, na
                 cnorm_a, cnorm_b = abs(na / target_norm), abs(nb / target_norm)
                 n_ratio = cnorm_b / (cnorm_a + 1e-10)
-                final = last_round
+                final = st.last
                 out = (torch.empty((R, C) if base_out.ndim >= 2 else (C,), dtype=torch.bfloat16, device=dev)
                        if (final and base_bf16 is not None)
                        else torch.empty((R, C) if base_out.ndim >= 2 else (C,), dtype=torch.float32, device=dev))
@@ -518,30 +522,24 @@ class FourierMerge(MergeTensorsBase):
                     logger.info(f"Arithmetic-FFT Merged {sb.name} x {weight_scale} on to {sa.name} x {norm_scale}")
                 else:                                          # :233-244  SLERP-FFT
                     a_prop = a_w / (a_w + b_w)
-                    branch = _slerp_pair(ws, slot_a, slot_b, sa, sb, na, nb, a_prop, cull_pct, target_norm,
+                    branch = _slerp_pair(ws, slot_a, slot_b, sa, sb, na, nb, a_prop, st.cull_pct, target_norm,
                                          base_bf16 if final else None, out, final, base_out)
                     info["branches"].append(branch)
                     merged = out
                     logger.info(f"SLERP-FFT Merged {sa.name} and {sb.name} with weight {a_prop}")
                 if final and merged.dtype == torch.bfloat16:
                     out_final = merged
-                    nxt.append((None, None)); nxt_w.append((a_w + b_w) / 2.0)
+                    nxt.append((None, None))
                 else:
                     inter = E.Source(x32=merged.reshape(R, C) if merged.ndim == 1 else merged,
                                      weight=(a_w + b_w) / 2.0, name=name_hash(f"{sa.name}_{sb.name}"))
-                    nxt.append((inter, None)); nxt_w.append((a_w + b_w) / 2.0)
-            stack, weights = nxt, nxt_w
-            cull_pct = cull_pct / 2.0                          # :254
+                    nxt.append((inter, None))
+            stack = nxt
 
         _, _, flags, _ = ws.read_ctl()
         info["flags"] = [int(v) for v in flags]
         if ws.select_sticky() != 0:
-            # the sampled window of a fast order-statistic select missed (or its candidate buffer
-            # overflowed): the thresholds are NaN.  Redo this tensor with the exhaustive select.
-            if safe_select:
-                raise RuntimeError(f"order-statistic select failed in safe mode for {layer_name}")
-            logger.warning(f"select window miss on {layer_name}; re-running with the exhaustive select")
-            return self._merge_sources_steps(sources, base_out, dev, layer_name=layer_name, safe_select=True)
+            return None, ws.select_sticky()
         if int(flags[1]) > 0:
             raise ValueError("Inf in ifft output")             # functions.py:215-217
         if out_final is None:
@@ -551,20 +549,16 @@ class FourierMerge(MergeTensorsBase):
             res = torch.where(torch.isnan(res), torch.zeros_like(res), res)
             if torch.any(torch.isinf(res)):
                 raise ValueError(f"Inf in merged tensor for {layer_name}")
-            return res.to(torch.bfloat16)
+            return res.to(torch.bfloat16), 0
         if int(flags[3]) > 0:
             raise ValueError(f"Inf in merged tensor for {layer_name}")   # fast_fourier.py:273-274
-        return out_final.reshape(base_out.shape)
+        return out_final.reshape(base_out.shape), 0
 
 
 # ------------------------------------------------------------------------------------------
-def _rows_into(ws: E.Workspace, slot: int, src: E.Source, sumsq_ptr: int):
-    E.fwd_rows_ptr(ws, slot, src, sumsq_ptr)
-
-
 def _rows_and_norm(ws: E.Workspace, slot: int, src: E.Source) -> float:
     acc = torch.zeros(1, dtype=torch.float64, device=ws.plan.device)
-    _rows_into(ws, slot, src, acc.data_ptr())
+    E.fwd_rows_ptr(ws, slot, src, acc.data_ptr())
     return E.f32(acc.item() ** 0.5)
 
 

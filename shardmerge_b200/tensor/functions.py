@@ -114,12 +114,18 @@ def normalize_tensor(tensor: torch.Tensor, device: str) -> tuple[torch.Tensor, f
     return (tensor / norm if norm != 0 else tensor), norm
 
 
-def _select_missed(safe: bool, what: str):
-    """A sampled order-statistic window missed (or overflowed): the thresholds were NaN and the blend is not the merge.
-    The caller redoes it with the exhaustive select, which must not miss."""
-    if safe:
-        raise RuntimeError(f"order-statistic select failed in safe mode in {what}")
-    logger.warning(f"select window miss in {what}; re-running with the exhaustive select")
+def retry_on_select_miss(run, where: str, safe: bool = False):
+    """run(safe) -> (result, sticky status of its order statistics).  A non-zero status means a sampled select window
+    missed (or overflowed): the thresholds were NaN and the result is not the merge.  Then it is run again with the
+    exhaustive select (safe=True), which must not miss.  `where` names the function or tensor in the messages."""
+    while True:
+        result, sticky = run(safe)
+        if sticky == 0:
+            return result
+        if safe:
+            raise RuntimeError(f"order-statistic select failed in safe mode {where}")
+        logger.warning(f"select window miss {where}; re-running with the exhaustive select")
+        safe = True
 
 
 def _blend_planes(ws: E.Workspace, mode: str, t: float, t_sum: float, cutoff_pct: float, cull_pct: float,
@@ -152,16 +158,17 @@ def interpolate_fft_components(v0_fft: torch.Tensor, v1_fft: torch.Tensor, t: fl
     allocated with torch.zeros_like(v0_fft, device=device))."""
     dev = _dev(device)
     R, C = _as_rows(v0_fft)
-    for safe in (False, True):
+
+    def blend(safe):
         ws = E.ws_for(v0_fft, dev, safe_select=safe)
         ws.ctl.zero_()
         _pack(ws, 0, v0_fft.reshape(R, C))
         _pack(ws, 1, v1_fft.reshape(R, C))
         _blend_planes(ws, "slerp", t, t_sum, cutoff_pct, cull_pct, True)
         ws.read_ctl()
-        if ws.select_sticky() == 0:
-            break
-        _select_missed(safe, "interpolate_fft_components")
+        return ws, ws.select_sticky()
+
+    ws = retry_on_select_miss(blend, "in interpolate_fft_components")
     full = _expand(ws, 0, tuple(v0_fft.shape))
     # imaginary part: Im X0 (exact for interp_imag=False, functions.py:160; within rounding noise of
     # the nested path otherwise, see module docstring)
@@ -216,19 +223,20 @@ def merge_tensors_fft2_slerp(v0: torch.Tensor, v1: torch.Tensor, t: float, devic
         E.inv_rows(ws, ws.re[0], ws.im[0], False, 1.0, None, out, check_ifft=True)
         _, _, flags, _ = ws.read_ctl()
     else:
-        for safe in (False, True):
+        def blend(safe):
+            w = ws
             if safe:
                 # the blend ran in place: the row spectra are gone, redo them in the exhaustive select's workspace
-                ws = E.ws_for(v0, dev, safe_select=True)
-                ws.ctl.zero_()
-                E.fwd_rows(ws, 0, E.Source(x32=x0), E.D_SUMSQ0)
-                E.fwd_rows(ws, 1, E.Source(x32=x1), E.D_SUMSQ1)
-            E.spectral_pair(ws, 0, 1, scale0=inv0, scale1=inv1, mode="slerp", t=t,
+                w = E.ws_for(v0, dev, safe_select=True)
+                w.ctl.zero_()
+                E.fwd_rows(w, 0, E.Source(x32=x0), E.D_SUMSQ0)
+                E.fwd_rows(w, 1, E.Source(x32=x1), E.D_SUMSQ1)
+            E.spectral_pair(w, 0, 1, scale0=inv0, scale1=inv1, mode="slerp", t=t,
                             t_sum=t_sum, cutoff_pct=cutoff_pct, cull_pct=cull_pct, out_scale=1.0, out=out)
-            _, _, flags, _ = ws.read_ctl()
-            if ws.select_sticky() == 0:
-                break
-            _select_missed(safe, "merge_tensors_fft2_slerp")
+            _, _, flags, _ = w.read_ctl()
+            return flags, w.select_sticky()
+
+        flags = retry_on_select_miss(blend, "in merge_tensors_fft2_slerp")
     if int(flags[0]) > 0:
         logger.info(f"Warning: NaN in ifft output: {int(flags[0])}")
     if int(flags[1]) > 0:                                     # functions.py:215-217

@@ -90,3 +90,32 @@ def test_no_cpu_fallback():
         F.fft_transform(torch.randn(8, 8), "cpu")
     with pytest.raises(RuntimeError):
         F.merge_tensors_fft2_slerp(torch.randn(8, 8), torch.randn(8, 8), 0.5, "cpu")
+
+
+def test_scalar_block_mirror_matches_header():
+    """_lib's copy of the scalar-block layout is the header's #defines, name for name."""
+    from shardmerge_b200 import _lib
+    header = (ROOT / "include" / "shardmerge_b200.h").read_text()
+    prefix = r"SM_(?:CTL|F|I|BRANCH|FS|SELECT)_\w+"
+    declared = {name: int(v) for name, v in re.findall(rf"^#define ({prefix})\s+(\d+)", header, re.M)}
+    assert len(declared) >= 29
+    mirrored = {name: getattr(_lib, name) for name in dir(_lib) if re.fullmatch(prefix, name)}
+    assert mirrored == declared
+    assert set(_lib.BRANCH_NAMES) == {v for k, v in declared.items() if k.startswith("SM_BRANCH_")}
+
+
+def test_pair_args_layout_matches_header(tmp_path):
+    """sizeof and every field offset of sm_pair_args, compiled from the header, equal those of _lib.PairArgs."""
+    import os
+    import subprocess
+    from shardmerge_b200 import _lib
+    fields = [f[0] for f in _lib.PairArgs._fields_]
+    src = tmp_path / "pair_args.c"
+    src.write_text("#include <stdio.h>\n#include <stddef.h>\n#include \"shardmerge_b200.h\"\nint main(void) {\n"
+                   "  printf(\"sizeof %zu\\n\", sizeof(sm_pair_args));\n"
+                   + "".join(f"  printf(\"{f} %zu\\n\", offsetof(sm_pair_args, {f}));\n" for f in fields) + "  return 0;\n}\n")
+    exe = tmp_path / "pair_args"
+    subprocess.run([os.environ.get("CC", "gcc"), "-I", str(ROOT / "include"), "-o", str(exe), str(src)], check=True)
+    got = dict(line.split() for line in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines())
+    assert int(got.pop("sizeof")) == ctypes.sizeof(_lib.PairArgs)
+    assert {f: int(v) for f, v in got.items()} == {f: getattr(_lib.PairArgs, f).offset for f in fields}

@@ -781,7 +781,7 @@ def test_elementwise_kernel_bandwidth(E):
 
 
 @pytest.mark.parametrize("n_models,shape", [(4, (512, 2048)), (3, (1024, 2048)), (4, (1, 8192)), (5, (256, 4096))])
-def test_fused_tree_matches_step_path(E, n_models, shape):
+def test_fused_tree_matches_merge_sources_steps(E, n_models, shape):
     """BASELINE config 4: the pair tree with every pair merge on the fused chain (FourierMerge._merge_sources_tree: fp32
     intermediates, external target norm, device-side role / branch decisions) against the host-driven step path on the
     same kernels -- same spectra, same exact thresholds, so the same tensor."""
@@ -797,10 +797,10 @@ def test_fused_tree_matches_step_path(E, n_models, shape):
     fts = [(base.float() + s * torch.randn(sh, generator=g, device=DEV)).to(torch.bfloat16) for s in sig]
     srcs = lambda: [E.make_source(base, ft, weight=a, name=f"m{k}") for k, (ft, a) in enumerate(zip(fts, alphas))]
     fm = _merger()
-    assert fm.fused_tree
     got = fm.merge_sources(srcs(), base, torch.device(DEV), layer_name="model.layers.0.x")
     info = dict(fm.last_info)
     assert info["branches"] == ["slerp"] * (n_models - 1)
+    assert len(info["swap"]) == n_models - 1                 # the fused tree ran: one device role decision per pair
     # deferred on the lanes as merge() does it
     fm.defer_checks = True
     got2 = fm.merge_sources(srcs(), base, torch.device(DEV), layer_name="model.layers.0.x", defer=True)
@@ -808,8 +808,7 @@ def test_fused_tree_matches_step_path(E, n_models, shape):
     torch.cuda.synchronize()
     assert np.array_equal(bits(got), bits(got2))
     fm_steps = _merger()
-    fm_steps.fused_tree = False
-    want = fm_steps.merge_sources(srcs(), base, torch.device(DEV), layer_name="model.layers.0.x")
+    want = fm_steps._merge_sources_steps(srcs(), base, torch.device(DEV), layer_name="model.layers.0.x")
     assert fm_steps.last_info["branches"] == ["slerp"] * (n_models - 1)
     assert abs(info["target_norm"] / fm_steps.last_info["target_norm"] - 1) < 1e-7
     # Rounds >= 2 blend spectra whose culled bins hold rounding noise: the last bit of a round-1 scalar decides ~10 % of

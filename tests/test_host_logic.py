@@ -19,7 +19,7 @@ from shardmerge_b200 import schedule
 from shardmerge_b200.config import MergeConfig, MergeModel
 from shardmerge_b200.constants import INPUT_LAYER, OUTPUT_LAYER
 from shardmerge_b200.index import InMemoryIndex, LocalSafetensorsIndex, canonical_layer_order
-from shardmerge_b200.merge.fast_fourier import clamp, name_hash, task_arithmetic
+from shardmerge_b200.merge.fast_fourier import clamp, name_hash, task_arithmetic, tree_plan
 from shardmerge_b200.tensor.functions import correlated_pairs
 from shardmerge_b200.writer import ModelWriter, ShardLayer
 
@@ -95,6 +95,38 @@ def test_correlated_pairs_matches_oracle():
             assert sorted(used) == list(range(n))
     with pytest.raises(ValueError):
         list(correlated_pairs(torch.zeros(3, 3), "sideways"))
+
+
+def _oracle_tree(norms, weights, cull_start_pct):
+    """The rounds of oracle_np.merge_layer's pair loop (the stale-norm products, :171-254 of the reference) as
+    (x, y, a_w, b_w, cull_pct, last) with (x, -1, w, 0.0, cull_pct, False) for a model carried to the next round."""
+    rounds, w, cull = [], list(weights), cull_start_pct
+    while len(w) > 1:
+        n = len(w)
+        corr = np.zeros((n, n), dtype=np.float32)
+        for i in range(n):
+            for j in range(i + 1, n):
+                corr[i, j] = norms[i] * norms[j]
+        pairs = O.correlated_pairs(corr, "least")
+        rnd = [(x, y, w[x], w[y] if y >= 0 else 0.0, cull, y >= 0 and len(pairs) == 1) for x, y, _ in pairs]
+        rounds.append(rnd)
+        w = [a_w if y < 0 else (a_w + b_w) / 2.0 for _, y, a_w, b_w, _, _ in rnd]
+        cull = cull / 2.0
+    return rounds
+
+
+@pytest.mark.parametrize("kind", ["equal", "random"])
+def test_tree_plan_matches_oracle_loop(kind):
+    rng = np.random.default_rng(5)
+    for m in range(1, 13):
+        sumsq = [0.04] * m if kind == "equal" else list(rng.uniform(1e-4, 2.0, m))
+        weights = list(rng.uniform(0.1, 1.0, m))
+        norms, target_norm, rounds = tree_plan(sumsq, weights, 0.20, 1e-10)
+        want_norms = [np.float32(v ** 0.5) for v in sumsq]
+        assert norms == [float(v) for v in want_norms]
+        assert abs(target_norm / (float(np.mean(np.array(want_norms, dtype=np.float32))) + 1e-10) - 1) < 1e-6
+        assert [[tuple(st) for st in rnd] for rnd in rounds] == _oracle_tree(want_norms, weights, 0.20), m
+        assert len(rounds) == (m - 1).bit_length() and sum(st.last for rnd in rounds for st in rnd) == (m > 1)
 
 
 def _toy_model(seed, L=3, H=16):

@@ -39,12 +39,12 @@ for tag, (x0, x1) in (("round 1 (deltas)", ((fts[0].float() - base.float()), (ft
     a, b = ws.re[0][:, :Ch + 1], ws.re[1][:, :Ch + 1]
     us = timeit(lambda: E.fstats_cutoff(ws, ws.re[0], ws.re[1], int(2 * N * 0.08), 0.5))
     h = ws.ctl.cpu()
-    o = _lib.CTL_FS_OFF
-    st = h[o:o + 128]
+    o = _lib.SM_CTL_FS
+    st = h[o:o + _lib.SM_FS_STATE_BYTES]
     lo, hi = st[16:24].view(torch.int32).tolist()
     lo_f = torch.tensor([lo], dtype=torch.int32).view(torch.float32).item(); hi_f = torch.tensor([hi], dtype=torch.int32).view(torch.float32).item()
     inwin = (((a.abs() >= lo_f) & (a.abs() <= hi_f)).float().mean().item() + ((b.abs() >= lo_f) & (b.abs() <= hi_f)).float().mean().item()) / 2
     prod0 = ((a * b) == 0).float().mean().item()
     print(f"{tag}: cutoff {us:.1f} us  window [{lo_f:.3e}, {hi_f:.3e}] width 2^{(hi - lo).bit_length()}  keys in window {inwin:.4f}  "
           f"zero products {prod0:.4f}  exact zeros {((a == 0).float().mean().item()):.4f}/{((b == 0).float().mean().item()):.4f}  "
-          f"|re| quantiles a {[float(q) for q in torch.quantile(a.abs().flatten()[:4000000], torch.tensor([0.05, 0.1, 0.2, 0.25, 0.5], device=dev))]}  status {ws.fs_status()}")
+          f"|re| quantiles a {[float(q) for q in torch.quantile(a.abs().flatten()[:4000000], torch.tensor([0.05, 0.1, 0.2, 0.25, 0.5], device=dev))]}  sticky {ws.fs_status()}")

@@ -34,4 +34,4 @@ cull = 0.10 if culled else 0.20
 print(("culled " if culled else "plain  ") + f"{R}x{C}")
 print("  cutoff  %.1f us" % run(lambda: E.fstats_cutoff(ws, ws.re[0], ws.re[1], int(2 * N * cut), 0.375)))
 print("  blend   %.1f us" % run(lambda: E.fstats_blend_cull(ws, ws.re[0], ws.re[1], 1.0, out, int(N * cull))))
-print("  status", ws.fs_status(), "thr_cut %.3e thr_cull %.3e" % (float(ws.flt[E.F_THR_CUT]), float(ws.flt[E.F_THR_CULL])))
+print("  sticky", ws.fs_status(), "thr_cut %.3e thr_cull %.3e" % (float(ws.flt[E.F_THR_CUT]), float(ws.flt[E.F_THR_CULL])))
