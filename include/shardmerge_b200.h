@@ -66,6 +66,17 @@ int sm_fwd_rows_bf16(const sm_plan* plan, const void* tables, const void* base_b
  * at shard/merge/fast_fourier.py:228-230), sumsq accumulates sum(x^2). */
 int sm_fwd_rows_f32(const sm_plan* plan, const void* tables, const float* x, float m1, float m2,
                     float* re, float* im, double* sumsq, void* stream);
+/* Both finetunes of a pair merge that share one base, in ONE pass that reads the base once: (re0, im0) and (re1, im1)
+ * receive exactly what sm_fwd_rows_bf16(base, ft0) and sm_fwd_rows_bf16(base, ft1) write, ctl is the pair merge's scalar
+ * block (below), zeroed by the caller: its SM_CTL_SUMSQ doubles receive += sum(delta^2) of each model, and the pass's
+ * last CTA then makes the decisions sm_pair_merge_async makes from the two norms (scales, norms, swap, branch,
+ * target_norm; target_norm > 0 overrides the mean of the two norms), counting CTAs in the SM_CTL_TICKET word.
+ * sm_fwd_rows_pair_supported(plan) != 0 says whether the plan's row length has a paired kernel (C = 4096 with an even
+ * row count, C = 14336); sm_fwd_rows_bf16_pair fails on any other plan. */
+int sm_fwd_rows_pair_supported(const sm_plan* plan);
+int sm_fwd_rows_bf16_pair(const sm_plan* plan, const void* tables, const void* base_bf16, const void* ft0_bf16,
+                          const void* ft1_bf16, float* re0, float* im0, float* re1, float* im1, void* ctl,
+                          double target_norm_offset, double target_norm, void* stream);
 /* Column half of fft_transform, in place.  The spectrum is multiplied by *scale_dev (if
  * non-NULL) else by scale_host: this is where `tensor / norm` of normalize_tensor
  * (functions.py:88) is applied (the FFT is linear).  write_im = 0 skips storing the
@@ -201,6 +212,7 @@ int sm_pack_half(const sm_plan* plan, const float* in_c64, float* re, float* im,
 #define SM_CTL_FLAGS   128    /* u32[4]     nan/inf after ifft, nan/inf final                  */
 #define SM_CTL_INT     144    /* i32[4]     indexed by SM_I_*                                  */
 #define SM_CTL_TN      160    /* double     target_norm                                        */
+#define SM_CTL_TICKET  168    /* u32        CTAs of the paired row pass that have finished     */
 #define SM_CTL_SEL     192    /* 2 x SM_SELECT_STATE_BYTES: cutoff select, cull select (step-by-step path) */
 #define SM_CTL_FS      512    /* 2 x SM_FS_STATE_BYTES: fused cutoff statistics, fused blend + cull   */
 #define SM_F_THR_CUT 0

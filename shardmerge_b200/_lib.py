@@ -27,6 +27,8 @@ SIGNATURES = {
     "sm_plan_table_bytes": (_sz, [_vp]),
     "sm_plan_init_tables": (_i, [_vp, _vp, _vp]),
     "sm_fwd_rows_bf16": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sm_fwd_rows_pair_supported": (_i, [_vp]),
+    "sm_fwd_rows_bf16_pair": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _vp]),
     "sm_fwd_rows_f32": (_i, [_vp, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp]),
     "sm_fwd_cols": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _i, _vp]),
     "sm_inv_norm": (_i, [_vp, _vp, _vp]),
@@ -71,8 +73,8 @@ class PairArgs(C.Structure):
 # the scalar block of the fused pair merge and the statistics states inside it: the header's #defines, one to one
 SM_SELECT_STATE_BYTES, SM_SELECT_STICKY_OFF = 64, 44
 SM_FS_STATE_BYTES, SM_FS_STATUS_OFF, SM_FS_STICKY_OFF = 128, 28, 72
-SM_CTL_BYTES, SM_CTL_SUMSQ, SM_CTL_SUMS, SM_CTL_FLT, SM_CTL_FLAGS, SM_CTL_INT, SM_CTL_TN, SM_CTL_SEL, SM_CTL_FS = (
-    1024, 0, 16, 64, 128, 144, 160, 192, 512)
+SM_CTL_BYTES, SM_CTL_SUMSQ, SM_CTL_SUMS, SM_CTL_FLT, SM_CTL_FLAGS, SM_CTL_INT, SM_CTL_TN, SM_CTL_TICKET, SM_CTL_SEL, SM_CTL_FS = (
+    1024, 0, 16, 64, 128, 144, 160, 168, 192, 512)
 SM_F_THR_CUT, SM_F_THR_CULL, SM_F_DOT, SM_F_SCALE_X, SM_F_SCALE_Y, SM_F_OUT_SCALE, SM_F_NORM_X, SM_F_NORM_Y = (
     0, 1, 2, 6, 7, 8, 9, 10)
 SM_I_SWAP, SM_I_BRANCH = 0, 1

@@ -287,19 +287,69 @@ struct RowDeltaStaged2 {        // stage-1 source: staging = [base row0 | base r
   }
 };
 
-// X[n] and X[Ch - n] of both rows from Z[n] = (ar, ai) and Z[Ch - n] = (br, bi); w = W_C^n
-__device__ __forceinline__ void untangle_pair2(pf ar, pf ai, pf br, pf bi, cf w, float* re0, float* im0, int P, int n, int m) {
+// X[n] and X[Ch - n] of both lanes from Z[n] = (ar, ai) and Z[Ch - n] = (br, bi); w = W_C^n; lane 0 -> (reA, imA),
+// lane 1 -> (reB, imB)
+__device__ __forceinline__ void untangle_pair2(pf ar, pf ai, pf br, pf bi, cf w, float* reA, float* imA, float* reB, float* imB,
+                                               int n, int m) {
   const pf h = pf_bcast(0.5f);
   const pf er = h * (ar + br), ei = h * (ai - bi), pr = h * (ai + bi), qi = zero_of(ar) - h * (ar - br);
   const pf wx = pf_bcast(w.x), wy = pf_bcast(w.y);
   const pf tr = pf_fma(pr, wx, zero_of(ar) - qi * wy);       // pr * w.x - qi * w.y
   const pf ti = pf_fma(pr, wy, qi * wx);                      // pr * w.y + qi * w.x
   const pf xr = er + tr, xi = ei + ti;
-  re0[n] = pf_lo(xr); re0[P + n] = pf_hi(xr); im0[n] = pf_lo(xi); im0[P + n] = pf_hi(xi);
+  reA[n] = pf_lo(xr); reB[n] = pf_hi(xr); imA[n] = pf_lo(xi); imB[n] = pf_hi(xi);
   if (m != n) {
     const pf yr = er - tr, yi = ti - ei;
-    re0[m] = pf_lo(yr); re0[P + m] = pf_hi(yr); im0[m] = pf_lo(yi); im0[P + m] = pf_hi(yi);
+    reA[m] = pf_lo(yr); reB[m] = pf_hi(yr); imA[m] = pf_lo(yi); imB[m] = pf_hi(yi);
   }
+}
+// two adjacent rows: lane 1 is the row below lane 0's
+__device__ __forceinline__ void untangle_pair2(pf ar, pf ai, pf br, pf bi, cf w, float* re0, float* im0, int P, int n, int m) {
+  untangle_pair2(ar, ai, br, bi, w, re0, im0, re0 + P, im0 + P, n, m);
+}
+
+// ---- both finetunes of a pair merge over ONE base (sm_fwd_rows_bf16_pair): the same row of model 0 and model 1 in one
+// CTA, so the base row is staged (k_row2_fwd) or fetched from HBM (k_row1_fwd_eo) once for both.  Per model the arithmetic
+// is that of the single-model pass.  The second model's tensors and the pair merge's scalar block:
+struct RowFwdPair {
+  const uint16_t* ft1; float* re1; float* im1;
+  unsigned char* ctl; double target_norm_offset, ext_tn;
+};
+
+struct RowDeltaStagedPair {     // stage-1 source: staging = [base row | ft0 row | ft1 row], bf16; lane k = ft_k - base
+  const uint32_t* b32; const uint32_t* f0; const uint32_t* f1; pf* acc;
+  __device__ __forceinline__ void load(int i, pf& re, pf& im) const {
+    const uint32_t b = b32[i], g0 = f0[i], g1 = f1[i];
+    const float br = bf16_bits_to_f32(b & 0xffffu), bi = bits_f32(b & 0xffff0000u);
+    re = pf_make(bf16_bits_to_f32(g0 & 0xffffu), bf16_bits_to_f32(g1 & 0xffffu)) - pf_make(br, br);
+    im = pf_make(bits_f32(g0 & 0xffff0000u), bits_f32(g1 & 0xffff0000u)) - pf_make(bi, bi);
+    *acc = pf_fma(re, re, pf_fma(im, im, *acc));
+  }
+};
+
+// End of a paired pass: the per-thread fp64 sums of squares of model 0 / model 1 -> sumsq[0], sumsq[1]; the last CTA to
+// finish then makes the pair merge's decisions from the two totals, as k_prepare (pipeline.cu) does after two single-model
+// passes.  The ticket word is zeroed with the rest of the scalar block before the pass.
+template <int T>
+__device__ __forceinline__ void row_pair_finish(double acc0, double acc1, double* sumsq, const RowFwdPair& pr) {
+  constexpr int NW = (T + 31) / 32;
+  __shared__ double wsum[2][NW];
+  acc0 = warp_sum(acc0);
+  acc1 = warp_sum(acc1);
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (lane == 0) { wsum[0][wid] = acc0; wsum[1][wid] = acc1; }
+  __syncthreads();
+  if (wid != 0) return;
+  double v0 = lane < NW ? wsum[0][lane] : 0.0, v1 = lane < NW ? wsum[1][lane] : 0.0;
+  v0 = warp_sum(v0);
+  v1 = warp_sum(v1);
+  if (lane != 0) return;
+  atomicAdd(sumsq, v0);
+  atomicAdd(sumsq + 1, v1);
+  __threadfence();
+  if (atomicAdd(reinterpret_cast<unsigned int*>(pr.ctl + SM_CTL_TICKET), 1u) != gridDim.x - 1u) return;
+  __threadfence();
+  sm_prepare_scalars(pr.ctl, __ldcg(sumsq), __ldcg(sumsq + 1), pr.target_norm_offset, pr.ext_tn);
 }
 
 // kEO: the two lanes are the even / odd halves of ONE row instead of two rows (see k_row1_fwd_eo below): C = 8192 then has
@@ -319,10 +369,12 @@ struct RowDeltaStagedEO {        // stage-1 source: complex elements 2i (lane 0)
   }
 };
 
-template <int R1, int R2, int R3, int T, bool kEO>
+// kPair: the lanes are row r of model 0 (a.ft, a.re, a.im) and row r of model 1 (pr): sm_fwd_rows_bf16_pair
+template <int R1, int R2, int R3, int T, bool kEO, bool kPair = false>
 __global__ void __launch_bounds__(T, 3) k_row2_fwd(int R, int C, int P, const __grid_constant__ RowFwdArgs a,
                                                 const cf* __restrict__ twC, const cf* __restrict__ twQ,
-                                                double* __restrict__ sumsq, int work_bytes) {
+                                                double* __restrict__ sumsq, int work_bytes, const __grid_constant__ RowFwdPair pr) {
+  static_assert(!(kEO && kPair), "k_row2_fwd: the lanes are either even / odd halves or two models");
   sm_pdl_enter();
   constexpr int CH = R1 * R2 * R3;
   constexpr int S3 = CH / R3;                       // stride (and butterfly count) of the last stage
@@ -332,22 +384,23 @@ __global__ void __launch_bounds__(T, 3) k_row2_fwd(int R, int C, int P, const __
   RowSmem2 sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
   char* stage = reinterpret_cast<char*>(g_dyn_smem) + work_bytes;
   const int tid = threadIdx.x;
-  constexpr int kRows = kEO ? 1 : 2;                // rows per iteration
+  constexpr int kRows = (kEO || kPair) ? 1 : 2;     // rows per iteration, per tensor
   constexpr int kTw = kEO ? 4 : 2;                  // W_CH^e = twC[e * kTw]
-  const int npairs = kEO ? R : (R >> 1);
+  const int npairs = (kEO || kPair) ? R : (R >> 1);
   const uint32_t row_bytes = 2u * (uint32_t)C * kRows;    // bf16 bytes of one iteration's rows, per tensor
   if (tid == 0) { mbar_init(&full, 1); mbar_fence_init(); }
   __syncthreads();
   auto prefetch = [&](int pair) {                   // the rows of an iteration are contiguous: one bulk copy per tensor
     if (tid == 0 && pair < npairs) {
-      mbar_expect_tx(&full, 2u * row_bytes);
+      mbar_expect_tx(&full, (kPair ? 3u : 2u) * row_bytes);
       bulk_g2s(stage, a.base + (size_t)pair * kRows * C, row_bytes, &full);
       bulk_g2s(stage + row_bytes, a.ft + (size_t)pair * kRows * C, row_bytes, &full);
+      if constexpr (kPair) bulk_g2s(stage + 2 * row_bytes, pr.ft1 + (size_t)pair * C, row_bytes, &full);
     }
   };
   prefetch((int)blockIdx.x);
   uint32_t phase = 0;
-  double accd = 0.0;
+  double accd = 0.0, accd1 = 0.0;                   // accd1: model 1 of a paired pass
   // every twiddle of this thread is the same for all row pairs; the loads are issued ahead of the barrier / wait that
   // precedes their use, so their latency is never exposed (the kernel is latency bound: 3 CTAs of 4 warps per SM)
   const int p2 = tid / R1, q2 = tid - p2 * R1;
@@ -363,6 +416,11 @@ __global__ void __launch_bounds__(T, 3) k_row2_fwd(int R, int C, int P, const __
       constexpr int Nr = CH / R1;
       if constexpr (kEO) {
         RowDeltaStagedEO src{reinterpret_cast<const uint2*>(stage), reinterpret_cast<const uint2*>(stage + row_bytes), &accp};
+#pragma unroll
+        for (int j = 0; j < R1; ++j) src.load(tid + j * Nr, re[j], im[j]);
+      } else if constexpr (kPair) {
+        RowDeltaStagedPair src{reinterpret_cast<const uint32_t*>(stage), reinterpret_cast<const uint32_t*>(stage + row_bytes),
+                               reinterpret_cast<const uint32_t*>(stage + 2 * row_bytes), &accp};
 #pragma unroll
         for (int j = 0; j < R1; ++j) src.load(tid + j * Nr, re[j], im[j]);
       } else {
@@ -434,41 +492,52 @@ __global__ void __launch_bounds__(T, 3) k_row2_fwd(int R, int C, int P, const __
       __syncthreads();                              // the buffer has been read: the next pair's stage 1 may overwrite it
       Dft<R3>::run(ar, ai);
       Dft<R3>::run(br, bi);
-      float* re0 = a.re + (size_t)pair * 2 * P;
-      float* im0 = a.im + (size_t)pair * 2 * P;
+      // lane 0 -> (reA, imA), lane 1 -> (reB, imB): the next row of the same model (P floats further), or the same row of
+      // model 1
+      float* reA = a.re + (size_t)pair * kRows * P;
+      float* imA = a.im + (size_t)pair * kRows * P;
+      auto untangle = [&](pf ar_, pf ai_, pf br_, pf bi_, cf w_, int n) {
+        if constexpr (kPair) untangle_pair2(ar_, ai_, br_, bi_, w_, reA, imA, pr.re1 + (size_t)pair * P, pr.im1 + (size_t)pair * P, n, CH - n);
+        else untangle_pair2(ar_, ai_, br_, bi_, w_, reA, imA, P, n, CH - n);
+      };
       if (tid != 0) {
 #pragma unroll
         for (int k = 0; k < R3; ++k) {              // n = t + S3*k  <->  Ch - n = (S3 - t) + S3*(R3-1-k)
           const int n = bA + S3 * k;
-          untangle_pair2(ar[k], ai[k], br[R3 - 1 - k], bi[R3 - 1 - k], w[k], re0, im0, P, n, CH - n);
+          untangle(ar[k], ai[k], br[R3 - 1 - k], bi[R3 - 1 - k], w[k], n);
         }
       } else {
         // butterfly 0: n = S3*k <-> S3*(R3-k); n = 0 pairs with itself and also yields the Nyquist bin Ch
         {
           const pf h = ar[0], g = ai[0];
           const pf x0 = h + g, xn = h - g;
-          re0[0] = pf_lo(x0); re0[P] = pf_hi(x0); im0[0] = 0.f; im0[P] = 0.f;
-          re0[CH] = pf_lo(xn); re0[P + CH] = pf_hi(xn); im0[CH] = 0.f; im0[P + CH] = 0.f;
+          float* reB = kPair ? pr.re1 + (size_t)pair * P : reA + P;
+          float* imB = kPair ? pr.im1 + (size_t)pair * P : imA + P;
+          reA[0] = pf_lo(x0); reB[0] = pf_hi(x0); imA[0] = 0.f; imB[0] = 0.f;
+          reA[CH] = pf_lo(xn); reB[CH] = pf_hi(xn); imA[CH] = 0.f; imB[CH] = 0.f;
         }
 #pragma unroll
         for (int k = 1; k <= R3 / 2; ++k) {         // w[k] = W^(S3*k)
           const int n = S3 * k;
-          untangle_pair2(ar[k], ai[k], ar[R3 - k], ai[R3 - k], w[k], re0, im0, P, n, CH - n);
+          untangle(ar[k], ai[k], ar[R3 - k], ai[R3 - k], w[k], n);
         }
         // butterfly S3/2: n = S3/2 + S3*k <-> S3/2 + S3*(R3-1-k); w[R3/2 + 1 + k] = W^(S3/2 + S3*k)
 #pragma unroll
         for (int k = 0; k < R3 / 2 - 1; ++k) {
           const int n = S3 / 2 + S3 * k;
-          untangle_pair2(br[k], bi[k], br[R3 - 1 - k], bi[R3 - 1 - k], w[R3 / 2 + 1 + k], re0, im0, P, n, CH - n);
+          untangle(br[k], bi[k], br[R3 - 1 - k], bi[R3 - 1 - k], w[R3 / 2 + 1 + k], n);
         }
         {                                           // the last pair of that butterfly has no slot left in w[]
           const int k = R3 / 2 - 1, n = S3 / 2 + S3 * k;
-          untangle_pair2(br[k], bi[k], br[R3 - 1 - k], bi[R3 - 1 - k], ldg_cf(twC + n), re0, im0, P, n, CH - n);
+          untangle(br[k], bi[k], br[R3 - 1 - k], bi[R3 - 1 - k], ldg_cf(twC + n), n);
         }
       }
     }
-    accd += (double)pf_lo(accp) + (double)pf_hi(accp);   // fp32 over one thread's share of one row, fp64 across
+    // fp32 over one thread's share of one row, fp64 across
+    if constexpr (kPair) { accd += (double)pf_lo(accp); accd1 += (double)pf_hi(accp); }
+    else accd += (double)pf_lo(accp) + (double)pf_hi(accp);
   }
+  if constexpr (kPair) { row_pair_finish<T>(accd, accd1, sumsq, pr); return; }
   double acc = warp_sum(accd);
   const int lane = tid & 31, wid = tid >> 5;
   if (lane == 0) wsum[wid] = acc;
@@ -685,10 +754,12 @@ __device__ __forceinline__ void combine_untangle4(pf xr, pf xi, pf yr, pf yi, co
   if (m != n) untangle_pair1(enr - onr, eni - oni, emr + omr, emi + omi, ldg_cf(twC + n + H), re0, im0, n + H, m);   // (n + H, m)
 }
 
-template <int R1, int R2, int R3, int R4, int T, int kCtas>
+// kPair: one CTA transforms row r of model 0 (a.ft, a.re, a.im), then row r of model 1 (pr); the second read of the base
+// row hits L2: sm_fwd_rows_bf16_pair
+template <int R1, int R2, int R3, int R4, int T, int kCtas, bool kPair = false>
 __global__ void __launch_bounds__(T, kCtas) k_row1_fwd_eo(int R, int C, int P, const __grid_constant__ RowFwdArgs a,
                                                       const cf* __restrict__ twC, const cf* __restrict__ twQ2,
-                                                      double* __restrict__ sumsq) {
+                                                      double* __restrict__ sumsq, const __grid_constant__ RowFwdPair pr) {
   sm_pdl_enter();
   constexpr int CH = R1 * R2 * R3 * R4;             // length of the even / odd transforms = Ch / 2
   constexpr int NB1 = CH / R1, NB2 = CH / R2, NB3 = CH / R3, S4 = CH / R4;
@@ -698,102 +769,112 @@ __global__ void __launch_bounds__(T, kCtas) k_row1_fwd_eo(int R, int C, int P, c
   __shared__ double wsum[16];
   RowSmem2X<false> sm{reinterpret_cast<ulonglong2*>(g_dyn_smem)};
   const int tid = threadIdx.x;
-  double accd = 0.0;
+  double accd = 0.0, accd1 = 0.0;                   // accd1: model 1 of a paired pass
   if (tid == 0 && (int)blockIdx.x < R) {
     bulk_prefetch_l2(a.base + (size_t)blockIdx.x * C, 2u * (uint32_t)C);
     bulk_prefetch_l2(a.ft + (size_t)blockIdx.x * C, 2u * (uint32_t)C);
   }
   for (int row = blockIdx.x; row < R; row += gridDim.x) {
-    pf accp = pf_make(0.f, 0.f);
-    {  // stage 1: delta + radix R1 (s = 1); the sub-transforms have twiddles W_CH = W_C^4: twiddle tables are read at stride 4
-      RowDeltaGlobalEO src{reinterpret_cast<const uint2*>(a.base + (size_t)row * C), reinterpret_cast<const uint2*>(a.ft + (size_t)row * C), &accp};
 #pragma unroll 1
-      for (int b = tid; b < NB1; b += T) stockham_bfly_first<R1, pf>(b, CH, twQ2, src, sm, 2);
-    }
-    __syncthreads();
-    if (tid == 0 && row + (int)gridDim.x < R) {
-      bulk_prefetch_l2(a.base + (size_t)(row + gridDim.x) * C, 2u * (uint32_t)C);
-      bulk_prefetch_l2(a.ft + (size_t)(row + gridDim.x) * C, 2u * (uint32_t)C);
-    }
-    {  // stage 2: radix R2, s = R1, in place, butterflies t (and t + T)
-      pf re[H2][R2], im[H2][R2];
-#pragma unroll
-      for (int h = 0; h < H2; ++h)
-#pragma unroll
-        for (int j = 0; j < R2; ++j) sm.load(tid + h * T + j * NB2, re[h][j], im[h][j]);
+    for (int m = 0; m < (kPair ? 2 : 1); ++m) {      // the model of this iteration
+      const uint16_t* ft = (kPair && m != 0) ? pr.ft1 : a.ft;
+      pf accp = pf_make(0.f, 0.f);
+      {  // stage 1: delta + radix R1 (s = 1); the sub-transforms have twiddles W_CH = W_C^4: twiddle tables are read at stride 4
+        RowDeltaGlobalEO src{reinterpret_cast<const uint2*>(a.base + (size_t)row * C), reinterpret_cast<const uint2*>(ft + (size_t)row * C), &accp};
+#pragma unroll 1
+        for (int b = tid; b < NB1; b += T) stockham_bfly_first<R1, pf>(b, CH, twQ2, src, sm, 2);
+      }
       __syncthreads();
-#pragma unroll
-      for (int h = 0; h < H2; ++h) {
-        Dft<R2>::run(re[h], im[h]);
-        const int b = tid + h * T;
-        const int p = b / s2, q = b - p * s2;
-        const int obase = q + s2 * R2 * p, tstep = s2 * p * 4;
-        sm.store(obase, re[h][0], im[h][0]);
-#pragma unroll
-        for (int k = 1; k < R2; ++k) {
-          const cf w = ldg_cf(twC + tstep * k);
-          pf xr = re[h][k], xi = im[h][k];
-          cmul(xr, xi, w.x, w.y);
-          sm.store(obase + k * s2, xr, xi);
+      if (tid == 0) {                                 // the next iteration's rows -> L2 while this one is transformed
+        if (kPair && m == 0) {
+          bulk_prefetch_l2(pr.ft1 + (size_t)row * C, 2u * (uint32_t)C);
+        } else if (row + (int)gridDim.x < R) {
+          bulk_prefetch_l2(a.base + (size_t)(row + gridDim.x) * C, 2u * (uint32_t)C);
+          bulk_prefetch_l2(a.ft + (size_t)(row + gridDim.x) * C, 2u * (uint32_t)C);
         }
       }
-    }
-    __syncthreads();
-    {  // stage 3: radix R3, s = R1*R2, in place, butterflies t and t + T
-      pf re[2][R3], im[2][R3];
+      {  // stage 2: radix R2, s = R1, in place, butterflies t (and t + T)
+        pf re[H2][R2], im[H2][R2];
 #pragma unroll
-      for (int h = 0; h < 2; ++h)
+        for (int h = 0; h < H2; ++h)
 #pragma unroll
-        for (int j = 0; j < R3; ++j) sm.load(tid + h * T + j * NB3, re[h][j], im[h][j]);
+          for (int j = 0; j < R2; ++j) sm.load(tid + h * T + j * NB2, re[h][j], im[h][j]);
+        __syncthreads();
+#pragma unroll
+        for (int h = 0; h < H2; ++h) {
+          Dft<R2>::run(re[h], im[h]);
+          const int b = tid + h * T;
+          const int p = b / s2, q = b - p * s2;
+          const int obase = q + s2 * R2 * p, tstep = s2 * p * 4;
+          sm.store(obase, re[h][0], im[h][0]);
+#pragma unroll
+          for (int k = 1; k < R2; ++k) {
+            const cf w = ldg_cf(twC + tstep * k);
+            pf xr = re[h][k], xi = im[h][k];
+            cmul(xr, xi, w.x, w.y);
+            sm.store(obase + k * s2, xr, xi);
+          }
+        }
+      }
       __syncthreads();
+      {  // stage 3: radix R3, s = R1*R2, in place, butterflies t and t + T
+        pf re[2][R3], im[2][R3];
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        Dft<R3>::run(re[h], im[h]);
-        const int b = tid + h * T;
-        const int p = b / s3, q = b - p * s3;
-        const int obase = q + s3 * R3 * p, tstep = s3 * p * 4;
-        sm.store(obase, re[h][0], im[h][0]);
+        for (int h = 0; h < 2; ++h)
 #pragma unroll
-        for (int k = 1; k < R3; ++k) {
-          const cf w = ldg_cf(twC + tstep * k);
-          pf xr = re[h][k], xi = im[h][k];
-          cmul(xr, xi, w.x, w.y);
-          sm.store(obase + k * s3, xr, xi);
+          for (int j = 0; j < R3; ++j) sm.load(tid + h * T + j * NB3, re[h][j], im[h][j]);
+        __syncthreads();
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          Dft<R3>::run(re[h], im[h]);
+          const int b = tid + h * T;
+          const int p = b / s3, q = b - p * s3;
+          const int obase = q + s3 * R3 * p, tstep = s3 * p * 4;
+          sm.store(obase, re[h][0], im[h][0]);
+#pragma unroll
+          for (int k = 1; k < R3; ++k) {
+            const cf w = ldg_cf(twC + tstep * k);
+            pf xr = re[h][k], xi = im[h][k];
+            cmul(xr, xi, w.x, w.y);
+            sm.store(obase + k * s3, xr, xi);
+          }
         }
       }
-    }
-    __syncthreads();
-    {  // stage 4 (last) on the butterflies t and S4 - t (thread 0: 0 and S4 / 2), then combine + untangle
-      const int bA = tid, bB = tid == 0 ? S4 / 2 : S4 - tid;
-      pf ar[R4], ai[R4], br[R4], bi[R4];
+      __syncthreads();
+      {  // stage 4 (last) on the butterflies t and S4 - t (thread 0: 0 and S4 / 2), then combine + untangle
+        const int bA = tid, bB = tid == 0 ? S4 / 2 : S4 - tid;
+        pf ar[R4], ai[R4], br[R4], bi[R4];
 #pragma unroll
-      for (int j = 0; j < R4; ++j) { sm.load(bA + j * S4, ar[j], ai[j]); sm.load(bB + j * S4, br[j], bi[j]); }
-      __syncthreads();                              // the buffer has been read: the next row's stage 1 may overwrite it
-      Dft<R4>::run(ar, ai);
-      Dft<R4>::run(br, bi);
-      float* re0 = a.re + (size_t)row * P;
-      float* im0 = a.im + (size_t)row * P;
-      if (tid != 0) {
+        for (int j = 0; j < R4; ++j) { sm.load(bA + j * S4, ar[j], ai[j]); sm.load(bB + j * S4, br[j], bi[j]); }
+        __syncthreads();                              // the buffer has been read: the next row's stage 1 may overwrite it
+        Dft<R4>::run(ar, ai);
+        Dft<R4>::run(br, bi);
+        float* re0 = ((kPair && m != 0) ? pr.re1 : a.re) + (size_t)row * P;
+        float* im0 = ((kPair && m != 0) ? pr.im1 : a.im) + (size_t)row * P;
+        if (tid != 0) {
 #pragma unroll
-        for (int k = 0; k < R4; ++k)                // n = t + S4*k  <->  CH - n = (S4 - t) + S4*(R4-1-k)
-          combine_untangle4(ar[k], ai[k], br[R4 - 1 - k], bi[R4 - 1 - k], twC, re0, im0, bA + S4 * k, CH);
-      } else {
-        {  // n = 0: Z[0] = E0 + O0 -> X[0], X[Ch]; Z[CH] = E0 - O0 pairs with itself -> X[CH]
-          const float e0r = pf_lo(ar[0]), e0i = pf_lo(ai[0]), o0r = pf_hi(ar[0]), o0i = pf_hi(ai[0]);
-          const float zr = e0r + o0r, zi = e0i + o0i;
-          re0[0] = zr + zi; im0[0] = 0.f; re0[2 * CH] = zr - zi; im0[2 * CH] = 0.f;
-          untangle_pair1(e0r - o0r, e0i - o0i, e0r - o0r, e0i - o0i, ldg_cf(twC + CH), re0, im0, CH, CH);
+          for (int k = 0; k < R4; ++k)                // n = t + S4*k  <->  CH - n = (S4 - t) + S4*(R4-1-k)
+            combine_untangle4(ar[k], ai[k], br[R4 - 1 - k], bi[R4 - 1 - k], twC, re0, im0, bA + S4 * k, CH);
+        } else {
+          {  // n = 0: Z[0] = E0 + O0 -> X[0], X[Ch]; Z[CH] = E0 - O0 pairs with itself -> X[CH]
+            const float e0r = pf_lo(ar[0]), e0i = pf_lo(ai[0]), o0r = pf_hi(ar[0]), o0i = pf_hi(ai[0]);
+            const float zr = e0r + o0r, zi = e0i + o0i;
+            re0[0] = zr + zi; im0[0] = 0.f; re0[2 * CH] = zr - zi; im0[2 * CH] = 0.f;
+            untangle_pair1(e0r - o0r, e0i - o0i, e0r - o0r, e0i - o0i, ldg_cf(twC + CH), re0, im0, CH, CH);
+          }
+#pragma unroll
+          for (int k = 1; k <= R4 / 2; ++k)           // butterfly 0: n = S4*k <-> S4*(R4-k)
+            combine_untangle4(ar[k], ai[k], ar[R4 - k], ai[R4 - k], twC, re0, im0, S4 * k, CH);
+#pragma unroll
+          for (int k = 0; k < R4 / 2; ++k)            // butterfly S4/2: n = S4/2 + S4*k <-> S4/2 + S4*(R4-1-k)
+            combine_untangle4(br[k], bi[k], br[R4 - 1 - k], bi[R4 - 1 - k], twC, re0, im0, S4 / 2 + S4 * k, CH);
         }
-#pragma unroll
-        for (int k = 1; k <= R4 / 2; ++k)           // butterfly 0: n = S4*k <-> S4*(R4-k)
-          combine_untangle4(ar[k], ai[k], ar[R4 - k], ai[R4 - k], twC, re0, im0, S4 * k, CH);
-#pragma unroll
-        for (int k = 0; k < R4 / 2; ++k)            // butterfly S4/2: n = S4/2 + S4*k <-> S4/2 + S4*(R4-1-k)
-          combine_untangle4(br[k], bi[k], br[R4 - 1 - k], bi[R4 - 1 - k], twC, re0, im0, S4 / 2 + S4 * k, CH);
       }
+      if (kPair && m != 0) accd1 += (double)pf_lo(accp) + (double)pf_hi(accp);
+      else accd += (double)pf_lo(accp) + (double)pf_hi(accp);
     }
-    accd += (double)pf_lo(accp) + (double)pf_hi(accp);
   }
+  if constexpr (kPair) { row_pair_finish<T>(accd, accd1, sumsq, pr); return; }
   double acc = warp_sum(accd);
   const int lane = tid & 31, wid = tid >> 5;
   if (lane == 0) wsum[wid] = acc;
@@ -1570,7 +1651,7 @@ static int try_row2_fwd(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, co
     if (e != cudaSuccess) { sm_set_error("row2 setup: %s", cudaGetErrorString(e)); return -100; }
     int grid = num_sms() * (occ > 0 ? occ : 1);
     if (grid > p.R / 2) grid = p.R / 2;
-    sm_launch(k_row2_fwd<R1, R2, R3, T, false>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes);
+    sm_launch(k_row2_fwd<R1, R2, R3, T, false>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes, RowFwdPair{});
     SM_LAUNCH_CHECK();
     return 0;
   } else {
@@ -1613,18 +1694,19 @@ static int launch_row2_inv4(const SmPlan& p, const RowInvArgs& ia, const cf* twC
   return 0;
 }
 
-// one row per CTA, lanes = even / odd halves (k_row1_fwd_eo): Ch = 2 * R1*R2*R3*R4
-template <int R1, int R2, int R3, int R4, int T, int kCtas>
-static int launch_row1_fwd_eo(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st) {
+// one row per CTA, lanes = even / odd halves (k_row1_fwd_eo): Ch = 2 * R1*R2*R3*R4; kPair: that row of both models (pr)
+template <int R1, int R2, int R3, int R4, int T, int kCtas, bool kPair = false>
+static int launch_row1_fwd_eo(const SmPlan& p, const RowFwdArgs& fa, const cf* twC, const cf* twQ, double* sumsq, cudaStream_t st,
+                              const RowFwdPair& pr = RowFwdPair{}) {
   constexpr int CH = R1 * R2 * R3 * R4;
   if (fa.mode != 0 || p.R < 1 || p.C % 8 != 0 || p.Ch != 2 * CH) return 1;
   static bool done = false;
   const int smem = CH * 16;
-  cudaError_t e = opt_in(k_row1_fwd_eo<R1, R2, R3, R4, T, kCtas>, &done);
+  cudaError_t e = opt_in(k_row1_fwd_eo<R1, R2, R3, R4, T, kCtas, kPair>, &done);
   if (e != cudaSuccess) { sm_set_error("row1 fwd eo setup: %s", cudaGetErrorString(e)); return -100; }
   int grid = num_sms() * kCtas;
   if (grid > p.R) grid = p.R;
-  sm_launch(k_row1_fwd_eo<R1, R2, R3, R4, T, kCtas>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq);
+  sm_launch(k_row1_fwd_eo<R1, R2, R3, R4, T, kCtas, kPair>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, pr);
   SM_LAUNCH_CHECK();
   return 0;
 }
@@ -1643,7 +1725,7 @@ static int launch_row1_fwd_eo3(const SmPlan& p, const RowFwdArgs& fa, const cf* 
   if (e != cudaSuccess) { sm_set_error("row1 fwd eo3 setup: %s", cudaGetErrorString(e)); return -100; }
   int grid = num_sms() * (occ > 0 ? occ : 1);
   if (grid > p.R) grid = p.R;
-  sm_launch(k_row2_fwd<R1, R2, R3, T, true>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes);
+  sm_launch(k_row2_fwd<R1, R2, R3, T, true>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes, RowFwdPair{});
   SM_LAUNCH_CHECK();
   return 0;
 }
@@ -1781,14 +1863,16 @@ static int launch_row_ct(bool inverse, const SmPlan& p, const RowFwdArgs* fa, co
   return 0;
 }
 
+static bool row_radices_are(const SmPlan& p, int n, int a, int b, int c, int d) {
+  if (p.n_row != n) return false;
+  const int want[4] = {a, b, c, d};
+  for (int i = 0; i < n; ++i) if (p.row_rad[i] != want[i]) return false;
+  return true;
+}
+
 static int try_row_ct(bool inverse, const SmPlan& p, const RowFwdArgs* fa, const RowInvArgs* ia, const cf* twC,
                       const cf* twQ, double* sumsq, cudaStream_t st) {
-  auto is = [&](int n, int a, int b, int c, int d) {
-    if (p.n_row != n) return false;
-    const int want[4] = {a, b, c, d};
-    for (int i = 0; i < n; ++i) if (p.row_rad[i] != want[i]) return false;
-    return true;
-  };
+  auto is = [&](int n, int a, int b, int c, int d) { return row_radices_are(p, n, a, b, c, d); };
   if (is(3, 16, 8, 8, 1) && p.row_threads == 64 && p.row_pad) return launch_row_ct<16, 8, 8, 1, 64, true>(inverse, p, fa, ia, twC, twQ, sumsq, st);
   if (is(3, 16, 16, 8, 1) && p.row_threads == 128 && p.row_pad) return launch_row_ct<16, 16, 8, 1, 128, true>(inverse, p, fa, ia, twC, twQ, sumsq, st);
   if (is(3, 16, 16, 16, 1) && p.row_threads == 256 && p.row_pad) return launch_row_ct<16, 16, 16, 1, 256, true>(inverse, p, fa, ia, twC, twQ, sumsq, st);
@@ -1815,6 +1899,61 @@ extern "C" int sm_fwd_rows_bf16(const sm_plan* plan, const void* tables, const v
   a.mode = 0; a.base = (const uint16_t*)base_bf16; a.ft = (const uint16_t*)ft_bf16;
   a.m1 = 1.f; a.m2 = 1.f; a.re = re; a.im = im;
   return launch_row_fwd(plan->p, tables, a, sumsq, (cudaStream_t)stream);
+}
+
+// ---- both finetunes over one shared base in one pass (sm_fwd_rows_bf16_pair).  A plan gets the paired kernel only where
+// sm_fwd_rows_bf16 runs the same kernel per model (try_row_ct -> try_row2_fwd / try_row2_fwd4), so each model's spectrum
+// is bit for bit the single-model pass's: C = 4096 (k_row2_fwd: 24 KB staged per row instead of 32 KB per row pair; the
+// CTA stays at 3 per SM, a 4th does not fit 228 KB with the 35 KB work buffer) and C = 14336 (k_row1_fwd_eo).  C = 28672
+// through k_row1_fwd_eo<7,16,8,8,448,1,true> measured the same row-pass time as two single-model passes (B200, 1000 W:
+// 6.86 / 6.87 against 6.81 / 6.94 ms per 2 Llama-70B layers) and C = 8192 has no paired kernel: both keep two passes.
+enum RowPairKind { kRowPairNone = 0, kRowPairRow2, kRowPairEo7168 };
+static RowPairKind row_pair_kind(const SmPlan& p) {
+  if (p.C % 8 != 0 || p.R < 1) return kRowPairNone;
+  if (row_radices_are(p, 3, 16, 16, 8, 1) && p.row_threads == 128 && p.row_pad && p.R % 2 == 0) return kRowPairRow2;
+  if (row_radices_are(p, 4, 7, 16, 8, 8) && p.row_threads == 448 && p.row_pad && p.Ch == 7168) return kRowPairEo7168;
+  return kRowPairNone;
+}
+
+template <int R1, int R2, int R3, int T>
+static int launch_row2_fwd_pair(const SmPlan& p, const RowFwdArgs& fa, const RowFwdPair& pr, const cf* twC, const cf* twQ,
+                                double* sumsq, cudaStream_t st) {
+  constexpr int CH = R1 * R2 * R3;
+  static bool done = false;
+  static int occ = 0;
+  const int work_bytes = ((CH + (CH >> 4) + 1) * 16 + 127) / 128 * 128;
+  const int smem = work_bytes + 6 * p.C;           // staging: the base row and the row of each finetune
+  cudaError_t e = opt_in(k_row2_fwd<R1, R2, R3, T, false, true>, &done);
+  if (e == cudaSuccess && occ == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_row2_fwd<R1, R2, R3, T, false, true>, T, smem);
+  if (e != cudaSuccess) { sm_set_error("row2 pair setup: %s", cudaGetErrorString(e)); return -100; }
+  int grid = num_sms() * (occ > 0 ? occ : 1);
+  if (grid > p.R) grid = p.R;
+  sm_launch(k_row2_fwd<R1, R2, R3, T, false, true>, dim3(grid), dim3(T), (size_t)(smem), st, p.R, p.C, p.P, fa, twC, twQ, sumsq, work_bytes, pr);
+  SM_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int sm_fwd_rows_pair_supported(const sm_plan* plan) { return row_pair_kind(plan->p) != kRowPairNone ? 1 : 0; }
+
+extern "C" int sm_fwd_rows_bf16_pair(const sm_plan* plan, const void* tables, const void* base_bf16, const void* ft0_bf16,
+                                     const void* ft1_bf16, float* re0, float* im0, float* re1, float* im1, void* ctl,
+                                     double target_norm_offset, double target_norm, void* stream) {
+  const SmPlan& p = plan->p;
+  RowFwdArgs a{};
+  a.mode = 0; a.base = (const uint16_t*)base_bf16; a.ft = (const uint16_t*)ft0_bf16;
+  a.m1 = 1.f; a.m2 = 1.f; a.re = re0; a.im = im0;
+  const RowFwdPair pr{(const uint16_t*)ft1_bf16, re1, im1, (unsigned char*)ctl, target_norm_offset, target_norm};
+  double* sumsq = reinterpret_cast<double*>((unsigned char*)ctl + SM_CTL_SUMSQ);
+  const cf* twC = tabC(p, tables);
+  const cf* twQ = tabQ(p, tables);
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (row_pair_kind(p)) {
+    case kRowPairRow2: return launch_row2_fwd_pair<16, 16, 8, 128>(p, a, pr, twC, twQ, sumsq, st);
+    case kRowPairEo7168: return launch_row1_fwd_eo<7, 8, 8, 8, 224, 2, true>(p, a, twC, twQ, sumsq, st, pr);
+    default: break;
+  }
+  sm_set_error("sm_fwd_rows_bf16_pair: no paired row kernel for [%d][%d] (sm_fwd_rows_pair_supported)", p.R, p.C);
+  return -102;
 }
 
 extern "C" int sm_fwd_rows_f32(const sm_plan* plan, const void* tables, const float* x, float m1, float m2,

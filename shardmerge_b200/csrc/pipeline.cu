@@ -7,7 +7,8 @@
 // one-thread kernel (k_prepare) makes the same decisions on the device right after the row
 // passes: it writes the per-model spectrum scales 1/||delta||, target_norm, the role flag
 // `swap` and the branch code into the scalar block, and every later kernel reads what it needs
-// from there.  The chain always continues down the SLERP branch (what the BASELINE configs
+// from there.  When both finetunes share one base, one paired row pass transforms both (the base
+// is read once) and its last CTA makes these decisions instead (sm_prepare_scalars, sm_internal.h).  The chain always continues down the SLERP branch (what the BASELINE configs
 // take); if k_prepare found another branch, or an order-statistic window missed, the caller sees
 // it in the scalar block afterwards and re-runs that tensor on the step-by-step path.
 #include <vector>
@@ -15,34 +16,12 @@
 
 namespace {
 
-// ext_tn > 0: the target norm is given (the mean over ALL models of the layer in a pair tree, fast_fourier.py:165);
 // use_host_sumsq: the row passes ran earlier and the host passes their sums of squares in (tree round 1)
 __global__ void k_prepare(unsigned char* ctl, double target_norm_offset, double ext_tn, int use_host_sumsq, double hs0, double hs1) {
   sm_pdl_enter();
   double* sumsq = reinterpret_cast<double*>(ctl + SM_CTL_SUMSQ);
   if (use_host_sumsq) { sumsq[0] = hs0; sumsq[1] = hs1; }
-  float* flt = reinterpret_cast<float*>(ctl + SM_CTL_FLT);
-  int* ints = reinterpret_cast<int*>(ctl + SM_CTL_INT);
-  double* tn_out = reinterpret_cast<double*>(ctl + SM_CTL_TN);
-  // torch.norm(delta) is an fp32 scalar; .item() widens it to a Python float
-  const float nx = (float)sqrt(sumsq[0]), ny = (float)sqrt(sumsq[1]);
-  const int swap = fabsf(nx) < fabsf(ny) ? 1 : 0;              // fast_fourier.py:212
-  const double na = swap ? (double)ny : (double)nx, nb = swap ? (double)nx : (double)ny;
-  const float mean32 = (nx + ny) / 2.0f;                        // torch.tensor(layer_norms).mean()  (:165)
-  const double tn = ext_tn > 0.0 ? ext_tn : (double)mean32 + target_norm_offset;
-  const double cnorm_a = fabs(na / tn), cnorm_b = fabs(nb / tn);
-  const double n_ratio = cnorm_b / (cnorm_a + 1e-10);
-  int branch = SM_BRANCH_SLERP;
-  if (cnorm_a < 1e-6) branch = SM_BRANCH_ADD;                                   // :223
-  else if (cnorm_b < 1e-6 || n_ratio < 0.1) branch = SM_BRANCH_ARITH;            // :226
-  else if (nb < 1e-4 || na < 1e-4) branch = SM_BRANCH_EARLY;                     // functions.py:184-190
-  else if (nb / (na + 1e-10) < 0.1) branch = SM_BRANCH_LINEAR;                   // functions.py:199-202
-  flt[SM_F_SCALE_X] = nx != 0.f ? 1.0f / nx : 1.0f;             // normalize_tensor: x * (1/norm), fp32
-  flt[SM_F_SCALE_Y] = ny != 0.f ? 1.0f / ny : 1.0f;
-  flt[SM_F_OUT_SCALE] = (float)tn;
-  flt[SM_F_NORM_X] = nx; flt[SM_F_NORM_Y] = ny;
-  ints[SM_I_SWAP] = swap; ints[SM_I_BRANCH] = branch;
-  *tn_out = tn;
+  sm_prepare_scalars(ctl, sumsq[0], sumsq[1], target_norm_offset, ext_tn);
 }
 
 // ------------------------------------------------------------------ optional per-class timing
@@ -101,17 +80,24 @@ extern "C" int sm_pair_merge_async(const sm_plan* plan, const void* tables, cons
   int rc;
   SM_CUDA_CHECK(cudaMemsetAsync(ctl, 0, SM_CTL_BYTES, st));
   const bool rows_done = a->rows_done != 0;
-  if (!rows_done) {
-    // bf16 (base, finetune) pairs: 2N + 2N read, 4N written; fp32 tree intermediates: 4N read, 4N written
-    Scope s(st, SM_CLS_ROW_FWD, 16.0 * N, 2);
-    if (a->x32_0 != nullptr) {
-      if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_0, 1.f, 1.f, a->re[0], a->im[0], dbl + 0, st))) return rc;
-    } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base0, a->ft0, a->re[0], a->im[0], dbl + 0, st))) return rc;
-    if (a->x32_1 != nullptr) {
-      if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_1, 1.f, 1.f, a->re[1], a->im[1], dbl + 1, st))) return rc;
-    } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base1, a->ft1, a->re[1], a->im[1], dbl + 1, st))) return rc;
-  }
-  {
+  const bool paired_rows = !rows_done && a->x32_0 == nullptr && a->x32_1 == nullptr && a->base0 == a->base1 &&
+                           sm_fwd_rows_pair_supported(plan);
+  if (paired_rows) {
+    // one shared base: 2N + 2 x 2N read, 2 x 4N written; the pass's last CTA also does what k_prepare does
+    Scope s(st, SM_CLS_ROW_FWD, 14.0 * N, 1);
+    if ((rc = sm_fwd_rows_bf16_pair(plan, tables, a->base0, a->ft0, a->ft1, a->re[0], a->im[0], a->re[1], a->im[1], ctl,
+                                    a->target_norm_offset, a->target_norm, st))) return rc;
+  } else {
+    if (!rows_done) {
+      // bf16 (base, finetune) pairs: 2N + 2N read, 4N written; fp32 tree intermediates: 4N read, 4N written
+      Scope s(st, SM_CLS_ROW_FWD, 16.0 * N, 2);
+      if (a->x32_0 != nullptr) {
+        if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_0, 1.f, 1.f, a->re[0], a->im[0], dbl + 0, st))) return rc;
+      } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base0, a->ft0, a->re[0], a->im[0], dbl + 0, st))) return rc;
+      if (a->x32_1 != nullptr) {
+        if ((rc = sm_fwd_rows_f32(plan, tables, a->x32_1, 1.f, 1.f, a->re[1], a->im[1], dbl + 1, st))) return rc;
+      } else if ((rc = sm_fwd_rows_bf16(plan, tables, a->base1, a->ft1, a->re[1], a->im[1], dbl + 1, st))) return rc;
+    }
     Scope s(st, SM_CLS_SCALARS, 0.0, 1);
     sm_launch(k_prepare, dim3(1), dim3(1), (size_t)(0), st, ctl, a->target_norm_offset, a->target_norm, rows_done ? 1 : 0,
                                rows_done ? a->sumsq[0] : 0.0, rows_done ? a->sumsq[1] : 0.0);

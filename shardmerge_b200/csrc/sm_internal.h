@@ -52,6 +52,36 @@ static inline void sm_launch(void (*kernel)(KA...), dim3 grid, dim3 block, size_
   cfg.attrs = at; cfg.numAttrs = 1;
   (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<A&&>(args)...);      // errors surface in SM_LAUNCH_CHECK()
 }
+
+// The decisions the reference makes on the host from the two delta norms of a pair merge: which model is "a" (the larger
+// norm, fast_fourier.py:212-215), which branch runs (:223-244) and target_norm (:165).  Writes the per-model spectrum
+// scales 1/||delta||, the norms, target_norm, the role flag `swap` and the branch code into the scalar block.  One thread.
+// ext_tn > 0: the target norm is given (the mean over ALL models of the layer in a pair tree, fast_fourier.py:165).
+__device__ __forceinline__ void sm_prepare_scalars(unsigned char* ctl, double sumsq0, double sumsq1, double target_norm_offset,
+                                                   double ext_tn) {
+  float* flt = reinterpret_cast<float*>(ctl + SM_CTL_FLT);
+  int* ints = reinterpret_cast<int*>(ctl + SM_CTL_INT);
+  double* tn_out = reinterpret_cast<double*>(ctl + SM_CTL_TN);
+  // torch.norm(delta) is an fp32 scalar; .item() widens it to a Python float
+  const float nx = (float)sqrt(sumsq0), ny = (float)sqrt(sumsq1);
+  const int swap = fabsf(nx) < fabsf(ny) ? 1 : 0;              // fast_fourier.py:212
+  const double na = swap ? (double)ny : (double)nx, nb = swap ? (double)nx : (double)ny;
+  const float mean32 = (nx + ny) / 2.0f;                        // torch.tensor(layer_norms).mean()  (:165)
+  const double tn = ext_tn > 0.0 ? ext_tn : (double)mean32 + target_norm_offset;
+  const double cnorm_a = fabs(na / tn), cnorm_b = fabs(nb / tn);
+  const double n_ratio = cnorm_b / (cnorm_a + 1e-10);
+  int branch = SM_BRANCH_SLERP;
+  if (cnorm_a < 1e-6) branch = SM_BRANCH_ADD;                                   // :223
+  else if (cnorm_b < 1e-6 || n_ratio < 0.1) branch = SM_BRANCH_ARITH;            // :226
+  else if (nb < 1e-4 || na < 1e-4) branch = SM_BRANCH_EARLY;                     // functions.py:184-190
+  else if (nb / (na + 1e-10) < 0.1) branch = SM_BRANCH_LINEAR;                   // functions.py:199-202
+  flt[SM_F_SCALE_X] = nx != 0.f ? 1.0f / nx : 1.0f;             // normalize_tensor: x * (1/norm), fp32
+  flt[SM_F_SCALE_Y] = ny != 0.f ? 1.0f / ny : 1.0f;
+  flt[SM_F_OUT_SCALE] = (float)tn;
+  flt[SM_F_NORM_X] = nx; flt[SM_F_NORM_Y] = ny;
+  ints[SM_I_SWAP] = swap; ints[SM_I_BRANCH] = branch;
+  *tn_out = tn;
+}
 #endif
 
 // table layout inside the caller's buffer: [W_C : C entries][W_R : R entries][quads : 4 * (Ch / row_rad[0])]

@@ -646,7 +646,10 @@ def pair_merge_async(ws: Workspace, s0: Source, s1: Source, base_out: Optional[t
     if PROFILER is not None:
         fs = lib.sm_fstats_supported(pl.handle) and not ws.safe_select
         cl = lib.sm_plan_col_launches(pl.handle)          # launches of one column transform (column bands x sweeps)
-        PROFILER.launches += (0 if rows_done else 2) + 1 + 2 * cl + ((2 + 2) if fs else (11 + 2 + 1 + 11)) + (cl if sweeps else 0) + 1
+        # two finetunes of one base: one paired row pass that also makes the scalar decisions (csrc/pipeline.cu)
+        paired = (not rows_done and s0.is_bf16 and s1.is_bf16 and s0.base.data_ptr() == s1.base.data_ptr()
+                  and lib.sm_fwd_rows_pair_supported(pl.handle))
+        PROFILER.launches += (1 if paired else (0 if rows_done else 2) + 1) + 2 * cl + ((2 + 2) if fs else (11 + 2 + 1 + 11)) + (cl if sweeps else 0) + 1
         PROFILER.fused_calls += 1
     _lib.check(lib.sm_pair_merge_async(pl.handle, pl.tables.data_ptr(), ctypes.byref(a), _stream(dev)), "sm_pair_merge_async")
     if _ring is None:
