@@ -6,8 +6,8 @@ ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS   := $(ARCH) -std=c++17 -O3 -lineinfo -Xcompiler -fPIC -Xptxas -v
 CSRC      := shardmerge_b200/csrc
 LIB       := shardmerge_b200/libshardmerge_b200.so
-HDRS      := $(CSRC)/elem_codec.cuh $(CSRC)/fft_core.cuh $(CSRC)/fft_bodies.cuh $(CSRC)/plan.h $(CSRC)/sm_internal.h include/shardmerge_b200.h
-OBJS      := build/kernels_fft.o build/kernels_stats.o build/kernels_fstats.o build/kernels_elem.o build/kernels_lora.o build/kernels_lowrank.o build/pipeline.o
+HDRS      := $(CSRC)/elem_codec.cuh $(CSRC)/fft_core.cuh $(CSRC)/fft_bodies.cuh $(CSRC)/plan.h $(CSRC)/select_core.cuh $(CSRC)/sm_internal.h include/shardmerge_b200.h
+OBJS      := build/kernels_fft.o build/kernels_stats.o build/kernels_fstats.o build/kernels_elem.o build/kernels_lora.o build/kernels_lowrank.o build/kernels_sparse.o build/pipeline.o
 
 all: $(LIB) hostemu
 

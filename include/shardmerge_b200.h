@@ -317,6 +317,35 @@ int sm_lowrank_right(int R, int C, int k, int w_dtype, const void* W, int m_dtyp
 int sm_lowrank_left(int R, int C, int k, int w_dtype, const void* W, int m_dtype, const void* M, const float* Q, float* Z,
                     void* ws, size_t ws_bytes, void* stream);
 
+/* ---- TIES and DARE: sparsified task vectors, sign election, disjoint mean (DESIGN.md section 8) ------------------------
+ * n elements; base in base_dtype, `fts` = HOST array of n_models device pointers, `ft_dtypes` = HOST array of their dtype
+ * codes (0 fp32, 1 bf16, 2 fp16, each tensor its own); 1..SM_SPARSE_MAX_MODELS models; every tensor 16-byte aligned.
+ * d_i = fp32(ft_i) - fp32(base), one rounding, formed on load and never stored.
+ *
+ * sm_sparse_select (TIES): for every model, the k largest |d_i| with ties taken by the lower flat index, as one
+ * sm_sparse_thr per model at the start of ws: element j is kept iff |d|bits > key || (|d|bits == key && j <= last)
+ * (|d|bits = the fp32 bit pattern with the sign cleared).  k = 0 gives key = 0xffffffff, last = -1 (nothing kept).
+ * status != 0 would mean the select did not resolve (not expected: the select is exact).  ws: 256-byte aligned, at least
+ * sm_sparse_ws_bytes(n, n_models) bytes; no host synchronisation.
+ *
+ * sm_sparse_merge, per element:
+ *   mode 0 TIES:        t_i = kept_i ? d_i : 0                      (kept by the thresholds `thr` of sm_sparse_select)
+ *   mode 1 DARE-TIES:   t_i = kept_i ? d_i / density : 0            (kept iff (word >> 8) < keep24, word = word j & 3 of
+ *   mode 2 DARE-linear:                                              Philox4x32-10 at counter (c lo, c hi, 0, 0), c = j >> 2,
+ *                                                                    key (keys[2i], keys[2i+1]), HOST array)
+ *   v_i = weights[i] * t_i;  modes 0 and 1: S = sum v_i, mask_i = sign(v_i) == (S >= 0 ? +1 : -1); mode 2: mask_i = 1;
+ *   m = sum mask_i v_i,  D = sum mask_i weights[i] (1 if 0),  out = round_to(base_dtype)(fp32(base) + scale * (m / D)).
+ * Every operation is one fp32 rounding, sums in ascending i from +0.0.  nonfinite: n_models u32 (zeroed by the call),
+ * += the number of non-finite d_i of each model.  `out` must not alias an input. */
+#define SM_SPARSE_MAX_MODELS 64
+typedef struct sm_sparse_thr { uint32_t key; uint32_t status; int64_t last; } sm_sparse_thr;
+size_t sm_sparse_ws_bytes(size_t n, int n_models);
+int sm_sparse_select(size_t n, uint64_t k, int base_dtype, const void* base, const int* ft_dtypes, const void* const* fts,
+                     int n_models, void* ws, size_t ws_bytes, void* stream);
+int sm_sparse_merge(int mode, size_t n, int base_dtype, const void* base, const int* ft_dtypes, const void* const* fts,
+                    int n_models, const float* weights, const uint32_t* keys, float density, uint32_t keep24, float scale,
+                    const void* thr, uint32_t* nonfinite, void* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

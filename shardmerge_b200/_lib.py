@@ -52,6 +52,9 @@ SIGNATURES = {
     "sm_lowrank_ws_bytes": (_sz, [_i, _i, _i]),
     "sm_lowrank_right": (_i, [_i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "sm_lowrank_left": (_i, [_i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "sm_sparse_ws_bytes": (_sz, [_sz, _i]),
+    "sm_sparse_select": (_i, [_sz, _u64, _i, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
+    "sm_sparse_merge": (_i, [_i, _sz, _i, _vp, _vp, _vp, _i, _vp, _vp, _f, C.c_uint32, _f, _vp, _vp, _vp, _vp]),
     "sm_copy_bytes": (_i, [_vp, _vp, _sz, _vp]),
     "sm_expand_full": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "sm_pack_half": (_i, [_vp, _vp, _vp, _vp, _vp]),

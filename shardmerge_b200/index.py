@@ -141,6 +141,9 @@ class InMemoryIndex(_IndexBase):
     def tensor_shapes(self, model_uri: str) -> Dict[str, tuple]:
         return {n: tuple(t.shape) for n, t in self.models[model_uri].items()}
 
+    def tensor_dtypes(self, model_uri: str) -> Dict[str, torch.dtype]:
+        return {n: t.dtype for n, t in self.models[model_uri].items()}
+
     def _host_tensor(self, model_uri: str, tensor_name: str) -> torch.Tensor:
         return self.models[model_uri][tensor_name]
 
@@ -257,6 +260,17 @@ class LocalSafetensorsIndex(_IndexBase):
         for shard in sorted(set(index["weight_map"].values())):
             for key, (_, shape, _, _) in self._meta(self.storage_dir / model_uri / shard)[1].items():
                 out[key] = shape
+        return out
+
+    def tensor_dtypes(self, model_uri: str) -> Dict[str, torch.dtype]:
+        """dtypes from the safetensors headers (no tensor data is read); a bound adapter has its base's."""
+        if model_uri in self._adapters:
+            return self.tensor_dtypes(self._adapters[model_uri].base)
+        out: Dict[str, torch.dtype] = {}
+        index = self.model_indexes[model_uri]
+        for shard in sorted(set(index["weight_map"].values())):
+            for key, (dtype, _, _, _) in self._meta(self.storage_dir / model_uri / shard)[1].items():
+                out[key] = dtype
         return out
 
     def tensor_numels(self, model_uri: str) -> Dict[str, int]:

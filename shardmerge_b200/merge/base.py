@@ -11,11 +11,13 @@ from __future__ import annotations
 
 import logging
 from abc import ABC, abstractmethod
-from typing import List
+from typing import List, Optional
 
 import torch
 
+from .. import lora
 from ..config import MergeConfig, MergeModel
+from ..constants import INPUT_LAYER
 from ..lora import UnsupportedAdapter
 from ..writer import ModelWriter, ShardLayer
 
@@ -81,6 +83,47 @@ class MergeTensorsBase(ABC):
             if want - have or have - want:
                 raise ValueError(f"Model {m.model} architecture mismatch with base model {self.config.output_base_model}\n"
                                  f"Missing keys: {want - have}\nExtra keys: {have - want}")
+
+    # ---- INPUT_LAYER / OUTPUT_LAYER tensors (embed, final norm, lm_head) are copied, not merged --------------------------
+    def _adapter_part(self, model_uri: str, name: str) -> Optional[lora.Part]:
+        """lora.Part of `name` when `model_uri` is a LoRA adapter, else None (also for index managers without adapters)."""
+        part_of = getattr(self.index_manager, "adapter_part", None)
+        return None if part_of is None else part_of(model_uri, name)
+
+    async def _adapter_tensor(self, model_uri: str, part: lora.Part, base: Optional[torch.Tensor], device: str) -> torch.Tensor:
+        """The adapter's finetuned tensor: `base` itself, the adapter's full tensor, or base + scaling * B @ A formed on the
+        device from the factors (the base tensor is the caller's: it crosses the host link once per merged tensor)."""
+        if part.kind == "base":
+            return base
+        got = [await self.index_manager.get_tensor(model_uri, key, device=device).get() for key in part.keys]
+        if part.kind == "full":
+            return got[0]
+        return lora.materialize(base, got[0], got[1], part.scaling)
+
+    def _passthrough_source(self, shard_layer: ShardLayer):
+        """(model entry, model uri) an INPUT_LAYER / OUTPUT_LAYER tensor is copied from: the first `is_input` /
+        `is_output` finetune (shard/merge/fast_fourier.py:104-130), else the output base (entry None)."""
+        attr = "is_input" if shard_layer.layer_number == INPUT_LAYER else "is_output"
+        chosen = next((m for m in self.config.finetune_merge if getattr(m, attr)), None)
+        return chosen, (chosen.model if chosen is not None else self.config.output_base_model)
+
+    async def _passthrough(self, shard_layer: ShardLayer, device) -> torch.Tensor:
+        chosen, source = self._passthrough_source(shard_layer)
+        name = shard_layer.layer_name
+        logger.info(f"Passthrough - {name} from {source}")
+        part = self._adapter_part(source, name)
+        if part is not None:
+            base = None if part.kind == "full" else await self.index_manager.get_tensor(chosen.base, name, device=device).get()
+            return await self._adapter_tensor(source, part, base, device)
+        return await self.index_manager.get_tensor(source, name, device=device).get()
+
+    def _prefetch_passthrough(self, shard_layer: ShardLayer, device, prefetch):
+        chosen, source = self._passthrough_source(shard_layer)
+        name = shard_layer.layer_name
+        part = self._adapter_part(source, name)
+        if part is not None and part.kind != "full":
+            prefetch(chosen.base, name, device)
+        prefetch(source, name, device)          # an adapter's factors or full tensor, if it has any for `name`
 
     def get_writer(self, layer_order: list, **kwargs) -> ModelWriter:
         return ModelWriter(base_index=self.index_doc, output_path=self.config.output_path, layer_order=layer_order,

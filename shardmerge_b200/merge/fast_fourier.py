@@ -23,7 +23,6 @@ from typing import List, NamedTuple, Optional
 import torch
 
 from .. import engine as E
-from .. import lora
 from ..config import MergeConfig
 from ..constants import INPUT_LAYER, OUTPUT_LAYER
 from ..tensor.functions import correlated_pairs, retry_on_select_miss
@@ -172,45 +171,13 @@ class FourierMerge(MergeTensorsBase):
                                      f"FFT path:\n{lines}")
 
     # -------------------------------------------------------------------------------------
-    def _adapter_part(self, model_uri: str, name: str) -> Optional[lora.Part]:
-        """lora.Part of `name` when `model_uri` is a LoRA adapter, else None (also for index managers without adapters)."""
-        part_of = getattr(self.index_manager, "adapter_part", None)
-        return None if part_of is None else part_of(model_uri, name)
-
-    async def _adapter_tensor(self, model_uri: str, part: lora.Part, base: Optional[torch.Tensor], device: str) -> torch.Tensor:
-        """The adapter's finetuned tensor: `base` itself, the adapter's full tensor, or base + scaling * B @ A formed on the
-        device from the factors (the base tensor is the caller's: it crosses the host link once per merged tensor)."""
-        if part.kind == "base":
-            return base
-        got = [await self.index_manager.get_tensor(model_uri, key, device=device).get() for key in part.keys]
-        if part.kind == "full":
-            return got[0]
-        return lora.materialize(base, got[0], got[1], part.scaling)
-
-    async def _passthrough(self, shard_layer, device, attr: str) -> torch.Tensor:
-        chosen = next((m for m in self.config.finetune_merge if getattr(m, attr)), None)
-        source = chosen.model if chosen is not None else self.config.output_base_model
-        name = shard_layer.layer_name
-        logger.info(f"Passthrough - {name} from {source}")
-        part = self._adapter_part(source, name)
-        if part is not None:
-            base = None if part.kind == "full" else await self.index_manager.get_tensor(chosen.base, name, device=device).get()
-            return await self._adapter_tensor(source, part, base, device)
-        return await self.index_manager.get_tensor(source, name, device=device).get()
-
     def prefetch_layer(self, shard_layer, device: str):
         prefetch = getattr(self.index_manager, "prefetch", None)
         if prefetch is None or not str(device).startswith("cuda"):
             return
         number, name = shard_layer.layer_number, shard_layer.layer_name
         if number in (INPUT_LAYER, OUTPUT_LAYER):
-            attr = "is_input" if number == INPUT_LAYER else "is_output"
-            chosen = next((m for m in self.config.finetune_merge if getattr(m, attr)), None)
-            source = chosen.model if chosen is not None else self.config.output_base_model
-            part = self._adapter_part(source, name)
-            if part is not None and part.kind != "full":
-                prefetch(chosen.base, name, device)
-            prefetch(source, name, device)          # an adapter's factors or full tensor, if it has any for `name`
+            self._prefetch_passthrough(shard_layer, device, prefetch)
             return
         wanted = [self.config.output_base_model]
         for m in self.config.finetune_merge:
@@ -221,10 +188,8 @@ class FourierMerge(MergeTensorsBase):
 
     async def _merge_layer(self, shard_layer, device: str) -> torch.Tensor:
         number = shard_layer.layer_number
-        if number == INPUT_LAYER:
-            return await self._passthrough(shard_layer, device, "is_input")
-        if number == OUTPUT_LAYER:
-            return await self._passthrough(shard_layer, device, "is_output")
+        if number in (INPUT_LAYER, OUTPUT_LAYER):
+            return await self._passthrough(shard_layer, device)
 
         dev = E._require_cuda(device)
         name = shard_layer.layer_name
