@@ -39,6 +39,17 @@ def f32_to_bf16(x: np.ndarray) -> np.ndarray:
     return r
 
 
+def widen(x: np.ndarray) -> np.ndarray:
+    """A stored tensor as fp32, exactly: uint16 arrays are bf16 bit patterns, float16 and float32 arrays are taken as
+    they are (what `.to(torch.float32)` does to a bf16, fp16 or fp32 tensor)."""
+    x = np.asarray(x)
+    if x.dtype == np.uint16:
+        return bf16_to_f32(x)
+    if x.dtype in (np.float16, np.float32):
+        return x.astype(np.float32)
+    raise TypeError(f"no stored tensor dtype is carried as {x.dtype} (uint16 = bf16 bits, float16, float32)")
+
+
 def norm32(x: np.ndarray) -> float:
     """torch.norm of an fp32 tensor, restated with an accurate (fp64) accumulation and the
     fp32 result torch would hand back through .item()."""
@@ -218,15 +229,15 @@ def merge_layer(base_out_bf16, models, target_norm_offset=1e-10, cull_start_pct=
     """FourierMerge._merge_layer for a regular (model.layers.*) tensor,
     shard/merge/fast_fourier.py:132-276, with the disk cache replaced by a dict.
 
-    base_out_bf16: uint16 bit patterns of the output-base tensor.
-    models: list of dicts {base: u16 array, ft: u16 array, alpha: float, name: str}
+    base_out_bf16: the output-base tensor -- uint16 bf16 bit patterns, or a float16 / float32 array (see `widen`).
+    models: list of dicts {base: array, ft: array, alpha: float, name: str}, arrays stored as base_out_bf16 may be
             (already filtered by use_layer_index, :135).
     Returns uint16 bit patterns of the merged bf16 tensor.
     """
     cache = {}
     norms, stack, weights = [], [], []
     for m in models:                                                         # :147-158
-        delta = (bf16_to_f32(m["ft"]) - bf16_to_f32(m["base"])).astype(np.float32)   # base.py:128-132
+        delta = (widen(m["ft"]) - widen(m["base"])).astype(np.float32)   # base.py:128-132
         norms.append(np.float32(norm32(delta)))
         cache[m["name"]] = delta
         stack.append(m["name"]); weights.append(float(m["alpha"]))
@@ -271,7 +282,7 @@ def merge_layer(base_out_bf16, models, target_norm_offset=1e-10, cull_start_pct=
         cull_pct = cull_pct / 2.0                                            # :254
     result = cache[stack[0]]                                                 # :256-257
     with np.errstate(invalid="ignore"):
-        result = (bf16_to_f32(base_out_bf16) + result).astype(np.float32)    # :269
+        result = (widen(base_out_bf16) + result).astype(np.float32)          # :269
     result = np.where(np.isnan(result), np.float32(0), result).astype(np.float32)   # :270-271
     if np.any(np.isinf(result)):                                             # :273-274
         raise ValueError("Inf in merged tensor")

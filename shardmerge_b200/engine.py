@@ -382,7 +382,10 @@ def select_kth(ws: Workspace, plane0: torch.Tensor, plane1: Optional[torch.Tenso
 
 
 def slerp_reduce(ws: Workspace, re0: torch.Tensor, re1: torch.Tensor):
+    """Masked SLERP sums into D_S00 / D_S11 / D_S01.  The kernel adds its partial sums atomically, so they start from
+    zero here: a tree runs one pair after another on the same workspace, and the scalar block is zeroed once per tensor."""
     pl, lib = ws.plan, ws.plan.lib
+    ws.dbl[D_S00:D_S00 + 3].zero_()
     _lib.check(_run("reduce", 1, 4 * pl.R * pl.C, pl.device, lambda: lib.sm_slerp_reduce(
         pl.handle, re0.data_ptr(), re1.data_ptr(), ws.fptr(F_THR_CUT), ws.dptr(D_S00), _stream(pl.device))), "sm_slerp_reduce")
 

@@ -124,7 +124,8 @@ class FourierMerge(MergeTensorsBase):
         self._lane_streams: dict = {}    # device index -> [streams]
         self._lane_next = 0
         self._tree_waiting: list = []    # pair trees whose row passes are enqueued but whose norms have not been read yet
-        self.keep_intermediates = False  # tests: keep the tree's fp32 round results in self.last_tree
+        self.keep_intermediates = False  # tests: keep the tree's fp32 round results in self.last_tree (the step path also keeps
+                                         # the last round's when the output base is not bf16: the merged delta before the base)
         self.last_tree: list = []
 
     def get_readme(self) -> str:
@@ -443,6 +444,7 @@ class FourierMerge(MergeTensorsBase):
         # stack entries: (source, slot of its row spectrum or None)
         stack = [(s, i) for i, s in enumerate(sources)]
         out_final: Optional[torch.Tensor] = None
+        kept = []
         for steps in rounds:
             nxt = []
             for st in steps:
@@ -499,7 +501,10 @@ class FourierMerge(MergeTensorsBase):
                     inter = E.Source(x32=merged.reshape(R, C) if merged.ndim == 1 else merged,
                                      weight=(a_w + b_w) / 2.0, name=name_hash(f"{sa.name}_{sb.name}"))
                     nxt.append((inter, None))
+                    kept.append((sa.name, sb.name, inter.x32))
             stack = nxt
+        if self.keep_intermediates:
+            self.last_tree = kept
 
         _, _, flags, _ = ws.read_ctl()
         info["flags"] = [int(v) for v in flags]
@@ -566,7 +571,8 @@ def _pair_elementwise(sa, sb, ca, cb, scale, final, base_out, ws, out):
     if final and out.dtype == torch.bfloat16 and sa.is_bf16 and sb.is_bf16:
         E.delta_axpby_bf16(base_out, sa, ca, sb, cb, scale, out, ws.flags)
         return out
-    res = (sa.delta_f32() * ca + sb.delta_f32() * cb) * scale
+    # a stacked source's delta keeps its leading dimensions, a tree intermediate is one [R][C] matrix
+    res = (sa.delta_f32().reshape(out.shape) * ca + sb.delta_f32().reshape(out.shape) * cb) * scale
     _store(res, final, base_out, out)
     return out
 

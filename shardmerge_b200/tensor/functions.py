@@ -308,7 +308,9 @@ def correlate_pairs(tensors: torch.Tensor, work_device: str, store_device: str) 
 def correlated_pairs(correlation_matrix: torch.Tensor, way: Literal['least', 'most'] = 'least'
                      ) -> Generator[tuple[int, int, float], None, None]:
     """Greedy pairing over the upper triangle by least / most |correlation|; every index is used
-    once, leftovers are yielded as (i, -1, corr[i, i]) (functions.py:316-365)."""
+    once, leftovers are yielded as (i, -1, corr[i, i]) (functions.py:316-365).  Only finite
+    entries are candidates: with +Inf entries alone left (the norm product of a model whose
+    delta holds an Inf) the reference's min / max runs over an empty selection and raises."""
     if way not in ("least", "most"):
         raise ValueError("Invalid way. Choose 'least' or 'most'.")
     c = correlation_matrix.detach().to("cpu", torch.float64)
@@ -318,9 +320,14 @@ def correlated_pairs(correlation_matrix: torch.Tensor, way: Literal['least', 'mo
         best = None
         for ii, x in enumerate(free):                         # row-major scan = first match of torch.nonzero
             for y in free[ii + 1:]:
-                v = abs(c[x, y].item())
+                v = c[x, y].item()
+                if v == float("inf"):
+                    continue
+                v = abs(v)
                 if best is None or (v < best[0] if way == "least" else v > best[0]):
                     best = (v, x, y)
+        if best is None:
+            raise ValueError(f"correlated_pairs: every correlation left between indices {free} is infinite")
         _, x, y = best
         yield (x, y, correlation_matrix[x, y].item())
         free.remove(x); free.remove(y)
